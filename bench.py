@@ -2,6 +2,7 @@
 """Benchmark of the gecco sampling hot path (BASELINE.json: point clouds/sec, 2048 points, full EDM sampler).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4}] [--impl {b200,reference,reference-cuda}]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`, SURVEY.md §8d); `--config 2` is the default and the N = 1 headline:
   1  ShapeNet-PointFlow unconditional: LinearLift + GaussianReparam, 4 clouds per GPU (the reference's CPU-runnable case)
@@ -20,6 +21,9 @@ events on the launching stream by the engine's per-kernel-class profiler.
 travel to the GPU box) on the host cores, on a bounded sample of the same workload.
 `--impl reference-cuda`: the same restatement as plain PyTorch eager on the B200 (cuBLAS / SDPA / native group-norm and
 grid-sampler kernels), fp32 and bf16 autocast: the library path a gecco-torch user has today (BASELINE.md §4).
+`--dump-outputs DIR`: the result of the last timed step, `samples.npy` (configs 1-4, float64 data-space clouds) or
+`loss.npy` + `parameters.npy` (config 5, the updated flat fp32 weights, sampled to fit 64 MB).  Inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -86,6 +90,26 @@ def peaks():
         return dict(hbm=j["hbm_gbs"], tf_burst=j["bf16_tflops"], tf_sustained=j.get("bf16_tflops_sustained", j["bf16_tflops"]),
                     source="measured (MEASURED_PEAKS.json)")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sustained=1400.0, source="fallback (B200_PROFILING.md)")
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Writes every array as <directory>/<name>.npy, float64 kept and anything else as float32, DUMP_BYTES in all.  An
+    array over its equal share keeps a fixed, seeded sample of its rows (dim 0, in order), so that two builds run with
+    the same arguments write the same positions and can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096  # room for the .npy header
+    for name, t in arrays.items():
+        t = t.detach().cpu().reshape(t.shape if t.dim() else (1,))
+        t = t if t.dtype == torch.float64 else t.float()
+        rows = max(1, share // (t[0].numel() * t.element_size()))
+        if rows < t.shape[0]:
+            t = t[torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+        np.save(os.path.join(directory, name + ".npy"), t.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -243,14 +267,14 @@ def run_own(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=device)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return ms.item()
+        return ms.item(), out
 
     for _ in range(args.warmup):
         out = step_resident()
@@ -258,11 +282,13 @@ def run_own(args):
     eng = E.engine_for(*model._network())
     clocks = ClockSampler(local) if rank == 0 else None
     E.launch_count(reset=True)
-    ms = timed(step_resident, args.steps)
+    ms, out = timed(step_resident, args.steps)
     launches = E.launch_count(reset=True)
     graph_status = eng.graph_status()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"samples": out})
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clk = clocks.stop() if clocks else None
 
     # host time to enqueue one step (no synchronisation inside): if it approaches ms_per_step the run is launch-bound
@@ -410,6 +436,8 @@ def run_train(args):
     launches = E.launch_count(reset=True)
     if trainer.graph_mode:  # the captured forward + backward replays its library kernels without passing the C ABI again
         launches += trainer.graph_library_launches * args.steps
+    if args.dump_outputs and rank == 0:  # the step returns the loss; the updated weights are the rest of its result
+        dump_outputs(args.dump_outputs, {"loss": loss, "parameters": trainer.state.p})
     ms_e2e, _ = timed(step_e2e, args.steps)
     clk = clocks.stop() if clocks else None
     mem_gb = torch.cuda.max_memory_allocated(device) / 2**30
@@ -591,10 +619,17 @@ def main():
     ap.add_argument("--config", type=int, default=int(os.environ.get("GECCO_BENCH_CONFIG", "2")), choices=sorted(CONFIGS))
     ap.add_argument("--clouds", type=int, default=0, help="clouds per GPU (default: the config's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (at most 64 MB "
+                         "in all; a larger output is replaced by a fixed, seeded sample of its rows)")
     args = ap.parse_args()
     if args.impl != "b200":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl b200")
         run_reference(args)
         return
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; gecco_b200 has no CPU path (use --impl reference for the CPU baseline)")
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -602,7 +637,9 @@ def main():
         # convenience: re-launch under torchrun
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr",
                "127.0.0.1", "--master-port", "29531", __file__, "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup",
-               str(args.warmup), "--config", str(args.config)] + (["--no-cpu-baseline"] if args.no_cpu_baseline else [])
+               str(args.warmup), "--config", str(args.config), "--clouds", str(args.clouds)] \
+            + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) \
+            + (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         raise SystemExit(subprocess.call(cmd))
     if args.config == 5:
         return run_train(args)

@@ -71,14 +71,21 @@ def test_cond_uvl_cache_upsample_roundtrip():
     data = O.diffusion_to_data(cfg, sd, diff, K)
     assert rel(data, g["rt_data"]) < TOL
     assert rel(O.data_to_diffusion(cfg, sd, data, K), g["rt_back"]) < 1e-4
-    # samples are compared in diffusion space: data space goes through exp() of the depth coordinate
-    s = O.sample_stochastic(cfg, sd, r["sample_shape"], feats, K, rng=synth.gen(r["sample_seed"]), num_steps=r["sample_steps"])
+    # samples are compared in diffusion space: data space goes through exp() of the depth coordinate.  With random-init UVL
+    # weights the sampler trajectories amplify fp32 rounding: on a CPU like the one that minted the goldens the oracle
+    # matches them bit for bit, but another thread count or vector ISA (1 thread, AVX2, SSE) moves the 5-step sample by up
+    # to 5e-3 (max) and the upsampled cloud by up to 4e-2 (rms), where a wrong noise draw moves it by 1.2 (rms).  The short
+    # trajectory (2 steps from sigma 2, oracle/make_golden.py) amplifies nothing (<= 1e-4 on every CPU) and is held tight.
     to_diff = lambda d: O.data_to_diffusion(cfg, sd, d, K.double())
-    assert rel(to_diff(s), to_diff(g["sample"])) < 2e-4
+    s2 = O.sample_stochastic(cfg, sd, (2, 160, 3), feats, K, rng=synth.gen(5), num_steps=2, sigma_max=2.0)
+    assert rel(to_diff(s2), to_diff(g["sample2"])) < 2e-4
+    s = O.sample_stochastic(cfg, sd, r["sample_shape"], feats, K, rng=synth.gen(r["sample_seed"]), num_steps=r["sample_steps"])
+    assert rel(to_diff(s), to_diff(g["sample"])) < 2e-2
     seed_cloud = O.diffusion_to_data(cfg, sd, torch.randn(r["B"], r["ups_n_seed"], 3, generator=synth.gen(r["ups_seed_cloud_seed"])), K)
     u = O.upsample(cfg, sd, seed_cloud, n_new=r["ups_n_new"], features=feats, K=K, seed=r["ups_seed"],
                    num_substeps=r["ups_substeps"], num_steps=r["ups_steps"])
-    assert rel(to_diff(u), to_diff(g["upsample"])) < 2e-4
+    u_ref = to_diff(g["upsample"])
+    assert (to_diff(u) - u_ref).pow(2).mean().sqrt() < 0.15 * u_ref.pow(2).mean().sqrt()
 
 
 def test_upsample_argument_check():
