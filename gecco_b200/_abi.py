@@ -249,6 +249,18 @@ class UpsampleStepArgs(C.Structure):
     ]
 
 
+CHAMFER_ALL, CHAMFER_PAIRED, CHAMFER_SELF = 0, 1, 2
+
+
+class ChamferArgs(C.Structure):
+    _fields_ = [
+        ("a", C.c_void_p), ("ma", C.c_int32), ("na", C.c_int32),
+        ("b", C.c_void_p), ("mb", C.c_int32), ("nb", C.c_int32),
+        ("mode", C.c_int32),
+        ("out", C.c_void_p),
+    ]
+
+
 class ProfileEntry(C.Structure):
     _fields_ = [("name", C.c_char * 32), ("launches", C.c_int64), ("ms", C.c_double), ("flops", C.c_double),
                 ("bytes", C.c_double)]
@@ -299,6 +311,7 @@ def load() -> C.CDLL:
     lib.gecco_train_colsum2_parts.restype = C.c_int32
     lib.gecco_train_colsum2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     lib.gecco_graph_status.restype = C.c_int
+    lib.gecco_chamfer.argtypes = [C.c_void_p, C.c_void_p]
     _lib = lib
     return lib
 

@@ -498,6 +498,30 @@ int32_t gecco_train_colsum2_parts(int32_t rows_per_cloud, int32_t c);
 int gecco_train_colsum2(const float* dy, const float* x, float* out, int32_t clouds, int32_t rows_per_cloud, int32_t c,
                         void* stream);
 
+/* ------------------------------------------------------------------------
+ * Chamfer distance between point clouds, the distance under the 1-NNA / MMD / COV sample-quality metrics
+ * (gecco_b200/metrics.py; PointFlow's compute_all_metrics protocol; gecco-jax metrics.py has the same role):
+ *   CD(X, Y) = mean_{x in X} min_{y in Y} |x - y|^2 + mean_{y in Y} min_{x in X} |x - y|^2
+ * (squared Euclidean distances, means not sums, no normalisation of the clouds).
+ * a: fp32 [ma, na, 3] contiguous, b: fp32 [mb, nb, 3] contiguous; na, nb >= 1, the smaller of the two at most 32768.
+ * mode GECCO_CHAMFER_ALL   : out [ma, mb], out[i][j] = CD(a[i], b[j]);
+ *      GECCO_CHAMFER_PAIRED: out [ma],     out[i] = CD(a[i], b[i]), ma == mb (bitwise equal to the ALL diagonal);
+ *      GECCO_CHAMFER_SELF  : out [ma, ma], CD(a[i], a[j]); b is NULL or a; each pair i < j is computed once and written to
+ *                            both halves (exactly symmetric), the diagonal is exactly 0.
+ * One block per cloud pair, both directions in one pass; results are bitwise deterministic.  Non-finite points are not
+ * detected here (the minima would silently skip NaN): the caller checks its input.
+ * ------------------------------------------------------------------------ */
+#define GECCO_CHAMFER_ALL 0
+#define GECCO_CHAMFER_PAIRED 1
+#define GECCO_CHAMFER_SELF 2
+typedef struct gecco_chamfer_args {
+  const float* a; int32_t ma, na;
+  const float* b; int32_t mb, nb;
+  int32_t mode;
+  float* out;
+} gecco_chamfer_args;
+int gecco_chamfer(const gecco_chamfer_args* args, void* stream);
+
 /* Per-kernel-class device timing of the engine (tracing aid; the reference has none, SURVEY.md §5).  Between
  * start and stop every engine launch on this thread is bracketed by CUDA events on its stream; stop synchronises
  * the device and returns, per class, the launch count, summed device time and the algorithmic FLOPs / bytes. */
