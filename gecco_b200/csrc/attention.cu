@@ -445,17 +445,8 @@ static int launch_unpool_t(const gecco_unpool_args& a, cudaStream_t s) {
   return GECCO_OK;
 }
 
-// GECCO_UNPOOL_TC=0 keeps the mma.sync kernel even where the tcgen05 kernel applies (A/B measurements).
-static bool unpool_tc_enabled() {
-  static const bool on = [] {
-    const char* v = getenv("GECCO_UNPOOL_TC");
-    return !(v != nullptr && v[0] == '0');
-  }();
-  return on;
-}
-
 int launch_unpool_attention(const gecco_unpool_args& a, cudaStream_t s) {
-  if (unpool_tc_enabled() && unpool_tc_supported(a)) return launch_unpool_tc(a, s);
+  if (unpool_tc_supported(a)) return launch_unpool_tc(a, s);
   GECCO_REQUIRE(a.inducers == NI, "unpool attention: only 64 inducers are supported (got %d)", a.inducers);
   GECCO_REQUIRE(a.rows_per_cloud % 128 == 0, "unpool attention: rows_per_cloud must be a multiple of 128");
   GECCO_REQUIRE(a.ldq % 8 == 0 && a.ldkv % 8 == 0 && a.ldo % 8 == 0 && a.v_off % 8 == 0, "unpool attention: misaligned layout");

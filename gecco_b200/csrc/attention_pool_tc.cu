@@ -29,8 +29,6 @@
 #include "kernels.cuh"
 #include "ptx.cuh"
 
-#include <stdlib.h>
-
 namespace gecco {
 namespace {
 
@@ -67,7 +65,6 @@ struct PParams {
   int clouds, rows_per_cloud, valid_rows;
   int tiles, splits, tps;      // 128-point tiles per cloud, key splits, tiles per split
   int items;                   // clouds * NP * splits
-  int rev;                     // walk the clouds backwards (GECCO_POOL_REV)
   float* partial;              // [cloud][head][split][64][HD + 2] (splits > 1)
   __nv_bfloat16* out;          // [clouds * 64, ldo] (splits == 1)
   long long ldo;
@@ -83,7 +80,6 @@ struct Cursor {
     split = item % p.splits;
     pair = (item / p.splits) % NP;
     cloud = item / (p.splits * NP);
-    if (p.rev) cloud = p.clouds - 1 - cloud;  // last clouds first: the projection before this kernel wrote them last (L2)
     tile = split * p.tps;
     tile_end = min(p.tiles, tile + p.tps);
   }
@@ -484,16 +480,12 @@ int launch_pool_tc(const gecco_pool_args& a, cudaStream_t stream, int* splits_us
   const int sms = sm_count();
   // key splits: enough (cloud, pair, split) items for the 2 x SMs warpgroup slots, bounded by the caller's partial buffer
   int splits = (2 * sms) / (a.clouds * NP);
-  if (const char* v = getenv("GECCO_POOL_TC_SPLITS")) splits = atoi(v);  // development aid
   if (splits > a.splits) splits = a.splits;
   if (splits > p.tiles) splits = p.tiles;
   if (splits < 1 || a.partial == nullptr) splits = 1;
   p.tps = ceil_div(p.tiles, splits);
   p.splits = ceil_div(p.tiles, p.tps);
   p.items = a.clouds * NP * p.splits;
-  static int rev = -1;
-  if (rev < 0) { const char* v = getenv("GECCO_POOL_REV"); rev = v ? atoi(v) : 0; }
-  p.rev = rev;
   p.partial = a.partial;
   p.out = static_cast<__nv_bfloat16*>(a.out_bf16);
   p.ldo = a.ldo;

@@ -45,7 +45,6 @@ static_assert(SMEM_BYTES <= 232448, "shared memory budget");
 
 struct UParams {
   int tiles_per_cloud, num_tiles, tiles_per_cta;
-  int hints;  // GECCO_HINT_UNPOOL: L2 residency hints, bits 0-1 q loads, 6-7 y stores
 };
 
 __device__ __forceinline__ float ex2f(float x) {
@@ -141,7 +140,7 @@ unpool_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
         const uint32_t slot = g % QSLOTS, use = g / QSLOTS;
         mbar_wait(&q_empty[slot], (use & 1u) ^ 1u);
         mbar_arrive_expect_tx(&q_full[slot], Q_SLOT_BYTES);
-        tma_load_2d_h(sQ + slot * Q_SLOT_BYTES, &tma_q, &q_full[slot], h * HD, t * TM, l2_policy(p.hints & 3));  // columns past 384 are zero-filled
+        tma_load_2d(sQ + slot * Q_SLOT_BYTES, &tma_q, &q_full[slot], h * HD, t * TM);  // columns past 384 are zero-filled
       }
     }
   } else if (uwarp == 1) {
@@ -238,7 +237,7 @@ unpool_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
       fence_proxy_async_smem();
       named_bar_sync(1 + w, 128);
       if (storer) {
-        tma_store_2d_addr_h(&tma_y, smem_u32(y_stage), h_of * HD, t_of * TM, l2_policy((p.hints >> 6) & 3));
+        tma_store_2d_addr(&tma_y, smem_u32(y_stage), h_of * HD, t_of * TM);
         tma_store_commit();
       }
     };
@@ -344,7 +343,7 @@ int launch_unpool_tc(const gecco_unpool_args& a, cudaStream_t stream) {
   const long long rows = (long long)a.clouds * a.rows_per_cloud;
   __nv_bfloat16* vt = static_cast<__nv_bfloat16*>(a.vt_scratch);
   if (!a.vt_ready) {
-    launch_pdl(transpose_v_kernel, dim3(a.clouds, 2), dim3(256), 0, stream, static_cast<const __nv_bfloat16*>(a.kv), a.ldkv, a.v_off, vt);
+    launch_small(transpose_v_kernel, dim3(a.clouds, 2), dim3(256), 0, stream, static_cast<const __nv_bfloat16*>(a.kv), a.ldkv, a.v_off, vt);
     GECCO_CHECK_LAUNCH("transpose_v_kernel");
   }
 
@@ -359,9 +358,6 @@ int launch_unpool_tc(const gecco_unpool_args& a, cudaStream_t stream) {
   p.num_tiles = a.clouds * p.tiles_per_cloud;
   const int sms = sm_count();
   p.tiles_per_cta = ceil_div(p.num_tiles, sms);
-  static int hints = -1;
-  if (hints < 0) { const char* v = getenv("GECCO_HINT_UNPOOL"); hints = v ? atoi(v) : 0; }
-  p.hints = hints;
   const int grid = ceil_div(p.num_tiles, p.tiles_per_cta);
 
   static bool attr_set = false;

@@ -36,27 +36,19 @@ extern thread_local long long g_launches;
 
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
-// Programmatic dependent launch of the SMALL kernels (folds, AdaGN apply, lookup, head, ...) is opt-in
-// (GECCO_SMALL_PDL=1): measured A/B on one B200 it LOSES 2 % of the sampler step (595-599 against 585-586 ms) -- the
-// dependents that become resident early are the persistent one-CTA-per-SM GEMMs, which then sit on the SMs' shared
-// memory while the small kernel is still running.  The tcgen05 kernels keep their own PDL launches.
-bool small_kernel_pdl_enabled();
-
-// Launch helper of the small kernels.  With the attribute the kernel may become resident while its predecessor drains;
-// every kernel launched through it starts with griddepcontrol.wait (pdl_wait(), ptx.cuh) before it touches global memory,
-// so ordering stays transitive along the stream; launched plainly the instruction is a no-op.
+// Launch helper of the small kernels (folds, AdaGN apply, lookup, head, ...): a plain launch, without programmatic
+// dependent launch.  Measured A/B on one B200, launching them with the attribute LOSES 2 % of the sampler step (595-599
+// against 585-586 ms): the dependents that become resident early are the persistent one-CTA-per-SM GEMMs, which then sit
+// on the SMs' shared memory while the small kernel is still running.  The tcgen05 kernels keep their own PDL launches,
+// and the small kernels keep griddepcontrol.wait / launch_dependents (pdl_wait(), ptx.cuh): a tcgen05 kernel that
+// follows one relies on the trigger, and without the attribute the wait is a no-op.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
+inline cudaError_t launch_small(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = small_kernel_pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -1,8 +1,6 @@
 // Library-wide state of the C ABI: error text, device checks.
 #include "common.cuh"
 
-#include <stdlib.h>
-
 #include <string.h>
 
 namespace gecco {
@@ -32,14 +30,6 @@ int sm_count() {
 int resolve_driver();
 
 thread_local long long g_launches = 0;
-
-bool small_kernel_pdl_enabled() {
-  static const bool on = [] {
-    const char* v = getenv("GECCO_SMALL_PDL");
-    return v != nullptr && v[0] == '1';
-  }();
-  return on;
-}
 
 }  // namespace gecco
 

@@ -668,9 +668,9 @@ int launch_adagn(const gecco_adagn_args& a, cudaStream_t s) {
   GECCO_REQUIRE(a.ldx % 4 == 0 && (!a.out_bf16 || a.ldo16 % 4 == 0) && (!a.out_f32 || a.ldo32 % 4 == 0), "adagn: bad leading dimension");
   dim3 grid(ceil_div(a.rows_per_cloud, ADAGN_ROWS), a.clouds);
   const int threads = a.c / 4 < 256 ? ((a.c / 4 + 31) / 32) * 32 : 256;
-  launch_pdl(adagn_apply_kernel, grid, dim3(threads), 0, s, a.x, a.ldx, a.stats, a.stat_gs, a.t, a.t_stride, a.ctx_dim, a.scale_w,
-             a.scale_b, a.bias_w, a.bias_b, a.rows_per_cloud, a.valid_rows, a.c, a.groups, a.eps,
-             static_cast<__nv_bfloat16*>(a.out_bf16), a.ldo16, a.out_f32, a.ldo32);
+  launch_small(adagn_apply_kernel, grid, dim3(threads), 0, s, a.x, a.ldx, a.stats, a.stat_gs, a.t, a.t_stride, a.ctx_dim, a.scale_w,
+               a.scale_b, a.bias_w, a.bias_b, a.rows_per_cloud, a.valid_rows, a.c, a.groups, a.eps,
+               static_cast<__nv_bfloat16*>(a.out_bf16), a.ldo16, a.out_f32, a.ldo32);
   GECCO_CHECK_LAUNCH("adagn_apply_kernel");
   return GECCO_OK;
 }
@@ -688,15 +688,15 @@ int launch_fold_adagn(const gecco_fold_adagn_args& a, cudaStream_t s) {
   const char* ffv = getenv("GECCO_FOLD_FAST");  // GECCO_FOLD_FAST=0: the generic kernel (A/B measurements, tests)
   const bool fast_ok = !(ffv != nullptr && ffv[0] == '0');
   if (fast_ok && a.c == 384) {
-    launch_pdl(fold_adagn_fast_kernel<3>, grid, dim3(FOLD_THREADS), smem, s, a.w, a.ldw, a.bias, a.n_out, a.stats, a.stat_gs, a.groups,
-               (double)a.valid_rows * (a.c / a.groups), a.eps, a.t, a.t_stride, a.scale_w, a.scale_b, a.bias_w, a.bias_b,
-               a.clouds, static_cast<__nv_bfloat16*>(a.w_folded_bf16), a.ldwf, a.wf_cloud_stride, a.bias_folded, a.bias_stride);
+    launch_small(fold_adagn_fast_kernel<3>, grid, dim3(FOLD_THREADS), smem, s, a.w, a.ldw, a.bias, a.n_out, a.stats, a.stat_gs, a.groups,
+                 (double)a.valid_rows * (a.c / a.groups), a.eps, a.t, a.t_stride, a.scale_w, a.scale_b, a.bias_w, a.bias_b,
+                 a.clouds, static_cast<__nv_bfloat16*>(a.w_folded_bf16), a.ldwf, a.wf_cloud_stride, a.bias_folded, a.bias_stride);
     GECCO_CHECK_LAUNCH("fold_adagn_fast_kernel");
     return GECCO_OK;
   }
-  launch_pdl(fold_adagn_kernel, grid, dim3(FOLD_THREADS), smem, s, a.w, a.ldw, a.bias, a.n_out, a.c, a.stats, a.stat_gs, a.groups,
-             (double)a.valid_rows * (a.c / a.groups), a.eps, a.t, a.t_stride, a.scale_w, a.scale_b, a.bias_w, a.bias_b,
-             a.clouds, static_cast<__nv_bfloat16*>(a.w_folded_bf16), a.ldwf, a.wf_cloud_stride, a.bias_folded, a.bias_stride);
+  launch_small(fold_adagn_kernel, grid, dim3(FOLD_THREADS), smem, s, a.w, a.ldw, a.bias, a.n_out, a.c, a.stats, a.stat_gs, a.groups,
+               (double)a.valid_rows * (a.c / a.groups), a.eps, a.t, a.t_stride, a.scale_w, a.scale_b, a.bias_w, a.bias_b,
+               a.clouds, static_cast<__nv_bfloat16*>(a.w_folded_bf16), a.ldwf, a.wf_cloud_stride, a.bias_folded, a.bias_stride);
   GECCO_CHECK_LAUNCH("fold_adagn_kernel");
   return GECCO_OK;
 }
@@ -727,7 +727,7 @@ int launch_head(const gecco_head_args& a, cudaStream_t s) {
   dim3 grid(ceil_div(a.valid_rows, HEAD_WARPS * HEAD_ROWS_PER_WARP), a.clouds);
   const size_t sm = a.norm == 2 ? a.groups * 2 * sizeof(float) : 0;
   switch (a.c / 128) {
-#define GECCO_HEAD_CASE(NQ) case NQ: launch_pdl(head_kernel<NQ>, grid, dim3(HEAD_WARPS * 32), sm, s, a); break;
+#define GECCO_HEAD_CASE(NQ) case NQ: launch_small(head_kernel<NQ>, grid, dim3(HEAD_WARPS * 32), sm, s, a); break;
     GECCO_HEAD_CASE(1) GECCO_HEAD_CASE(2) GECCO_HEAD_CASE(3) GECCO_HEAD_CASE(4)
     GECCO_HEAD_CASE(5) GECCO_HEAD_CASE(6) GECCO_HEAD_CASE(7) GECCO_HEAD_CASE(8)
 #undef GECCO_HEAD_CASE

@@ -261,50 +261,16 @@ gecco_fold_adagn_args fold_base(const gecco_engine* e, const float* const* nw /*
   return a;
 }
 
-// GECCO_FUSED_MLP=1 routes the point-side MLP through the single fused kernel (mlp_fused.cu).  Off by default: at the
-// bench shape the fused kernel (446 us / layer) is still slower than the two pair GEMMs (253 us / layer), see DESIGN.md.
-// gecco_set_option("anorm", 0) / GECCO_ANORM=0 keeps the AdaGN -> per-cloud weight fold path everywhere (A/B measurements,
-// tests of the fold path at shapes where the A-operand transform would otherwise be taken).
+// gecco_set_option("anorm", 0) keeps the AdaGN -> per-cloud weight fold path everywhere (A/B measurements, tests of the
+// fold path at shapes where the A-operand transform would otherwise be taken).
 // (Measured and dropped: reading the fp32 stream instead of its bf16 copy -- through a TMA staging ring or straight from
 // global memory in the normalising warps -- saves the producers' bf16 write but starves the resident-tile pipeline: the
 // k|v|q projection went from 143 to 170-250 us.)
-int g_anorm_enabled = -1;
-int anorm_mode() {
-  if (g_anorm_enabled < 0) {
-    const char* v = getenv("GECCO_ANORM");
-    g_anorm_enabled = (v != nullptr && v[0] == '0') ? 0 : 1;
-  }
-  return g_anorm_enabled;
-}
-bool anorm_enabled() { return anorm_mode() != 0; }
-
-// gecco_set_option("chain", 0) / GECCO_CHAIN=0: the inducer side as separate GEMM / AdaGN launches (A/B measurements, tests)
-int g_chain_enabled = -1;
-bool chain_enabled() {
-  if (g_chain_enabled < 0) {
-    const char* v = getenv("GECCO_CHAIN");
-    g_chain_enabled = (v != nullptr && v[0] == '0') ? 0 : 1;
-  }
-  return g_chain_enabled != 0;
-}
-
-// gecco_set_option("mlp_pair", 0) / GECCO_MLP_PAIR=0: the point-side MLP as two GEMMs with the hidden tensor in HBM
-int g_mlp_pair_enabled = -1;
-bool mlp_pair_enabled() {
-  if (g_mlp_pair_enabled < 0) {
-    const char* v = getenv("GECCO_MLP_PAIR");
-    g_mlp_pair_enabled = (v != nullptr && v[0] == '0') ? 0 : 1;
-  }
-  return g_mlp_pair_enabled != 0;
-}
-
-bool fused_mlp_enabled() {
-  static const bool on = [] {
-    const char* v = getenv("GECCO_FUSED_MLP");
-    return v != nullptr && v[0] == '1';
-  }();
-  return on;
-}
+int g_anorm = 1;
+// gecco_set_option("chain", 0): the inducer side as separate GEMM / AdaGN launches (A/B measurements, tests)
+int g_chain = 1;
+// gecco_set_option("mlp_pair", 0): the point-side MLP as two GEMMs with the hidden tensor in HBM
+int g_mlp_pair = 1;
 
 #define TRY(expr)            \
   do {                       \
@@ -346,9 +312,8 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
   double* img_stats = head_stats + per_norm;
   // AdaGN on the point side: normalised inside the consuming GEMM (A-operand transform of the CTA-pair kernel) where
   // the shape allows, else folded into per-cloud weights (fold_adagn + bf16 copy xb of the residual stream).
-  const bool an = anorm_enabled() && !fused_mlp_enabled() && gemm_anorm_supported(rows, Np, C, C) &&
-                  gemm_anorm_supported(rows, Np, 3 * C, C) && gemm_anorm_supported(rows, Np, hid, C);
-  constexpr bool an32 = false;
+  const bool an = g_anorm && gemm_anorm_supported(rows, Np, C, C) && gemm_anorm_supported(rows, Np, 3 * C, C) &&
+                  gemm_anorm_supported(rows, Np, hid, C);
   __nv_bfloat16* const xb_out = w.xb;  // bf16 copy of the residual stream: the (un-normalised) operand of both paths
   auto set_anorm = [&](gecco_gemm_args& g, const float* const* nw, const double* st) {
     g.anorm.stats = st; g.anorm.stat_gs = C / sg; g.anorm.groups = sg; g.anorm.eps = 1e-5f;
@@ -363,8 +328,8 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     if (blocks > 1024) blocks = 1024;
     if ((long long)blocks * threads < clouds) blocks = ceil_div(clouds, threads);
     prof_begin(K_PREP, 0, 8.0 * w.n_stats, s);
-    launch_pdl(prep_kernel, dim3(blocks), dim3(threads), 0, s, w.stats, w.n_stats, sigma, sigma_stride, sigma_imm, t_embed, t_stride,
-               clouds, w.sigma_eff, w.c_noise);
+    launch_small(prep_kernel, dim3(blocks), dim3(threads), 0, s, w.stats, w.n_stats, sigma, sigma_stride, sigma_imm, t_embed, t_stride,
+                 clouds, w.sigma_eff, w.c_noise);
     prof_end(s);
     GECCO_CHECK_LAUNCH("prep_kernel");
   }
@@ -428,7 +393,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       set_anorm(g, lw + GECCO_LW_BN, stat(l, 0));
       g.bias = L.bcat + r0; g.bias_stride = 0;
       g.out_bf16 = w.big + r0; g.ldo16 = C3;
-      TRYP(K_GEMM_KVQ, 2 * Mv * Cd * (C3 - r0), Mv * (Cd * (an32 ? 4 : 2) + (C3 - r0) * 2.0) + 2.0 * (C3 - r0) * Cd, launch_gemm(g, s));
+      TRYP(K_GEMM_KVQ, 2 * Mv * Cd * (C3 - r0), Mv * (Cd * 2 + (C3 - r0) * 2.0) + 2.0 * (C3 - r0) * Cd, launch_gemm(g, s));
     } else {
       gecco_fold_adagn_args f = fold_base(e, lw + GECCO_LW_BN, stat(l, 0), w.c_noise, clouds, points);
       f.w = L.wcat + (size_t)r0 * C; f.ldw = C; f.bias = L.bcat + r0; f.n_out = C3 - r0;
@@ -462,7 +427,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     __nv_bfloat16* khv_l = kvc ? kvc->khv + (size_t)l * irows * 2 * C : w.khv;
     __nv_bfloat16* vt_l = kvc ? kvc->vt + (size_t)l * irows * C : w.vt;
     ch.hn = w.hn; ch.hh = w.hh; ch.h3 = w.h3; ch.khv = khv_l; ch.vt = vt_l;
-    const bool chain = chain_enabled() && inducer_chain_supported(ch);
+    const bool chain = g_chain && inducer_chain_supported(ch);
     bool kv_done = false;
     if (pooling && chain) {
       int nsplit = 1;
@@ -536,7 +501,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
       g.out_bf16 = xb_out; g.ldo16 = C;
       g.stats = stat(l, 3);
-      TRYP(K_GEMM_UNPOOL_OUT, 2 * Mv * Cd * Cd, Mv * Cd * (an32 ? 10 : 12) + 2 * Cd * Cd, launch_gemm(g, s));
+      TRYP(K_GEMM_UNPOOL_OUT, 2 * Mv * Cd * Cd, Mv * Cd * 12 + 2 * Cd * Cd, launch_gemm(g, s));
     }
     // x = x + mlp(AdaGN_mlp(x, t))  (:165-166): mlp_norm folded into mlp.0; statistics for the next broadcast_norm /
     // the head norm
@@ -556,7 +521,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       mp.anorm.bias_w = lw[GECCO_LW_MN + 2]; mp.anorm.bias_b = lw[GECCO_LW_MN + 3];
       mp.scratch = w.big;  // k | v | q of this layer have been consumed
     }
-    if (an && mlp_pair_enabled() && mlp_pair_supported(mp)) {
+    if (an && g_mlp_pair && mlp_pair_supported(mp)) {
       // one kernel: AdaGN on the A operand, the hidden tile of a row block parked in L2 between the products (mlp_pair.cu)
       TRYP(K_MLP_FUSED, 4 * Mv * Cd * Hd, Mv * Cd * 12 + 4 * Cd * Hd, launch_mlp_pair(mp, s));
     } else if (an) {
@@ -564,44 +529,30 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       set_anorm(g, lw + GECCO_LW_MN, stat(l, 3));
       g.bias = lw[GECCO_LW_MLP_B0]; g.bias_stride = 0; g.act = 1; g.act_alpha = L.mlp_alpha;
       g.out_bf16 = w.big; g.ldo16 = hid;
-      TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd * (an32 ? 4 : 2) + Hd * 2) + 2.0 * Cd * Hd, launch_gemm(g, s));
+      TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd * 2 + Hd * 2) + 2.0 * Cd * Hd, launch_gemm(g, s));
       g = gemm_base(w.big, hid, L.mlp_w2, hid, rows, C, hid, Np, points);
       g.bias = lw[GECCO_LW_MLP_B2];
       g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
       g.out_bf16 = xb_out; g.ldo16 = C;
       g.stats = next_stats;
-      TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * (an32 ? 8 : 10)) + 2 * Cd * Hd, launch_gemm(g, s));
+      TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * 10) + 2 * Cd * Hd, launch_gemm(g, s));
     } else {
       gecco_fold_adagn_args f = fold_base(e, lw + GECCO_LW_MN, stat(l, 3), w.c_noise, clouds, points);
       f.w = lw[GECCO_LW_MLP_W0]; f.ldw = C; f.bias = lw[GECCO_LW_MLP_B0]; f.n_out = hid;
       f.w_folded_bf16 = w.wfold; f.ldwf = C; f.wf_cloud_stride = (long long)hid * C;
       f.bias_folded = w.bfold; f.bias_stride = hid;
       TRYP(K_FOLD_ADAGN, 2.0 * clouds * Hd * Cd, Hd * Cd * (4.0 + 2.0 * clouds), launch_fold_adagn(f, s));
-      gecco_mlp_args m = {};
-      m.a = w.xb; m.lda = C;
-      m.w1 = w.wfold; m.ldw1 = C; m.w1_rows_per_cloud = hid;
-      m.b1 = w.bfold; m.b1_stride = hid;
-      m.act_alpha = L.mlp_alpha;
-      m.w2 = L.mlp_w2; m.ldw2 = hid; m.b2 = lw[GECCO_LW_MLP_B2];
-      m.m = rows; m.c = C; m.hidden = hid; m.rows_per_cloud = Np; m.valid_rows = points;
-      m.res = w.x; m.ldr = C; m.out_f32 = w.x; m.ldo32 = C; m.out_bf16 = w.xb; m.ldo16 = C;
-      m.stats = next_stats;
-      if (fused_mlp_enabled() && mlp_fused_supported(m)) {
-        // one kernel, hidden activation on chip (mlp_fused.cu)
-        TRYP(K_MLP_FUSED, 4 * Mv * Cd * Hd, Mv * Cd * 12 + 2.0 * clouds * Cd * Hd + 2 * Cd * Hd, launch_mlp_fused(m, s));
-      } else {
-        gecco_gemm_args g = gemm_base(w.xb, C, w.wfold, C, rows, hid, C, Np, points);
-        g.w_rows_per_cloud = hid;
-        g.bias = w.bfold; g.bias_stride = hid; g.act = 1; g.act_alpha = L.mlp_alpha;
-        g.out_bf16 = w.big; g.ldo16 = hid;
-        TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd + Hd) * 2 + 2.0 * clouds * Cd * Hd, launch_gemm(g, s));
-        g = gemm_base(w.big, hid, L.mlp_w2, hid, rows, C, hid, Np, points);
-        g.bias = lw[GECCO_LW_MLP_B2];
-        g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
-        g.out_bf16 = w.xb; g.ldo16 = C;
-        g.stats = next_stats;
-        TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * 10) + 2 * Cd * Hd, launch_gemm(g, s));
-      }
+      gecco_gemm_args g = gemm_base(w.xb, C, w.wfold, C, rows, hid, C, Np, points);
+      g.w_rows_per_cloud = hid;
+      g.bias = w.bfold; g.bias_stride = hid; g.act = 1; g.act_alpha = L.mlp_alpha;
+      g.out_bf16 = w.big; g.ldo16 = hid;
+      TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd + Hd) * 2 + 2.0 * clouds * Cd * Hd, launch_gemm(g, s));
+      g = gemm_base(w.big, hid, L.mlp_w2, hid, rows, C, hid, Np, points);
+      g.bias = lw[GECCO_LW_MLP_B2];
+      g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
+      g.out_bf16 = w.xb; g.ldo16 = C;
+      g.stats = next_stats;
+      TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * 10) + 2 * Cd * Hd, launch_gemm(g, s));
     }
   }
 
@@ -842,8 +793,8 @@ std::vector<unsigned char> sample_key(const gecco_sample_args* a) {
   put(&a->latents, sizeof(void*)); put(&a->noise, sizeof(void*)); put(&a->x_out, sizeof(void*));
   put(&a->ctx, sizeof(gecco_context));
   put(&a->workspace, sizeof(void*)); put(&a->workspace_bytes, sizeof(int64_t));
-  const int fused = (fused_mlp_enabled() ? 1 : 0) | (anorm_mode() << 1) | ((chain_enabled() ? 1 : 0) << 2) | ((mlp_pair_enabled() ? 1 : 0) << 3);
-  put(&fused, sizeof(int));
+  const int options = g_anorm | (g_chain << 1) | (g_mlp_pair << 2);
+  put(&options, sizeof(int));
   return k;
 }
 
@@ -857,9 +808,9 @@ void drop_graph(gecco_engine* e, size_t i) {
 
 }  // namespace
 void set_graphs_option(int value) { g_graphs_enabled = value != 0 ? 1 : 0; }
-void set_anorm_option(int value) { g_anorm_enabled = value != 0 ? 1 : 0; }
-void set_chain_option(int value) { g_chain_enabled = value != 0 ? 1 : 0; }
-void set_mlp_pair_option(int value) { g_mlp_pair_enabled = value != 0 ? 1 : 0; }
+void set_anorm_option(int value) { g_anorm = value != 0 ? 1 : 0; }
+void set_chain_option(int value) { g_chain = value != 0 ? 1 : 0; }
+void set_mlp_pair_option(int value) { g_mlp_pair = value != 0 ? 1 : 0; }
 }  // namespace gecco
 
 namespace gecco {
@@ -992,7 +943,7 @@ extern "C" int gecco_upsample_step(gecco_engine* e, const gecco_upsample_step_ar
   std::vector<unsigned char> key(sizeof(gecco_upsample_step_args) + 8);
   memcpy(key.data(), a, sizeof(gecco_upsample_step_args));
   memcpy(key.data() + sizeof(gecco_upsample_step_args), "upsample", 8);
-  key.push_back((unsigned char)((fused_mlp_enabled() ? 1 : 0) | (anorm_mode() << 1) | ((chain_enabled() ? 1 : 0) << 2) | ((mlp_pair_enabled() ? 1 : 0) << 3)));
+  key.push_back((unsigned char)(g_anorm | (g_chain << 1) | (g_mlp_pair << 2)));
   return run_graphed(e, key, static_cast<cudaStream_t>(stream), [&](cudaStream_t s) { return enqueue_upsample_step(e, a, s); });
 }
 
@@ -1007,7 +958,6 @@ int enqueue_upsample_step(gecco_engine* e, const gecco_upsample_step_args* a, cu
   KvCache kv_write = {reinterpret_cast<__nv_bfloat16*>(base + u.khv_off), reinterpret_cast<__nv_bfloat16*>(base + u.vt_off), 1};
   KvCache kv_read = kv_write;
   kv_read.mode = 2;
-  if (getenv("GECCO_UPSAMPLE_KV") != nullptr && getenv("GECCO_UPSAMPLE_KV")[0] == '0') kv_read.mode = 0;  // A/B: re-project per evaluation
   const long long ns = (long long)a->clouds * a->seed_points * 3, n3 = (long long)a->clouds * a->new_points * 3;
   // data_ctx = data + randn * t_cur; full evaluation on the seed cloud, inducer states cached (:430-437)
   TRY(launch_seed_renoise(a->seed_data, a->seed_noise, (float)a->t_cur, ns, seed_in, s));

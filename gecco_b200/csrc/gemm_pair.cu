@@ -17,7 +17,6 @@
 // per-cloud per-channel a = scale(t) * rstd_g, s = bias(t) - a * mean_g from the group statistics, computed one row
 // block ahead) and hand it to the MMA issuer.  No normalised tensor and no per-cloud folded weights exist in HBM.
 #include "common.cuh"
-#include <stdlib.h>
 #include "debug_api.h"
 #include "epilogue.cuh"
 #include "kernels.cuh"
@@ -47,6 +46,10 @@ constexpr int SMEM_FIXED = MAX_KB * A_KB_BYTES + 1024 /*align*/ + 512 /*barriers
 constexpr int NORM_BYTES = 2 * 2 * MAX_KB * BK * 4;  // a[K], s[K], double buffered over row blocks
 constexpr int ANORM_SMEM = NORM_BYTES;
 constexpr int XF_THREADS = 64;              // warps 2 and 3
+// L2 residency hints per launch class (bits 0-1 A loads, 2-3 residual loads, 4-5 fp32 stores, 6-7 bf16 stores; ptx.cuh
+// l2_policy kinds)
+constexpr int HINTS_RESIDUAL_PROJ = 160;  // residual projections (unpool out-proj): both outputs evict_last, the MLP reads them next
+constexpr int HINTS_OTHER_PROJ = 0;       // normalising (k|v|q) and plain projections
 
 struct PParams {
   EpiParams e;
@@ -61,12 +64,9 @@ struct PParams {
   const float *n_scale_w, *n_scale_b, *n_bias_w, *n_bias_b;
   int K;
   int a_hint;  // L2 residency hint of the A-operand loads (ptx.cuh l2_policy kinds)
-  int rev;  // row blocks are walked from the end (the previous kernel's last writes are read first, while still in L2)
 };
 
 __device__ __forceinline__ int num_kb_of(const PParams& p) { return p.num_kb; }
-// physical row block of the pb-th one this pair processes
-#define RB(pb) (p.rev ? p.num_pair_blocks - 1 - (pb) : (pb))
 
 // cycles spent in a barrier wait, accumulated into `acc` when the debug buffer is set
 #define TIMED_WAIT(acc, bar, parity)        \
@@ -159,7 +159,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();
   pdl_launch_dependents();
-  // warps 0-3 (TMA / MMA / allocator / residual loader: a handful of registers) hand their registers to the epilogue
 
   // warps 0-3 (TMA / MMA / allocator / residual loader: a handful of registers) hand their registers to the epilogue
   if (warp < 4) {
@@ -173,7 +172,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     const long long t_start = clock64();
     const uint64_t a_pol = l2_policy(p.a_hint);
     for (int pb = pair; pb < p.num_pair_blocks; pb += num_pairs, ++it) {
-      const int m0 = RB(pb) * 2 * BM + (int)rank * BM;
+      const int m0 = pb * 2 * BM + (int)rank * BM;
       const int cloud_w = p.w_rows_per_cloud ? (m0 / p.e.rows_per_cloud) * p.w_rows_per_cloud : 0;
       for (int nb = 0; nb < p.num_n_blocks; ++nb) {
         const int wrow = cloud_w + nb * BN + (int)rank * BNH;
@@ -271,7 +270,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     // (mean = s1 / n and E[x^2] - mean^2 need the precision, rstd does not) and the statistics loads are issued first.
     const double inv_count = 1.0 / count;
     auto make_norm = [&](int pb, uint32_t buf) {
-      const int m0 = RB(pb) * 2 * BM + (int)rank * BM;
+      const int m0 = pb * 2 * BM + (int)rank * BM;
       const int cloud = m0 / p.e.rows_per_cloud;
       const double* cst = p.n_stats + (long long)cloud * (K / p.n_stat_gs) * 2;
       float* na = sNorm + buf * 2 * MAX_KB * BK;
@@ -363,7 +362,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     if (p.e.has_res && !(p.e.skip & 2)) {
       uint32_t cnt[EPI_GROUPS] = {0, 0};
       for (int pb = pair; pb < p.num_pair_blocks; pb += num_pairs) {
-        const int m0 = RB(pb) * 2 * BM + (int)rank * BM;
+        const int m0 = pb * 2 * BM + (int)rank * BM;
         for (int nb = 0; nb < p.num_n_blocks; ++nb) epi_load_residual_panel(p.e, es, &tma_res, m0, nb * BN, cnt);
       }
     }
@@ -377,9 +376,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     long long w_accfull = 0, w_pref = 0;
     const long long t_start = clock64();
     EpiBias bias_r;
-    if (pair < p.num_pair_blocks) epi_bias_load(p.e, et, RB(pair) * 2 * BM + (int)rank * BM, 0, bias_r);
+    if (pair < p.num_pair_blocks) epi_bias_load(p.e, et, pair * 2 * BM + (int)rank * BM, 0, bias_r);
     for (int pb = pair; pb < p.num_pair_blocks; pb += num_pairs) {
-      const int m0 = RB(pb) * 2 * BM + (int)rank * BM;
+      const int m0 = pb * 2 * BM + (int)rank * BM;
       for (int nb = 0; nb < p.num_n_blocks; ++nb, ++tile) {
         const uint32_t slot = tile & 1u;
         long long tp0 = 0;
@@ -387,7 +386,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         epi_bias_stage(p.e, et, bias_r);
         // the next panel's bias is loaded under this panel
         if (nb + 1 < p.num_n_blocks) epi_bias_load(p.e, et, m0, (nb + 1) * BN, bias_r);
-        else if (pb + num_pairs < p.num_pair_blocks) epi_bias_load(p.e, et, RB(pb + num_pairs) * 2 * BM + (int)rank * BM, 0, bias_r);
+        else if (pb + num_pairs < p.num_pair_blocks) epi_bias_load(p.e, et, (pb + num_pairs) * 2 * BM + (int)rank * BM, 0, bias_r);
         if (GECCO_DBG_ON(p.dbg)) w_pref += clock64() - tp0;
         TIMED_WAIT(w_accfull, &acc_full[slot], (tile >> 1) & 1u);
         tc_fence_after_sync();
@@ -427,25 +426,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 
 }  // namespace
 
-// gecco_set_option("fast_epilogue", 0) / GECCO_FAST_EPILOGUE=0: the generic epilogue everywhere (A/B measurements, tests)
-int g_fast_epilogue = -1;
-bool fast_epilogue_enabled() {
-  if (g_fast_epilogue < 0) {
-    const char* v = getenv("GECCO_FAST_EPILOGUE");
-    g_fast_epilogue = (v != nullptr && v[0] == '0') ? 0 : 1;
-  }
-  return g_fast_epilogue != 0;
-}
-void set_fast_epilogue_option(int value) { g_fast_epilogue = value != 0 ? 1 : 0; }
-
-// GECCO_REV (bit mask): 1 residual projections (unpool out-proj), 4 normalising projections (k|v|q) walk the row blocks backwards
-static int pair_rev(const gecco_gemm_args& a) {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GECCO_REV"); v = e ? atoi(e) : 2; }
-  if (a.res != nullptr) return (v & 1) ? 1 : 0;
-  if (a.anorm.stats != nullptr) return (v & 4) ? 1 : 0;
-  return 0;
-}
+// gecco_set_option("fast_epilogue", 0): the generic epilogue everywhere (A/B measurements, tests)
+static bool g_fast_epilogue = true;
+void set_fast_epilogue_option(int value) { g_fast_epilogue = value != 0; }
 
 bool gemm_pair_shape_ok(int m, int rows_per_cloud, int n_out, int k) {
   if (k > MAX_KB * BK || k % 8 != 0 || m % (2 * BM) != 0 || m < 2 * BM * 8 || sm_count() < 2) return false;
@@ -500,23 +483,14 @@ int launch_gemm_pair(const gecco_gemm_args& a, cudaStream_t stream, int* handled
   p.dbg = g_gemm_debug;
   p.e.dbg = g_gemm_debug;
   p.e.skip = epi_skip_option();
-  {
-    // L2 residency hints per launch class (bits 0-1 A loads, 2-3 residual loads, 4-5 fp32 stores, 6-7 bf16 stores):
-    // GECCO_HINT_OUT residual projections (unpool out-proj), GECCO_HINT_KVQ normalising projections (k|v|q)
-    static int h_out = -1, h_kvq = -1;
-    if (h_out < 0) { const char* e = getenv("GECCO_HINT_OUT"); h_out = e ? atoi(e) : 160; }  // both outputs evict_last: the MLP reads them next
-    if (h_kvq < 0) { const char* e = getenv("GECCO_HINT_KVQ"); h_kvq = e ? atoi(e) : 0; }
-    const int h = a.res != nullptr ? h_out : (a.anorm.stats != nullptr ? h_kvq : 0);
-    p.e.hints = h;
-    p.a_hint = h & 3;
-  }
+  p.e.hints = a.res != nullptr ? HINTS_RESIDUAL_PROJ : HINTS_OTHER_PROJ;
+  p.a_hint = p.e.hints & 3;
   p.n_stats = a.anorm.stats; p.n_stat_gs = a.anorm.stat_gs; p.n_groups = a.anorm.groups; p.n_eps = a.anorm.eps;
   p.n_t = a.anorm.t; p.n_t_stride = a.anorm.t_stride;
   p.n_scale_w = a.anorm.scale_w; p.n_scale_b = a.anorm.scale_b; p.n_bias_w = a.anorm.bias_w; p.n_bias_b = a.anorm.bias_b;
   p.K = a.k;
-  p.rev = pair_rev(a);
   // bf16-only whole-tile projections take the fast epilogue
-  const bool fast = fast_epilogue_enabled() && a.res == nullptr && a.stats == nullptr && a.out_f32 == nullptr && a.geom == nullptr &&
+  const bool fast = g_fast_epilogue && a.res == nullptr && a.stats == nullptr && a.out_f32 == nullptr && a.geom == nullptr &&
                     a.bias != nullptr && a.out_bf16 != nullptr && a.n_out % BN == 0 &&
                     p.e.skip == 0;
   const int epi_bytes = (fast ? epi_fast_smem_bytes() : epi_smem_bytes(p.e.has_res, a.out_f32 != nullptr, a.out_bf16 != nullptr)) +
@@ -525,10 +499,6 @@ int launch_gemm_pair(const gecco_gemm_args& a, cudaStream_t stream, int* handled
   p.kbps = 1;
   for (int cand = p.num_kb; cand > 1; --cand)  // deepest weight stage that still leaves a 3-deep ring
     if (p.num_kb % cand == 0 && avail / (cand * B_STAGE_BYTES) >= 3) { p.kbps = cand; break; }
-  if (const char* v = getenv("GECCO_PAIR_KBPS")) {  // development aid: k-blocks per weight stage
-    const int want = atoi(v);
-    if (want >= 1 && p.num_kb % want == 0 && avail / (want * B_STAGE_BYTES) >= 2) p.kbps = want;
-  }
   p.bstages = avail / (p.kbps * B_STAGE_BYTES);
   if (p.bstages > MAX_BSTAGES) p.bstages = MAX_BSTAGES;
   GECCO_REQUIRE(p.bstages >= 2, "gemm_pair: shared memory budget");

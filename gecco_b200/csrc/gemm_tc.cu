@@ -38,7 +38,6 @@ struct KParams {
   EpiParams e;
   int K, w_rows_per_cloud;
   int num_m_blocks, num_n_blocks;
-  int rev;  // tiles are walked from the end (GECCO_TC_REV: the lookup's last writes are read first, while still in L2)
   int stages;
 };
 
@@ -96,7 +95,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
   // everything above overlaps the tail of the preceding kernel (programmatic dependent launch)
   pdl_wait();
   pdl_launch_dependents();
-  // warps 0-3 (TMA / MMA / allocator / residual loader: a handful of registers) hand their registers to the epilogue
 
   // warps 0-3 (TMA / MMA / allocator / residual loader: a handful of registers) hand their registers to the epilogue
   if (warp < 4) {
@@ -106,9 +104,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     int stage = 0;
     uint32_t phase = 0;
     for (int t = blockIdx.x; t < num_tiles; t += gridDim.x) {
-      const int tt = p.rev ? num_tiles - 1 - t : t;
-      const int m0 = (tt / p.num_n_blocks) * BM;
-      const int n0 = (tt % p.num_n_blocks) * BN;
+      const int m0 = (t / p.num_n_blocks) * BM;
+      const int n0 = (t % p.num_n_blocks) * BN;
       const int wrow = (p.w_rows_per_cloud ? (m0 / p.e.rows_per_cloud) * p.w_rows_per_cloud : 0) + n0;
       for (int kb = 0; kb < num_kb; ++kb) {
         mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -157,9 +154,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     if (p.e.has_res) {
       uint32_t cnt[EPI_GROUPS] = {0, 0};
       for (int t = blockIdx.x; t < num_tiles; t += gridDim.x) {
-        const int tt = p.rev ? num_tiles - 1 - t : t;
-        const int m0 = (tt / p.num_n_blocks) * BM;
-        const int n0 = (tt % p.num_n_blocks) * BN;
+        const int m0 = (t / p.num_n_blocks) * BM;
+        const int n0 = (t % p.num_n_blocks) * BN;
         epi_load_residual_panel(p.e, es, &tma_res, m0, n0, cnt);
       }
     }
@@ -172,22 +168,16 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     int it = 0;
     uint32_t cnt = 0;
     EpiBias bias_r;
-    if ((int)blockIdx.x < num_tiles) {
-      const int t0 = p.rev ? num_tiles - 1 - (int)blockIdx.x : (int)blockIdx.x;
-      epi_bias_load(p.e, et, (t0 / p.num_n_blocks) * BM, (t0 % p.num_n_blocks) * BN, bias_r);
-    }
+    if ((int)blockIdx.x < num_tiles)
+      epi_bias_load(p.e, et, ((int)blockIdx.x / p.num_n_blocks) * BM, ((int)blockIdx.x % p.num_n_blocks) * BN, bias_r);
     for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
       const int slot = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1;
-      const int tt = p.rev ? num_tiles - 1 - t : t;
-      const int m0 = (tt / p.num_n_blocks) * BM;
-      const int n0 = (tt % p.num_n_blocks) * BN;
+      const int m0 = (t / p.num_n_blocks) * BM;
+      const int n0 = (t % p.num_n_blocks) * BN;
       epi_bias_stage(p.e, et, bias_r);
       const int tn = t + gridDim.x;  // the next tile's bias is loaded under this tile
-      if (tn < num_tiles) {
-        const int tnn = p.rev ? num_tiles - 1 - tn : tn;
-        epi_bias_load(p.e, et, (tnn / p.num_n_blocks) * BM, (tnn % p.num_n_blocks) * BN, bias_r);
-      }
+      if (tn < num_tiles) epi_bias_load(p.e, et, (tn / p.num_n_blocks) * BM, (tn % p.num_n_blocks) * BN, bias_r);
       mbar_wait(&acc_full[slot], acc_phase);
       tc_fence_after_sync();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * ACC_COLS;
@@ -365,11 +355,6 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   p.e.skip = 0;
   p.e.hints = 0;
   p.num_m_blocks = ceil_div(a.m, BM);
-  {
-    static int rev = -1;
-    if (rev < 0) { const char* v = getenv("GECCO_TC_REV"); rev = v ? atoi(v) : 0; }
-    p.rev = (rev != 0 && a.geom != nullptr) ? 1 : 0;  // the image-feature projection behind the lookup
-  }
   p.num_n_blocks = ceil_div(a.n_out, BN);
   const int epi_bytes = epi_smem_bytes(p.e.has_res, a.out_f32 != nullptr, a.out_bf16 != nullptr);
   p.stages = (SMEM_LIMIT - SMEM_FIXED - epi_bytes) / (A_STAGE_BYTES + B_STAGE_BYTES);

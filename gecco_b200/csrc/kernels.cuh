@@ -23,12 +23,9 @@ bool g_use_pairs_ref();
 void set_fast_epilogue_option(int value);  // gemm_pair.cu: gecco_set_option("fast_epilogue", v)
 
 int launch_gemm(const gecco_gemm_args& a, cudaStream_t s);
-void set_graphs_option(int value);
+void set_graphs_option(int value);  // engine.cu: gecco_set_option("graphs", v)
 void set_chain_option(int value);  // engine.cu: gecco_set_option("chain", v)
-void set_anorm_option(int value);  // engine.cu: gecco_set_option("anorm", v)  // engine.cu: gecco_set_option("graphs", v)
-// Fused MLP (mlp_fused.cu): GEMM -> Gaussian activation -> GEMM -> + residual with the hidden tensor on chip.
-bool mlp_fused_supported(const gecco_mlp_args& a);
-int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t s);
+void set_anorm_option(int value);  // engine.cu: gecco_set_option("anorm", v)
 // CTA-pair MLP with the hidden tile parked in an L2-resident scratch and AdaGN on the A operand (mlp_pair.cu).
 bool mlp_pair_supported(const gecco_mlp_args& a);
 int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t s);

@@ -288,12 +288,12 @@ __device__ __forceinline__ uint64_t bf16x2_to_f32x2(uint32_t v) {
   return pack_f32x2(__uint_as_float(v << 16), __uint_as_float(v & 0xffff0000u));
 }
 
-// PACKED: blend and statistics on packed fp32x2 arithmetic (FFMA2 / FADD2) instead of scalar FFMA.
+// Blend and statistics run on packed fp32x2 arithmetic (FFMA2 / FADD2).
 // HYBRID: levels flagged in p.glob_mask are too large to stage (256^2 images: the 64 x 64 x 96 level is 786 KB per cloud);
 // their threads gather the four taps from the L2-resident channels-last map instead, with the taps of the NEXT point in
 // flight while the current one is blended, and the other levels still come from shared memory.  The large level is the
 // one with the FEWEST channels, so the global gather shrinks from 4 x 672 to 4 x 96 channels per point.
-template <int UPT, bool PACKED, bool HYBRID = false>
+template <int UPT, bool HYBRID = false>
 __global__ void __launch_bounds__(LS_THREADS, 1) lookup_staged_kernel(const LookupP p, const int S, const int pts_per_cta) {
   extern __shared__ __align__(16) uint8_t lsm[];
   pdl_wait();  // programmatic dependent launch: the predecessor has completed
@@ -475,45 +475,25 @@ __global__ void __launch_bounds__(LS_THREADS, 1) lookup_staged_kernel(const Look
 #pragma unroll
         for (int k = 0; k < UPT; ++k) {
           uint32_t o[4];
-          if (PACKED) {
-            uint64_t acc[4] = {0ull, 0ull, 0ull, 0ull};
+          uint64_t acc[4] = {0ull, 0ull, 0ull, 0ull};
 #pragma unroll
-            for (int t = 0; t < 4; ++t) {
-              const uint64_t ww = pack_f32x2(wt[t], wt[t]);
-              acc[0] = fma_f32x2(bf16x2_to_f32x2(q[t][k].x), ww, acc[0]);
-              acc[1] = fma_f32x2(bf16x2_to_f32x2(q[t][k].y), ww, acc[1]);
-              acc[2] = fma_f32x2(bf16x2_to_f32x2(q[t][k].z), ww, acc[2]);
-              acc[3] = fma_f32x2(bf16x2_to_f32x2(q[t][k].w), ww, acc[3]);
-            }
+          for (int t = 0; t < 4; ++t) {
+            const uint64_t ww = pack_f32x2(wt[t], wt[t]);
+            acc[0] = fma_f32x2(bf16x2_to_f32x2(q[t][k].x), ww, acc[0]);
+            acc[1] = fma_f32x2(bf16x2_to_f32x2(q[t][k].y), ww, acc[1]);
+            acc[2] = fma_f32x2(bf16x2_to_f32x2(q[t][k].z), ww, acc[2]);
+            acc[3] = fma_f32x2(bf16x2_to_f32x2(q[t][k].w), ww, acc[3]);
+          }
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              uint64_t a1 = pack_f32x2(s1[k][2 * j], s1[k][2 * j + 1]), a2 = pack_f32x2(s2[k][2 * j], s2[k][2 * j + 1]);
-              a1 = add_f32x2(a1, acc[j]);
-              a2 = fma_f32x2(acc[j], acc[j], a2);
-              unpack_f32x2(a1, s1[k][2 * j], s1[k][2 * j + 1]);
-              unpack_f32x2(a2, s2[k][2 * j], s2[k][2 * j + 1]);
-              float lo, hi;
-              unpack_f32x2(acc[j], lo, hi);
-              o[j] = pack_bf16x2(lo, hi);
-            }
-          } else {
-            float acc[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) acc[j] = 0.f;
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-              float f[8];
-              bf16x8_to_float(q[t][k], f);
-#pragma unroll
-              for (int j = 0; j < 8; ++j) acc[j] = fmaf(f[j], wt[t], acc[j]);
-            }
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              s1[k][j] += acc[j];
-              s2[k][j] = fmaf(acc[j], acc[j], s2[k][j]);
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j) o[j] = pack_bf16x2(acc[2 * j], acc[2 * j + 1]);
+          for (int j = 0; j < 4; ++j) {
+            uint64_t a1 = pack_f32x2(s1[k][2 * j], s1[k][2 * j + 1]), a2 = pack_f32x2(s2[k][2 * j], s2[k][2 * j + 1]);
+            a1 = add_f32x2(a1, acc[j]);
+            a2 = fma_f32x2(acc[j], acc[j], a2);
+            unpack_f32x2(a1, s1[k][2 * j], s1[k][2 * j + 1]);
+            unpack_f32x2(a2, s2[k][2 * j], s2[k][2 * j + 1]);
+            float lo, hi;
+            unpack_f32x2(acc[j], lo, hi);
+            o[j] = pack_bf16x2(lo, hi);
           }
           *reinterpret_cast<uint4*>(orow + k * kcol) = make_uint4(o[0], o[1], o[2], o[3]);
         }
@@ -583,10 +563,9 @@ StagedPlan plan_staged(const LookupP& p, int stat_groups) {
   // Measured at 64 clouds x 2048 points (tools/lookup_time.py): 137^2 pyramids (S = 2) 105 us against 228 us for the
   // global-gather kernel; 256^2 pyramids need S = 12 (7 threads per point, a tap-table entry per 8 channels) and are
   // slower than the global gather (270 against 236 us), so the automatic choice stops at S = 4.
-  // Hybrid plans (GECCO_LOOKUP_HYBRID=0 disables them): first everything staged; if no S <= 4 fits, the level with the
-  // largest map (the fewest channels in a CNN pyramid) stays in global memory and only the others are staged.
-  const char* hv = getenv("GECCO_LOOKUP_HYBRID");
-  const bool hybrid_ok = !(hv != nullptr && hv[0] == '0') && p.n_levels >= 2;
+  // Hybrid plans: first everything staged; if no S <= 4 fits, the level with the largest map (the fewest channels in a
+  // CNN pyramid) stays in global memory and only the others are staged.
+  const bool hybrid_ok = p.n_levels >= 2;
   int biggest = 0;
   for (int l = 1; l < p.n_levels; ++l)
     if ((size_t)p.lvl_h[l] * p.lvl_w[l] * p.lvl_c[l] > (size_t)p.lvl_h[biggest] * p.lvl_w[biggest] * p.lvl_c[biggest]) biggest = l;
@@ -725,22 +704,18 @@ int launch_lookup(const gecco_lookup_args& a, cudaStream_t s) {
     int per = ceil_div(ceil_div(a.points, z), 32) * 32;
     z = ceil_div(a.points, per);
     dim3 grid(plan.S, a.clouds, z);
-    const char* sc = getenv("GECCO_LOOKUP_SCALAR");  // A/B switch: scalar FFMA instead of packed fp32x2 arithmetic
-    const bool packed = !(sc != nullptr && sc[0] == '1');
     auto go = [&](auto kern, bool& done) {
       if (!done) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LS_SMEM_MAX);
         done = true;
       }
-      launch_pdl(kern, grid, dim3(LS_THREADS), plan.smem, s, p, plan.S, per);
+      launch_small(kern, grid, dim3(LS_THREADS), plan.smem, s, p, plan.S, per);
     };
-    static bool attr_done[6] = {false, false, false, false, false, false};
-    if (plan.glob_mask != 0 && plan.upt == 2) go(lookup_staged_kernel<2, true, true>, attr_done[4]);
-    else if (plan.glob_mask != 0) go(lookup_staged_kernel<1, true, true>, attr_done[5]);
-    else if (plan.upt == 2 && packed) go(lookup_staged_kernel<2, true>, attr_done[0]);
-    else if (plan.upt == 2) go(lookup_staged_kernel<2, false>, attr_done[1]);
-    else if (packed) go(lookup_staged_kernel<1, true>, attr_done[2]);
-    else go(lookup_staged_kernel<1, false>, attr_done[3]);
+    static bool attr_done[4] = {false, false, false, false};
+    if (plan.glob_mask != 0 && plan.upt == 2) go(lookup_staged_kernel<2, true>, attr_done[2]);
+    else if (plan.glob_mask != 0) go(lookup_staged_kernel<1, true>, attr_done[3]);
+    else if (plan.upt == 2) go(lookup_staged_kernel<2>, attr_done[0]);
+    else go(lookup_staged_kernel<1>, attr_done[1]);
     GECCO_CHECK_LAUNCH("lookup_staged_kernel");
     return GECCO_OK;
   }
@@ -760,8 +735,8 @@ int launch_fold_gn(const float* W, const float* bias, const double* stats, doubl
                    int c_in, int c_out, int clouds, void* wb, long long ldwb, float* bb, cudaStream_t s) {
   GECCO_REQUIRE(groups > 0 && groups <= 64 && c_in % groups == 0 && c_in % 2 == 0 && ldwb % 2 == 0, "fold_gn: bad layout");
   dim3 grid(ceil_div(c_out, FGN_ROWS), clouds);
-  launch_pdl(fold_gn_kernel, grid, dim3(128), 0, s, W, bias, stats, count, eps, groups, c_in, c_out, static_cast<__nv_bfloat16*>(wb),
-             ldwb, bb);
+  launch_small(fold_gn_kernel, grid, dim3(128), 0, s, W, bias, stats, count, eps, groups, c_in, c_out, static_cast<__nv_bfloat16*>(wb),
+               ldwb, bb);
   GECCO_CHECK_LAUNCH("fold_gn_kernel");
   return GECCO_OK;
 }

@@ -399,12 +399,12 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 
 }  // namespace
 
-bool mlp_fused_supported(const gecco_mlp_args& a) {
+static bool mlp_fused_supported(const gecco_mlp_args& a) {
   return a.c == C && a.hidden >= HC && a.hidden % HC == 0 && a.m > 0 && a.m % (2 * BM) == 0 &&
          a.rows_per_cloud % (2 * BM) == 0 && sm_count() >= 2;
 }
 
-int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
+static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
   GECCO_REQUIRE(a.a && a.w1 && a.w2 && a.b1 && a.b2, "mlp: null operand");
   GECCO_REQUIRE(a.res && a.out_f32, "mlp: the fp32 residual stream (res, out_f32) is required");
   GECCO_REQUIRE(mlp_fused_supported(a),

@@ -13,14 +13,13 @@
 //
 // The residual epilogue cannot afford the 64 KB of TMA-fed X buffers of epilogue.cuh next to a resident A tile and a weight
 // ring, so here every epilogue WARP owns one 4 KB staging block: the fp32 residual chunk of its 32 rows is fetched with
-// coalesced LDG.128 one chunk ahead (registers are the prefetch buffer; the producer warp pulls the tile into L2 with TMA
-// prefetches at the start of the D phase, so the loads hit L2), written into the block, read back row-per-thread, and
+// coalesced LDG.128 one chunk ahead (registers are the prefetch buffer; the producer warp pulls each output tile's
+// residual into L2 with TMA prefetches in the D phase, so the loads hit L2), written into the block, read back row-per-thread, and
 // the finished rows leave through the same block by one bulk tensor store.  No loader warp, no cross-warp barrier.
 //
 //   warp 0 : TMA producer            warps 2-3 : A-operand transform (AdaGN)
 //   warp 1 : MMA issuer (leader)     warps 4-11: epilogue
 #include "common.cuh"
-#include <stdlib.h>
 #include "debug_api.h"
 #include "epilogue.cuh"
 #include "kernels.cuh"
@@ -64,14 +63,16 @@ struct MParams {
   const float* n_t; int n_t_stride;
   const float *n_scale_w, *n_scale_b, *n_bias_w, *n_bias_b;
   long long* dbg;
-  int hints;  // GECCO_HINT_MLP: L2 residency hints, bits 0-1 A loads, 2-3 residual loads, 4-5 fp32 stores, 6-7 bf16 stores,
-              // 8-9 hidden-scratch stores, 10-11 hidden-scratch loads
-  int rev;    // GECCO_REV & 2: row blocks are walked from the end
-  int respf;  // GECCO_MLP_RESPF (development): 0 residual tile -> L2 at the start of the second product, 1 per output tile, 2 never
 };
 
+// L2 residency policies (ptx.cuh l2_policy kinds): the A operand and the residual are read once (evict_first), the hidden
+// tiles parked in the scratch are read back by the second product (evict_last), the outputs get the default
+constexpr int POL_A = 1, POL_RES = 1, POL_HIDDEN = 2, POL_OUT = 0;
+
+// physical row block of the pb-th one: row blocks are walked from the end, so the previous kernel's last writes are read
+// first, while still in L2
+#define RB(pb) (p.num_pair_blocks - 1 - (pb))
 // development aid: cycles spent in a barrier wait, accumulated when the debug buffer is set (gecco_set_debug_buffer)
-#define RB(pb) (p.rev ? p.num_pair_blocks - 1 - (pb) : (pb))
 #define TW(acc, bar, parity)              \
   do {                                    \
     if (p.dbg != nullptr) {               \
@@ -96,7 +97,7 @@ __device__ __forceinline__ float4 ldg128(const float* p, uint64_t pol) {
 struct ResRegs { float4 r[8]; };
 __device__ __forceinline__ void res_load(const MParams& p, int row0, int col0, int lane, ResRegs& R) {
   const float* base = p.res + (long long)(row0 + (lane >> 3)) * p.ldr + col0 + (lane & 7) * 4;
-  const uint64_t pol = l2_policy((p.hints >> 2) & 3);
+  const uint64_t pol = l2_policy(POL_RES);
 #pragma unroll
   for (int i = 0; i < 8; ++i) R.r[i] = ldg128(base + (long long)(4 * i) * p.ldr, pol);
 }
@@ -193,8 +194,8 @@ __device__ __forceinline__ void epi_panel_ldg(const MParams& p, const EpiThread&
     fence_proxy_async_smem();
     __syncwarp();
     if (elect_one()) {
-      tma_store_2d_addr_h(tma_o32, xs, col0, row0, l2_policy((p.hints >> 4) & 3));
-      tma_store_2d_addr_h(tma_o16, t.s16, col0, row0, l2_policy((p.hints >> 6) & 3));
+      tma_store_2d_addr_h(tma_o32, xs, col0, row0, l2_policy(POL_OUT));
+      tma_store_2d_addr_h(tma_o16, t.s16, col0, row0, l2_policy(POL_OUT));
       tma_store_commit();
     }
   };
@@ -285,7 +286,7 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant
       uint32_t it = 0;
       long long w_b1 = 0, w_a = 0, w_hr = 0, w_hs = 0, w_b2 = 0;
       const long long t_start = clock64();
-      const uint64_t h_pol = l2_policy((p.hints >> 10) & 3);  // hidden k-blocks coming back from the scratch
+      const uint64_t h_pol = l2_policy(POL_HIDDEN);  // hidden k-blocks coming back from the scratch
       for (int pb = pair; pb < p.num_pair_blocks; pb += num_pairs, ++it) {
         const int m0 = RB(pb) * 2 * BM + (int)rank * BM;
         // first product: A k-blocks once per row block, W1 half tiles per (tile, k-block)
@@ -297,24 +298,20 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant
             if (nb == 0) {
               TW(w_a, &a_empty[kb], ((it * 5u) & 1u) ^ 1u);  // fill 5 it of the slot
               mbar_arrive_expect_tx(&a_landed[kb], A_KB_BYTES);
-              tma_load_2d_h(sA + kb * A_KB_BYTES, &tma_a, &a_landed[kb], kb * BK, m0, l2_policy(p.hints & 3));
+              tma_load_2d_h(sA + kb * A_KB_BYTES, &tma_a, &a_landed[kb], kb * BK, m0, l2_policy(POL_A));
             }
             tma_load_2d_pair(sB + stage * B_STAGE_BYTES, &tma_w1, &b_full[stage], kb * BK, wrow);
             if (++stage == BST) { stage = 0; bphase ^= 1u; }
           }
         }
-        // the residual tile of this row block and the A tile of the next one -> L2
-        if ((p.respf & 3) == 0)
-          for (int c = 0; c < C / EPI_CHUNK; ++c) tma_prefetch_l2_2d(&tma_res, c * EPI_CHUNK, m0);
-        if (((p.respf >> 2) & 3) == 0 && pb + num_pairs < p.num_pair_blocks)
+        // the A tile of the next row block -> L2
+        if (pb + num_pairs < p.num_pair_blocks)
           for (int kb = 0; kb < KB1; ++kb) tma_prefetch_l2_2d(&tma_a, kb * BK, RB(pb + num_pairs) * 2 * BM + (int)rank * BM);
         // second product: hidden k-blocks from the scratch through the slots of the A tile, W2 half tiles
         for (int nb = 0; nb < ND; ++nb) {
           const int wrow = nb * BN + (int)rank * BNH;
-          if ((p.respf & 3) == 1)
-            for (int c = 0; c < BN / EPI_CHUNK; ++c) tma_prefetch_l2_2d(&tma_res, nb * BN + c * EPI_CHUNK, m0);
-          if (((p.respf >> 2) & 3) == 1 && nb == ND - 1 && pb + num_pairs < p.num_pair_blocks)
-            for (int kb = 0; kb < KB1; ++kb) tma_prefetch_l2_2d(&tma_a, kb * BK, RB(pb + num_pairs) * 2 * BM + (int)rank * BM);
+          // the residual of this output tile -> L2
+          for (int c = 0; c < BN / EPI_CHUNK; ++c) tma_prefetch_l2_2d(&tma_res, nb * BN + c * EPI_CHUNK, m0);
           for (int kb = 0; kb < KB2; ++kb) {
             const int slot = kb % KB1;
             const uint32_t fill = it * 5u + 1u + (uint32_t)(nb * 2 + kb / KB1);
@@ -602,16 +599,7 @@ int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {
   p.n_t = a.anorm.t; p.n_t_stride = a.anorm.t_stride;
   p.n_scale_w = a.anorm.scale_w; p.n_scale_b = a.anorm.scale_b; p.n_bias_w = a.anorm.bias_w; p.n_bias_b = a.anorm.bias_b;
   p.dbg = g_gemm_debug;
-  static int respf = -1;
-  if (respf < 0) { const char* v = getenv("GECCO_MLP_RESPF"); respf = v ? atoi(v) : 1; }
-  p.respf = respf;
-  static int rev = -1;
-  if (rev < 0) { const char* v = getenv("GECCO_REV"); rev = v ? atoi(v) : 2; }
-  p.rev = (rev & 2) ? 1 : 0;
-  static int hints = -1;
-  if (hints < 0) { const char* v = getenv("GECCO_HINT_MLP"); hints = v ? atoi(v) : 2565; }  // A, residual read once: evict_first; hidden scratch: evict_last
-  p.hints = hints;
-  p.u.hints = ((hints >> 8) & 3) << 6;  // hidden tiles going to the scratch (bits 8-9), coming back (bits 10-11)
+  p.u.hints = POL_HIDDEN << 6;  // bf16 stores of the first product's epilogue: the hidden tiles going to the scratch
   p.d.hints = 0;
 
   static bool attr_set = false;

@@ -117,7 +117,8 @@ def gemm_anorm_supported(m: int, rows_per_cloud: int, n_out: int, k: int) -> boo
 
 
 def set_option(name: str, value: int) -> None:
-    """gecco_set_option: "gemm_pairs", "graphs", "anorm" (see include/gecco_b200.h)."""
+    """gecco_set_option: "gemm_pairs", "graphs", "anorm", "chain", "mlp_pair", "fast_epilogue", "epi_skip" (see
+    include/gecco_b200.h)."""
     _abi.check(_abi.load().gecco_set_option(name.encode(), C.c_int(int(value))))
 
 

@@ -38,11 +38,20 @@ const char* gecco_last_error(void);
 /* Checks that `device` is sm_100 and resolves the driver entry points. */
 int gecco_init(int device);
 
-/* Tuning switches.  "gemm_pairs" (default 1): use the CTA-pair (cta_group::2) GEMM where it applies;
+/* Tuning switches.  The defaults are the production paths; the others serve as references in tests and A/B measurements.
+ * "gemm_pairs" (default 1): use the CTA-pair (cta_group::2) GEMM where it applies;
  * "graphs" (default 1, or GECCO_GRAPHS=0 in the environment): gecco_sample captures its launch sequence into a
  * CUDA graph on the first call with a given argument set and replays it afterwards;
- * "anorm" (default 1, or GECCO_ANORM=0): the engine normalises (AdaGN) inside the consuming projection where the shape
- * allows (gecco_anorm) instead of folding the normalisation into per-cloud weights. */
+ * "anorm" (default 1): the engine normalises (AdaGN) inside the consuming projection where the shape allows
+ * (gecco_anorm) instead of folding the normalisation into per-cloud weights;
+ * "chain" (default 1): the engine runs the inducer side of a layer as one cluster kernel where the shape allows, instead
+ * of separate GEMM / AdaGN launches;
+ * "mlp_pair" (default 1): the engine runs the point-side MLP as one CTA-pair kernel with the hidden tile in an
+ * L2-resident scratch (needs "anorm"), instead of two GEMMs with the hidden tensor in HBM;
+ * "fast_epilogue" (default 1): bf16-only whole-tile projections take the pair GEMM's fast epilogue (bit-identical
+ * results);
+ * "epi_skip" (default 0, development aid): bit mask that switches parts of the GEMM epilogue off -- 1 output stores,
+ * 2 residual, 4 proxy fence, 8 statistics atomics.  Any non-zero value gives wrong results. */
 int gecco_set_option(const char* name, int value);
 
 /* ------------------------------------------------------------------------

@@ -110,7 +110,7 @@ def test_inducer_chain_merges_key_splits(cuda, clouds, N, splits):
 
 
 def test_engine_chain_matches_separate_launches(cuda):
-    """One denoiser evaluation with the chain kernel against the same evaluation with GECCO_CHAIN off."""
+    """One denoiser evaluation with the chain kernel against the same evaluation with the "chain" option off."""
     from gecco_b200 import ops
     from tests import synth
     from tests.models_b200 import build as build_model

@@ -35,12 +35,11 @@ sig = torch.full((B,), 2.0, device=dev)
 K = torch.tensor([[1.0859, 0, 0.4964], [0, 1.0859, 0.4964], [0, 0, 1]], device=dev).expand(B, 3, 3).contiguous()
 lo = torch.empty(B * N, 672, device=dev, dtype=torch.bfloat16)
 lst = torch.zeros(B, 16, 2, dtype=torch.float64, device=dev)
-for name, sizes, variants in (("137^2", (34, 17, 8), ("0", "2", "4", "2s", "4s")), ("256^2", (64, 32, 16), ("0", "12", "12s"))):
+for name, sizes, variants in (("137^2", (34, 17, 8), ("0", "2", "4")), ("256^2", (64, 32, 16), ("0", "12"))):
     levels = [torch.randn(B, s, s, c, device=dev).bfloat16() for s, c in zip(sizes, (96, 192, 384))]
     nbytes = sum(l.numel() * 2 for l in levels) + lo.numel() * 2 + xin.numel() * 4
     for v in variants:
-        os.environ["GECCO_LOOKUP_SLICES"] = v.rstrip("s")
-        os.environ["GECCO_LOOKUP_SCALAR"] = "1" if v.endswith("s") else "0"  # scalar FFMA instead of packed fp32x2
+        os.environ["GECCO_LOOKUP_SLICES"] = v
         fn = lambda: ops.lookup(xin, levels, K, reparam_kind=1, mean=[0, 0, 1], sigma_r=[0.15] * 3, sigma=sig, rows_per_cloud=N,
                                 out_bf16=lo, stats=lst)
         hot, cold = t_us(fn), t_us(fn, cold=True)
