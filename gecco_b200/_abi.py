@@ -312,6 +312,7 @@ def load() -> C.CDLL:
     lib.gecco_train_colsum2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     lib.gecco_graph_status.restype = C.c_int
     lib.gecco_chamfer.argtypes = [C.c_void_p, C.c_void_p]
+    lib.gecco_emd.argtypes = [C.c_void_p, C.c_void_p]
     _lib = lib
     return lib
 

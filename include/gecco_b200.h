@@ -531,6 +531,33 @@ typedef struct gecco_chamfer_args {
 } gecco_chamfer_args;
 int gecco_chamfer(const gecco_chamfer_args* args, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Approximate earth mover's distance, the second distance of PointFlow's compute_all_metrics (1-NNA-EMD / MMD-EMD /
+ * COV-EMD): the approximate matching of Fan et al. 2017 (approxmatch / match_cost) divided by N, as PointFlow's
+ * emd_approx.  It is NOT the optimal transport cost: it lies above the exact assignment.
+ * For clouds X = {x_k}, Y = {y_l} of N points, d2[k,l] = |x_k - y_l|^2, dist = sqrt(d2), remL = remR = 1, cost = 0:
+ *   for j = 7, 6, ..., 0, -1, -2:   level = -4^j (0 for j = -2), e[k,l] = exp(level * d2[k,l])
+ *     ratioL[k] = remL[k] / (1e-9 + sum_l e[k,l] remR[l])
+ *     sumr[l]   = remR[l] sum_k e[k,l] ratioL[k]
+ *     ratioR[l] = min(remR[l] / (sumr[l] + 1e-9), 1) remR[l];   remR[l] = max(0, remR[l] - sumr[l])
+ *     w[k,l]    = e[k,l] ratioL[k] ratioR[l];   remL[k] = max(0, remL[k] - sum_l w[k,l]);   cost += sum_{k,l} w dist
+ *   EMD(X, Y) = cost / N
+ * Rows are normalised before columns, so EMD(X, Y) != EMD(Y, X); EMD(X, X) is small but not 0.  The levels are absolute:
+ * the result depends on the units of the clouds (no normalisation).  Which argument is which matters for the
+ * metrics: PointFlow's 1-NNA reads its ordered self matrices down the columns, i.e. by EMD(other, c) for cloud c
+ * (gecco_b200/metrics.py passes them transposed to its row-wise reduction).
+ * Arguments as gecco_chamfer, with na == nb (for both clouds of a pair), 1 <= na <= 4096; anything else is refused with
+ * GECCO_ERR_INVALID and a message.
+ * mode GECCO_CHAMFER_ALL   : out [ma, mb], out[i][j] = EMD(a[i], b[j]);
+ *      GECCO_CHAMFER_PAIRED: out [ma],     out[i] = EMD(a[i], b[i]), ma == mb (bitwise equal to the ALL diagonal);
+ *      GECCO_CHAMFER_SELF  : out [ma, ma], out[i][j] = EMD(a[i], a[j]) for every ordered pair i != j (not symmetric;
+ *                            bitwise equal to ALL of a with itself); b is NULL or a; the diagonal is not computed and
+ *                            is written as exactly 0.
+ * fp32 arithmetic, one block per cloud pair, no N x N buffer; results are bitwise deterministic.  Non-finite points are
+ * not detected here: the caller checks its input.
+ * ------------------------------------------------------------------------ */
+int gecco_emd(const gecco_chamfer_args* args, void* stream);
+
 /* Per-kernel-class device timing of the engine (tracing aid; the reference has none, SURVEY.md §5).  Between
  * start and stop every engine launch on this thread is bracketed by CUDA events on its stream; stop synchronises
  * the device and returns, per class, the launch count, summed device time and the algorithmic FLOPs / bytes. */
