@@ -261,6 +261,16 @@ class ChamferArgs(C.Structure):
     ]
 
 
+class NearestArgs(C.Structure):
+    _fields_ = [
+        ("x", C.c_void_p), ("y", C.c_void_p),
+        ("clouds", C.c_int32), ("nx", C.c_int32), ("ny", C.c_int32),
+        ("dist_xy", C.c_void_p), ("idx_xy", C.c_void_p),
+        ("dist_yx", C.c_void_p), ("idx_yx", C.c_void_p),
+        ("scratch", C.c_void_p), ("scratch_bytes", C.c_int64),
+    ]
+
+
 class ProfileEntry(C.Structure):
     _fields_ = [("name", C.c_char * 32), ("launches", C.c_int64), ("ms", C.c_double), ("flops", C.c_double),
                 ("bytes", C.c_double)]
@@ -313,6 +323,9 @@ def load() -> C.CDLL:
     lib.gecco_graph_status.restype = C.c_int
     lib.gecco_chamfer.argtypes = [C.c_void_p, C.c_void_p]
     lib.gecco_emd.argtypes = [C.c_void_p, C.c_void_p]
+    lib.gecco_nearest.argtypes = [C.c_void_p, C.c_void_p]
+    lib.gecco_nearest_scratch_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+    lib.gecco_nearest_scratch_bytes.restype = C.c_int64
     _lib = lib
     return lib
 

@@ -1,5 +1,6 @@
 """Sample-quality metrics: Chamfer distance (CD) and earth mover's distance (EMD) on the GPU, and the 1-NNA / MMD / COV
-numbers built on either.
+numbers built on either; per-point nearest neighbours and the per-cloud F-score / paired CD of conditional
+reconstructions.
 
 These are the numbers reported for GECCO and its peers (PointFlow, LION); gecco-jax computes them in ``metrics.py`` /
 ``benchmark.py``.  The definitions follow PointFlow's ``compute_all_metrics``:
@@ -37,17 +38,37 @@ These are the numbers reported for GECCO and its peers (PointFlow, LION); gecco-
 - No normalisation: clouds are compared as given, in data space, which is what the samplers return.  Centring or scaling
   the clouds (PointFlow normalises per shape or globally depending on the table) is the caller's choice.
 
+Conditional outputs (single-view reconstruction, inpainting, upsampling) each have their own ground-truth cloud and are
+scored per sample, as in Tatarchenko et al. 2019 ("What do single-view 3D reconstruction networks learn?"):
+
+- :func:`nearest_neighbours` gives, for every point of ``x`` and of ``y``, the index of its nearest point in the other
+  cloud of the pair and the squared distance to it.  Ties go to the lowest index, as everywhere in this module.
+- With ``d_xy`` the squared distances from the prediction to the target and ``d_yx`` those back, and a threshold ``tau``
+  (a distance, in the units of the clouds): ``precision(tau) = mean_i [d_xy[i] < tau^2]``,
+  ``recall(tau) = mean_j [d_yx[j] < tau^2]`` (strict, compared in float64), ``F(tau) = 2 P R / (P + R)`` and
+  ``F = 0`` when ``P + R = 0``.
+- ``reconstruction_metrics(...)["cd"]`` is the CD defined above, the same number :func:`chamfer_distance` computes, with
+  different arithmetic: the distance to every chosen neighbour is recomputed in fp32 difference form and the means are
+  taken in float64, where ``gecco_chamfer`` sums the fp32 expansion's minima; the tests hold the two to 1e-4
+  relative.  ``gecco_nearest`` has no point cap below 2^24 per cloud, where ``gecco_chamfer``
+  refuses pairs whose clouds both exceed 32768 points.
+
 The CD matrices come from the ``gecco_chamfer`` kernel (``csrc/chamfer.cu``): one block per cloud pair, both
 directions in one pass, fp32 arithmetic on clouds translated to the first cloud's bounding-box centre, bitwise
 deterministic.  The EMD matrices come from ``gecco_emd`` (``csrc/emd.cu``): one block per cloud pair, fp32, the match
-matrix never stored, bitwise deterministic.  CPU tensors are refused (there is no CPU path); ``metrics_from_distances``
+matrix never stored, bitwise deterministic.  The nearest neighbours come from ``gecco_nearest`` (``csrc/nearest.cu``):
+many blocks per pair, both directions in one pass, merged with 64-bit integer minima, bitwise deterministic; its error
+bound is stated in ``include/gecco_b200.h``.  CPU tensors are refused (there is no CPU path); ``metrics_from_distances``
 is plain torch on the small ``[M, M]`` matrices and takes CPU or GPU tensors.
 """
 from __future__ import annotations
 
 import ctypes as C
 import math
+import numbers
+from typing import NamedTuple, Sequence
 
+import numpy as np
 import torch
 from torch import Tensor
 
@@ -161,6 +182,83 @@ def emd_matrix(a: Tensor, b: Tensor | None = None) -> Tensor:
     return out
 
 
+NEAREST_MAX_POINTS = 1 << 24
+
+
+class NearestNeighbours(NamedTuple):
+    """Result of :func:`nearest_neighbours`: squared fp32 distances and int64 indices, ``[B, Nx]`` / ``[B, Ny]``."""
+    dist_xy: Tensor
+    idx_xy: Tensor
+    dist_yx: Tensor
+    idx_yx: Tensor
+
+
+def nearest_neighbours(x: Tensor, y: Tensor) -> NearestNeighbours:
+    """Nearest neighbours within each cloud pair, both directions: ``idx_xy[b, i] = argmin_j |x[b, i] - y[b, j]|^2``
+    (lowest j on ties) and ``dist_xy[b, i]`` the squared distance to it; ``idx_yx`` / ``dist_yx`` from y to x.
+    x: ``[B, Nx, 3]``, y: ``[B, Ny, 3]`` on one CUDA device, 1 to 2^24 points per cloud (float64 sampler output is cast
+    to fp32 on the device).  Distances are fp32, recomputed in difference form for the chosen neighbour; the bound on
+    how far they can lie above the exact minimum is stated in ``include/gecco_b200.h``."""
+    for t, name in ((x, "x"), (y, "y")):
+        if not isinstance(t, Tensor):
+            raise TypeError(f"{name}: expected a tensor, got {type(t).__name__}")
+    if x.dim() == 3 and y.dim() == 3 and (x.shape[0] != y.shape[0] or x.device != y.device):
+        raise ValueError(f"nearest_neighbours: x and y need the same number of clouds on one device, got {tuple(x.shape)} "
+                         f"on {x.device} and {tuple(y.shape)} on {y.device}")
+    for t, name in ((x, "x"), (y, "y")):
+        if t.dim() == 3 and t.shape[1] > NEAREST_MAX_POINTS:
+            raise ValueError(f"nearest_neighbours: {name}: at most {NEAREST_MAX_POINTS} points per cloud, got {t.shape[1]}")
+    a, b = _clouds(x, "x"), _clouds(y, "y")
+    clouds, nx, ny = a.shape[0], a.shape[1], b.shape[1]
+    lib = _lib_for(a)
+    dev = a.device
+    f32, i32 = torch.float32, torch.int32
+    out = NearestNeighbours(torch.empty(clouds, nx, device=dev, dtype=f32), torch.empty(clouds, nx, device=dev, dtype=i32),
+                            torch.empty(clouds, ny, device=dev, dtype=f32), torch.empty(clouds, ny, device=dev, dtype=i32))
+    nbytes = lib.gecco_nearest_scratch_bytes(clouds, nx, ny)
+    scratch = torch.empty((nbytes + 7) // 8, device=dev, dtype=torch.int64)
+    args = _abi.NearestArgs()
+    args.x, args.y = a.data_ptr(), b.data_ptr()
+    args.clouds, args.nx, args.ny = clouds, nx, ny
+    args.dist_xy, args.idx_xy = out.dist_xy.data_ptr(), out.idx_xy.data_ptr()
+    args.dist_yx, args.idx_yx = out.dist_yx.data_ptr(), out.idx_yx.data_ptr()
+    args.scratch, args.scratch_bytes = scratch.data_ptr(), nbytes
+    _abi.check(lib.gecco_nearest(C.byref(args), _stream(a)))
+    return out._replace(idx_xy=out.idx_xy.long(), idx_yx=out.idx_yx.long())
+
+
+def _thresholds(thresholds) -> list[float]:
+    """A non-empty sequence (or 1-D tensor / numpy array) of positive finite numbers (distances, in the units of the
+    clouds) -> floats."""
+    if isinstance(thresholds, (Tensor, np.ndarray)):  # 1-D arrays, e.g. np.linspace(0.005, 0.02, 4)
+        thresholds = thresholds.tolist() if thresholds.ndim == 1 else None
+    if not isinstance(thresholds, Sequence) or isinstance(thresholds, (str, bytes)) or len(thresholds) == 0:
+        raise ValueError(f"reconstruction_metrics: thresholds must be a non-empty sequence of distances, got {thresholds!r}")
+    out = []
+    for t in thresholds:
+        if isinstance(t, bool) or not isinstance(t, numbers.Real) or not math.isfinite(t) or t <= 0:
+            raise ValueError(f"reconstruction_metrics: thresholds must be positive finite numbers, got {t!r}")
+        out.append(float(t))
+    return out
+
+
+def reconstruction_metrics(pred: Tensor, target: Tensor, thresholds: Sequence[float]) -> dict:
+    """Per-cloud scores of conditional outputs against their own ground truth: pred ``[B, Np, 3]``, target
+    ``[B, Nt, 3]``, thresholds: distances tau in the units of the clouds (no default: the module does not normalise
+    clouds).  Returns float64 tensors ``cd [B]`` (mean of ``dist_xy`` plus mean of ``dist_yx``) and ``precision``,
+    ``recall``, ``fscore [B, T]`` (definitions: module docstring).  Averages over a test set, or the best of several
+    samples per input, are the caller's to take."""
+    th = _thresholds(thresholds)
+    nn = nearest_neighbours(pred, target)
+    d_xy, d_yx = nn.dist_xy.double(), nn.dist_yx.double()
+    tau2 = torch.tensor([t * t for t in th], dtype=torch.float64, device=d_xy.device)
+    precision = (d_xy[:, :, None] < tau2).sum(1).double() / d_xy.shape[1]
+    recall = (d_yx[:, :, None] < tau2).sum(1).double() / d_yx.shape[1]
+    s = precision + recall
+    fscore = torch.where(s > 0, 2 * precision * recall / torch.where(s > 0, s, 1.0), 0.0)
+    return dict(cd=d_xy.mean(1) + d_yx.mean(1), precision=precision, recall=recall, fscore=fscore)
+
+
 def metrics_from_distances(d_gg: Tensor, d_rr: Tensor, d_gr: Tensor) -> dict:
     """1-NNA, MMD and COV from the three distance matrices (CD or EMD): ``d_gg [Mg, Mg]`` among the generated clouds,
     ``d_rr [Mr, Mr]`` among the reference clouds, ``d_gr [Mg, Mr]`` between them.  Definitions and tie rule: module
@@ -210,4 +308,5 @@ def sample_metrics(samples: Tensor, reference: Tensor, distance: str = "cd") -> 
     return metrics_from_distances(d_gg, d_rr, d_gr)
 
 
-__all__ = ["chamfer_distance", "chamfer_matrix", "emd_distance", "emd_matrix", "metrics_from_distances", "sample_metrics"]
+__all__ = ["chamfer_distance", "chamfer_matrix", "emd_distance", "emd_matrix", "metrics_from_distances", "sample_metrics",
+           "NearestNeighbours", "nearest_neighbours", "reconstruction_metrics"]

@@ -558,6 +558,33 @@ int gecco_chamfer(const gecco_chamfer_args* args, void* stream);
  * ------------------------------------------------------------------------ */
 int gecco_emd(const gecco_chamfer_args* args, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Nearest neighbours between paired clouds, both directions: the per-point numbers under the F-score and the paired
+ * Chamfer distance of conditional reconstructions (gecco_b200/metrics.py; Tatarchenko et al. 2019).
+ * x: fp32 [clouds, nx, 3], y: fp32 [clouds, ny, 3], contiguous; 1 <= nx, ny <= 2^24 (16777216), clouds >= 0; anything
+ * else is refused with GECCO_ERR_INVALID and a message.  For every pair b:
+ *   idx_xy[b][i] = argmin_j |x[b][i] - y[b][j]|^2,  dist_xy[b][i] = |x[b][i] - y[b][idx_xy[b][i]]|^2   (int32 / fp32 [clouds, nx])
+ *   idx_yx[b][j] = argmin_i |y[b][j] - x[b][i]|^2,  dist_yx[b][j] likewise                          (int32 / fp32 [clouds, ny])
+ * Ties go to the lowest index.  The search runs on the fp32 expansion |x|^2 + |y|^2 - 2 x.y on coordinates translated to
+ * the bounding-box centre c of x[b]; the reported distance is recomputed from the caller's coordinates in difference
+ * form.  With R the largest |p - c| over the points of the pair and d* the exact minimum, every reported distance lies
+ * in [d* (1 - 5 * 2^-24), d* + 2^-13 d* + 72 * 2^-24 R^2] (derivation in csrc/nearest.cu); where the second nearest point
+ * lies further above the nearest than that, the index is the exact argmin.
+ * scratch: caller-owned device memory of gecco_nearest_scratch_bytes(clouds, nx, ny) = 8 * clouds * (nx + ny + 2)
+ * bytes, 16-byte aligned (uint64 keys [clouds * (nx + ny)], then a centre per pair); its contents on entry do not matter.
+ * Merges across blocks are 64-bit integer minima on (distance bits << 32 | index): results are bitwise deterministic.
+ * Non-finite points are not detected here: the caller checks its input.
+ * ------------------------------------------------------------------------ */
+typedef struct gecco_nearest_args {
+  const float* x; const float* y;
+  int32_t clouds, nx, ny;
+  float* dist_xy; int32_t* idx_xy;
+  float* dist_yx; int32_t* idx_yx;
+  void* scratch; int64_t scratch_bytes;
+} gecco_nearest_args;
+int64_t gecco_nearest_scratch_bytes(int32_t clouds, int32_t nx, int32_t ny);
+int gecco_nearest(const gecco_nearest_args* args, void* stream);
+
 /* Per-kernel-class device timing of the engine (tracing aid; the reference has none, SURVEY.md §5).  Between
  * start and stop every engine launch on this thread is bracketed by CUDA events on its stream; stop synchronises
  * the device and returns, per class, the launch count, summed device time and the algorithmic FLOPs / bytes. */

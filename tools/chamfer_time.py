@@ -114,15 +114,16 @@ def _events_ms(fn, reps: int) -> list[float]:
     return out
 
 
-def inner_loop_mix(lib_path: Path) -> dict | None:
-    """Opcode counts of the chamfer kernel's inner loop (the backward branch whose body holds the FFMA2s), per lane and
-    point pair.  None when cuobjdump is missing or the loop is not found."""
+def inner_loop_mix(lib_path: Path, kernel: str = "chamfer_kernel") -> dict | None:
+    """Opcode counts of the inner loop of `kernel` (chamfer_kernel or nearest_kernel: the backward branch whose body
+    holds the FFMA2s, three per row and step), per lane and point pair.  None when cuobjdump is missing or the loop is
+    not found."""
     tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
     if not Path(tool).exists():
         return None
     sass = subprocess.run([tool, "-sass", str(lib_path)], capture_output=True, text=True).stdout
     funcs = re.split(r"\n\s*Function : ", sass)
-    body = next((f for f in funcs if "chamfer_kernel" in f.split("\n", 1)[0]), None)
+    body = next((f for f in funcs if kernel in f.split("\n", 1)[0]), None)
     if body is None:
         return None
     ins = []
