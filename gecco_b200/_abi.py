@@ -271,6 +271,17 @@ class NearestArgs(C.Structure):
     ]
 
 
+class EmdExactArgs(C.Structure):
+    _fields_ = [
+        ("a", C.c_void_p), ("ma", C.c_int32), ("na", C.c_int32),
+        ("b", C.c_void_p), ("mb", C.c_int32), ("nb", C.c_int32),
+        ("mode", C.c_int32),
+        ("out", C.c_void_p),
+        ("lower", C.c_void_p),
+        ("match", C.c_void_p),
+    ]
+
+
 class ProfileEntry(C.Structure):
     _fields_ = [("name", C.c_char * 32), ("launches", C.c_int64), ("ms", C.c_double), ("flops", C.c_double),
                 ("bytes", C.c_double)]
@@ -323,6 +334,7 @@ def load() -> C.CDLL:
     lib.gecco_graph_status.restype = C.c_int
     lib.gecco_chamfer.argtypes = [C.c_void_p, C.c_void_p]
     lib.gecco_emd.argtypes = [C.c_void_p, C.c_void_p]
+    lib.gecco_emd_exact.argtypes = [C.c_void_p, C.c_void_p]
     lib.gecco_nearest.argtypes = [C.c_void_p, C.c_void_p]
     lib.gecco_nearest_scratch_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
     lib.gecco_nearest_scratch_bytes.restype = C.c_int64

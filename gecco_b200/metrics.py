@@ -1,6 +1,6 @@
-"""Sample-quality metrics: Chamfer distance (CD) and earth mover's distance (EMD) on the GPU, and the 1-NNA / MMD / COV
-numbers built on either; per-point nearest neighbours and the per-cloud F-score / paired CD of conditional
-reconstructions.
+"""Sample-quality metrics: Chamfer distance (CD), approximate and exact earth mover's distance (EMD, EMD*) on the GPU,
+and the 1-NNA / MMD / COV numbers built on any of them; per-point nearest neighbours and the per-cloud F-score / paired
+CD of conditional reconstructions; the exact optimal matching of paired clouds.
 
 These are the numbers reported for GECCO and its peers (PointFlow, LION); gecco-jax computes them in ``metrics.py`` /
 ``benchmark.py``.  The definitions follow PointFlow's ``compute_all_metrics``:
@@ -33,6 +33,17 @@ These are the numbers reported for GECCO and its peers (PointFlow, LION); gecco-
   small but not 0; the self matrix of :func:`emd_matrix` writes its diagonal as 0 (the metrics exclude it).  The levels
   are absolute, so EMD depends on the units of the clouds, like CD.
 - ``MMD-EMD``, ``COV-EMD``, ``1-NNA-EMD``: the definitions above with EMD in place of CD.
+- ``EMD*(X, Y) = min over permutations s of (1/N) sum_i |x_i - y_s(i)|``: the exact earth mover's distance, the optimal
+  assignment between clouds of the same N points (at most 4096), with the Euclidean distance (not its square) as the
+  cost.  It is what gecco-jax's ``metrics.py`` computes with scipy's ``linear_sum_assignment``.  EMD* is symmetric,
+  ``EMD*(X, X) = 0``, and ``EMD* <= EMD`` pair by pair (the approximate matching is one transport plan).  The
+  ``gecco_emd_exact`` kernel finds it by a forward auction with epsilon scaling down to ``eps = 2^-20 D``, D the
+  bounding-box diagonal of the pair, and certifies it: the reported value is the cost of the permutation found (rounded
+  up), and the final prices give a dual bound ``lower`` (rounded down) with ``lower <= OPT <= emd`` on the fp32 costs and
+  ``emd - lower <= 2^-20 D`` up to the rounding of the bids.  Against the exact distances the bounds widen by
+  ``6 * 2^-24 D`` (``include/gecco_b200.h``).  Ties: equal bids go to the lowest point of the first cloud, equal values
+  to the lowest point of the second; results are bitwise deterministic.  ``MMD-EMD*``, ``COV-EMD*`` and ``1-NNA-EMD*``
+  are the definitions above with EMD* in place of CD; its matrices are symmetric, so they have no orientation to choose.
 - Ties: every argmin takes the lowest index; for 1-NNA the index in the concatenation ``[S_g; S_r]`` (PointFlow leaves this
   to ``topk``).
 - No normalisation: clouds are compared as given, in data space, which is what the samplers return.  Centring or scaling
@@ -56,10 +67,11 @@ scored per sample, as in Tatarchenko et al. 2019 ("What do single-view 3D recons
 The CD matrices come from the ``gecco_chamfer`` kernel (``csrc/chamfer.cu``): one block per cloud pair, both
 directions in one pass, fp32 arithmetic on clouds translated to the first cloud's bounding-box centre, bitwise
 deterministic.  The EMD matrices come from ``gecco_emd`` (``csrc/emd.cu``): one block per cloud pair, fp32, the match
-matrix never stored, bitwise deterministic.  The nearest neighbours come from ``gecco_nearest`` (``csrc/nearest.cu``):
-many blocks per pair, both directions in one pass, merged with 64-bit integer minima, bitwise deterministic; its error
-bound is stated in ``include/gecco_b200.h``.  CPU tensors are refused (there is no CPU path); ``metrics_from_distances``
-is plain torch on the small ``[M, M]`` matrices and takes CPU or GPU tensors.
+matrix never stored, bitwise deterministic.  The exact EMD comes from ``gecco_emd_exact`` (``csrc/emd_exact.cu``): one
+block per cloud pair, the costs recomputed on the fly, bitwise deterministic.  The nearest neighbours come from
+``gecco_nearest`` (``csrc/nearest.cu``): many blocks per pair, both directions in one pass, merged with 64-bit integer
+minima, bitwise deterministic; its error bound is stated in ``include/gecco_b200.h``.  CPU tensors are refused (there is
+no CPU path); ``metrics_from_distances`` is plain torch on the small ``[M, M]`` matrices and takes CPU or GPU tensors.
 """
 from __future__ import annotations
 
@@ -182,6 +194,72 @@ def emd_matrix(a: Tensor, b: Tensor | None = None) -> Tensor:
     return out
 
 
+class OptimalMatching(NamedTuple):
+    """Result of :func:`optimal_matching`: the exact EMD (fp32 ``[B]``, the cost of the permutation found, rounded up),
+    its certified lower bound (fp32 ``[B]``, rounded down) and the permutation (int64 ``[B, N]``, ``idx[b, i]`` the
+    point of ``y[b]`` matched to ``x[b, i]``)."""
+    emd: Tensor
+    lower: Tensor
+    idx: Tensor
+
+
+def _launch_exact(a: Tensor, b: Tensor | None, mode: int, out: Tensor, lower: Tensor | None = None,
+                  match: Tensor | None = None) -> None:
+    """Runs ``gecco_emd_exact``; a pair whose auction did not finish (NaN in ``out``) raises GeccoError naming it."""
+    lib = _lib_for(a)
+    args = _abi.EmdExactArgs()
+    args.a, args.ma, args.na = a.data_ptr(), a.shape[0], a.shape[1]
+    if b is not None:
+        args.b, args.mb, args.nb = b.data_ptr(), b.shape[0], b.shape[1]
+    args.mode = mode
+    args.out = out.data_ptr()
+    args.lower = lower.data_ptr() if lower is not None else None
+    args.match = match.data_ptr() if match is not None else None
+    _abi.check(lib.gecco_emd_exact(C.byref(args), _stream(a)))
+    bad = torch.isnan(out).nonzero().tolist()
+    if bad:
+        shown = ", ".join(str(tuple(p)) if len(p) > 1 else str(p[0]) for p in bad[:10]) + (", ..." if len(bad) > 10 else "")
+        raise _abi.GeccoError(f"gecco_emd_exact: the auction did not finish for {len(bad)} cloud pair(s): {shown}")
+
+
+def optimal_matching(x: Tensor, y: Tensor) -> OptimalMatching:
+    """Paired exact EMD with its certificate and permutation: ``emd[b] = EMD*(x[b], y[b])``, ``lower[b]`` the dual
+    bound, ``idx[b]`` the optimal permutation found.  x, y: ``[B, N, 3]`` with the same N (at most 4096) on one CUDA
+    device (float64 sampler output is cast to fp32 on the device).  Definition, certificate and tie rule: module
+    docstring."""
+    for t, name in ((x, "x"), (y, "y")):
+        if not isinstance(t, Tensor):
+            raise TypeError(f"{name}: expected a tensor, got {type(t).__name__}")
+    if x.dim() == 3 and y.dim() == 3 and (x.shape[0] != y.shape[0] or x.device != y.device):
+        raise ValueError(f"optimal_matching: x and y need the same number of clouds on one device, got {tuple(x.shape)} "
+                         f"on {x.device} and {tuple(y.shape)} on {y.device}")
+    _emd_points("optimal_matching", (x, "x"), (y, "y"))
+    a, b = _clouds(x, "x"), _clouds(y, "y")
+    dev, m, n = a.device, a.shape[0], a.shape[1]
+    out = OptimalMatching(torch.empty(m, device=dev, dtype=torch.float32), torch.empty(m, device=dev, dtype=torch.float32),
+                          torch.empty(m, n, device=dev, dtype=torch.int32))
+    _launch_exact(a, b, _abi.CHAMFER_PAIRED, out.emd, out.lower, out.idx)
+    return out._replace(idx=out.idx.long())
+
+
+def emd_exact_matrix(a: Tensor, b: Tensor | None = None) -> Tensor:
+    """All-pairs exact EMD, fp32 ``[Ma, Mb]`` with ``out[i, j] = EMD*(a[i], b[j])`` (the upper value of the
+    certificate).  a: ``[Ma, N, 3]``, b: ``[Mb, N, 3]``, the same N (at most 4096).  ``b=None`` gives the self matrix of
+    ``a``: each pair computed once, exactly symmetric, diagonal exactly 0."""
+    _emd_points("emd_exact_matrix", (a, "a"), (b, "b"))
+    ta = _clouds(a, "a")
+    if b is None:
+        out = torch.empty(ta.shape[0], ta.shape[0], device=ta.device, dtype=torch.float32)
+        _launch_exact(ta, None, _abi.CHAMFER_SELF, out)
+        return out
+    tb = _clouds(b, "b")
+    if ta.device != tb.device:
+        raise ValueError(f"emd_exact_matrix: a is on {ta.device}, b on {tb.device}")
+    out = torch.empty(ta.shape[0], tb.shape[0], device=ta.device, dtype=torch.float32)
+    _launch_exact(ta, tb, _abi.CHAMFER_ALL, out)
+    return out
+
+
 NEAREST_MAX_POINTS = 1 << 24
 
 
@@ -290,7 +368,10 @@ def sample_metrics(samples: Tensor, reference: Tensor, distance: str = "cd") -> 
 
     - ``"cd"``: three ``gecco_chamfer`` launches (``S_g x S_g`` and ``S_r x S_r`` as self matrices, ``S_g x S_r``);
     - ``"emd"``: three ``gecco_emd`` launches in PointFlow's orientation (module docstring): ``emd_matrix(samples).T``,
-      ``emd_matrix(reference).T`` and ``emd_matrix(reference, samples).T``; N' must equal N (at most 4096).
+      ``emd_matrix(reference).T`` and ``emd_matrix(reference, samples).T``; N' must equal N (at most 4096);
+    - ``"emd_exact"``: three ``gecco_emd_exact`` launches, ``emd_exact_matrix(samples)``, ``emd_exact_matrix(reference)``
+      and ``emd_exact_matrix(samples, reference)``; N' must equal N (at most 4096).  EMD* is symmetric, so unlike
+      ``"emd"`` there is no orientation to choose;
 
     then :func:`metrics_from_distances`."""
     if distance == "cd":
@@ -303,10 +384,16 @@ def sample_metrics(samples: Tensor, reference: Tensor, distance: str = "cd") -> 
         d_gg = emd_matrix(samples).t()
         d_rr = emd_matrix(reference).t()
         d_gr = emd_matrix(reference, samples).t()
+    elif distance == "emd_exact":
+        _emd_points("sample_metrics", (samples, "samples"), (reference, "reference"))
+        d_gg = emd_exact_matrix(samples)
+        d_rr = emd_exact_matrix(reference)
+        d_gr = emd_exact_matrix(samples, reference)
     else:
-        raise ValueError(f"sample_metrics: distance must be 'cd' or 'emd', got {distance!r}")
+        raise ValueError(f"sample_metrics: distance must be 'cd', 'emd' or 'emd_exact', got {distance!r}")
     return metrics_from_distances(d_gg, d_rr, d_gr)
 
 
 __all__ = ["chamfer_distance", "chamfer_matrix", "emd_distance", "emd_matrix", "metrics_from_distances", "sample_metrics",
-           "NearestNeighbours", "nearest_neighbours", "reconstruction_metrics"]
+           "NearestNeighbours", "nearest_neighbours", "reconstruction_metrics", "OptimalMatching", "optimal_matching",
+           "emd_exact_matrix"]

@@ -559,6 +559,42 @@ int gecco_chamfer(const gecco_chamfer_args* args, void* stream);
 int gecco_emd(const gecco_chamfer_args* args, void* stream);
 
 /* ------------------------------------------------------------------------
+ * Exact earth mover's distance: the optimal assignment between two clouds of the same N points, as gecco-jax's
+ * metrics.py computes it with scipy's linear_sum_assignment:
+ *   EMD*(X, Y) = min over permutations s of (1/N) sum_i |x_i - y_s(i)|   (Euclidean distance, not its square)
+ * EMD* is symmetric, EMD*(X, X) = 0, and EMD* <= the approximate EMD of gecco_emd pair by pair.  No normalisation.
+ * Method (csrc/emd_exact.cu): a forward auction with epsilon scaling and Jacobi bidding, one block per cloud pair, the
+ * N x N costs recomputed on the fly in fp32 (c_ij = sqrt(dx^2 + dy^2 + dz^2), difference form, on clouds translated to
+ * the pair's bounding-box centre).  eps runs D/4, D/16, ..., 2^-20 D (ten phases), with D the bounding-box diagonal of
+ * the pair.  Equal bids go to the lowest person, equal values to the lowest object: results are bitwise deterministic.
+ * A certificate follows from the final prices p (weak duality), accumulated in double:
+ *   out   = (1/N) sum_i c_{i s(i)}                              (the cost of the permutation found, rounded up)
+ *   lower = (1/N) (sum_i min_j (c_ij + p_j) - sum_j p_j)        (rounded down)
+ * so that lower <= OPT <= out on the fp32 costs, and out - lower <= 2^-20 D up to the rounding of the bids.  The fp32
+ * costs lie within 5 * 2^-24 D of the exact distances (derivation in the source); for the exact optimum OPT*:
+ *   lower - 6 * 2^-24 D <= OPT* <= out + 6 * 2^-24 D.
+ * a: fp32 [ma, na, 3], b: fp32 [mb, nb, 3], contiguous; na == nb, 1 <= na <= 4096; modes as gecco_chamfer:
+ *   GECCO_CHAMFER_ALL   : out (and lower) [ma, mb], out[i][j] = EMD*(a[i], b[j]), a[i] the persons;
+ *   GECCO_CHAMFER_PAIRED: out [ma], out[i] = EMD*(a[i], b[i]), ma == mb (bitwise equal to the ALL diagonal); match, if
+ *                         not NULL, int32 [ma, na]: match[i][k] = s(k), the object of point k of a[i];
+ *   GECCO_CHAMFER_SELF  : out [ma, ma]; b is NULL or a; each pair i < j is computed once with a[i] as the persons
+ *                         (bitwise equal to ALL there) and written to both halves (exactly symmetric); the diagonal
+ *                         is exactly 0.
+ * lower may be NULL; match must be NULL outside PAIRED.  Anything else is refused with GECCO_ERR_INVALID and a message.
+ * A pair whose auction phase fails to finish within 2^20 rounds (convergence takes thousands) gets NaN in out and lower
+ * and -1 in match.  Non-finite points are not detected here: the caller checks its input.
+ * ------------------------------------------------------------------------ */
+typedef struct gecco_emd_exact_args {
+  const float* a; int32_t ma, na;
+  const float* b; int32_t mb, nb;
+  int32_t mode;
+  float* out;
+  float* lower;
+  int32_t* match;
+} gecco_emd_exact_args;
+int gecco_emd_exact(const gecco_emd_exact_args* args, void* stream);
+
+/* ------------------------------------------------------------------------
  * Nearest neighbours between paired clouds, both directions: the per-point numbers under the F-score and the paired
  * Chamfer distance of conditional reconstructions (gecco_b200/metrics.py; Tatarchenko et al. 2019).
  * x: fp32 [clouds, nx, 3], y: fp32 [clouds, ny, 3], contiguous; 1 <= nx, ny <= 2^24 (16777216), clouds >= 0; anything
