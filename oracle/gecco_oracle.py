@@ -186,6 +186,8 @@ def network(cfg: OracleConfig, sd: dict, geometry: Tensor, t: Tensor, features, 
     if cfg.kind == "uncond":
         x = F.linear(geometry, sd[p + "lift.weight"], sd[p + "lift.bias"])
         x, out_h = set_transformer(cfg, sd, x, t, hs)
+        if p + "lower.weight" in sd:  # LinearLift(do_norm=False): a bare Linear head (models/linear_lift.py:26-29)
+            return F.linear(x, sd[p + "lower.weight"], sd[p + "lower.bias"]), out_h
         x = F.layer_norm(x, (x.shape[-1],), eps=1e-5)
         return F.linear(x, sd[p + "lower.1.weight"], sd[p + "lower.1.bias"]), out_h
     xyz = F.linear(geometry, sd[p + "xyz_embed.weight"], sd[p + "xyz_embed.bias"])
@@ -354,7 +356,7 @@ def edm_loss(cfg: OracleConfig, sd: dict, examples: Tensor, u: Tensor, noise: Te
     ex_diff = data_to_diffusion(cfg, sd, examples, K)
     n = examples.shape[0]
     div = 1 / n
-    uu = div * u + div * torch.arange(n)  # :105-108
+    uu = div * u + div * torch.arange(n, device=u.device)  # :105-108
     lo, hi = math.log(sigma_min), math.log(cfg.sigma_max)
     sigma = (uu * (hi - lo) + lo).exp().reshape(-1, 1, 1)  # :110-113
     weight = (sigma**2 + cfg.sigma_data**2) / ((sigma * cfg.sigma_data) ** 2)  # :138

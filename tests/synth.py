@@ -64,15 +64,17 @@ def synth_state_dict(shapes: Dict[str, Sequence[int]], seed: int) -> Dict[str, t
 
 def network_shapes(kind: str, n_layers: int = N_LAYERS, c: int = FEATURE_DIM, heads: int = NUM_HEADS,
                    inducers: int = NUM_INDUCERS, hidden: int | None = None,
-                   context_dims: Sequence[int] = CONTEXT_DIMS) -> Dict[str, tuple]:
+                   context_dims: Sequence[int] = CONTEXT_DIMS, do_norm: bool = True) -> Dict[str, tuple]:
     """Names and shapes of the learnable tensors of the denoiser in the reference state_dict schema
-    (SURVEY.md §8b; prefix `backbone.model.`).  kind: "uncond" (LinearLift) or "cond" (RayNetwork)."""
+    (SURVEY.md §8b; prefix `backbone.model.`).  kind: "uncond" (LinearLift) or "cond" (RayNetwork).
+    do_norm=False is LinearLift(do_norm=False): the head is a bare Linear, `lower.*` instead of `lower.1.*`."""
     hidden = hidden or 2 * c
     p = "backbone.model."
     s: Dict[str, tuple] = {}
     if kind == "uncond":
         s[p + "lift.weight"], s[p + "lift.bias"] = (c, 3), (c,)
-        s[p + "lower.1.weight"], s[p + "lower.1.bias"] = (3, c), (3,)
+        lower = p + ("lower.1." if do_norm else "lower.")
+        s[lower + "weight"], s[lower + "bias"] = (3, c), (3,)
         st = p + "inner."
     else:
         s[p + "xyz_embed.weight"], s[p + "xyz_embed.bias"] = (c, 3), (c,)
@@ -116,13 +118,14 @@ def full_state_dict(kind: str, reparam: str, mean, sigma, seed: int, **kw) -> Di
 
 
 def tame(sd: Dict[str, torch.Tensor], out_scale: float) -> Dict[str, torch.Tensor]:
-    """The "tame" recipe: the same synthetic weights with the output head (`lower.1` / `output_proj.1`) scaled by
+    """The "tame" recipe: the same synthetic weights with the output head (`lower.1`, `lower` without the LayerNorm, or
+    `output_proj.1`) scaled by
     `out_scale`.  With the raw recipe the Lipschitz constant of F is far above 1 and the 64-step sampler amplifies any
     perturbation (the unmodified reference drifts by 10-35 % under its own bf16 autocast); scaled to ~1 the
     probability-flow map contracts and full trajectories can be held to a tight tolerance."""
     out = dict(sd)
     for k, v in sd.items():
-        if ".lower.1." in k or ".output_proj.1." in k:
+        if ".lower.1." in k or ".output_proj.1." in k or k.endswith((".lower.weight", ".lower.bias")):
             out[k] = v * out_scale
     return out
 

@@ -64,8 +64,9 @@ def test_lift(cuda):
     assert torch.allclose(stats[..., 1].cpu(), (v * v).sum(dim=(1, 3)), rtol=1e-5, atol=1e-3)
 
 
-@pytest.mark.parametrize("norm", [1, 2])
+@pytest.mark.parametrize("norm", [0, 1, 2])
 def test_head_modes(cuda, norm):
+    """Head (no norm: LinearLift(do_norm=False); LayerNorm; GroupNorm) and its EDM modes, at sigma_data 1 and 0.5."""
     from gecco_b200 import ops
 
     B, N, Np, C = 2, 150, 256, 384
@@ -77,7 +78,9 @@ def test_head_modes(cuda, norm):
     sigma = torch.tensor([0.7, 3.0])
     xd = x.to(cuda).reshape(B * Np, C)
     stats = ops.group_stats(xd, Np, N, 12)
-    if norm == 1:
+    if norm == 0:
+        nx = x[:, :N]
+    elif norm == 1:
         nx = F.layer_norm(x[:, :N], (C,), eps=1e-5)
     else:
         nx = F.group_norm(x[:, :N].transpose(1, 2), 16, eps=1e-5).transpose(1, 2)
@@ -85,36 +88,39 @@ def test_head_modes(cuda, norm):
     kw = dict(clouds=B, rows_per_cloud=Np, valid_rows=N, norm=norm, groups=16, stats=stats)
     Fg = ops.head(xd, w.to(cuda), b.to(cuda), mode=0, **kw)
     assert (Fg.cpu() - Fref).abs().max().item() < 2e-4
-    s = sigma[:, None, None]
-    Dref = xin / (s**2 + 1) + s / (s**2 + 1).sqrt() * Fref
-    Dg = ops.head(xd, w.to(cuda), b.to(cuda), mode=1, xin=xin.to(cuda), sigma=sigma.to(cuda), **kw)
-    assert (Dg.cpu() - Dref).abs().max().item() < 3e-4
-    # Euler then Heun with a shared sigma (sampler use)
-    sig1 = torch.tensor([2.5], device=cuda)
-    s1 = 2.5
-    t_hat, t_next, churn = 2.5, 1.7, 0.3
-    x_hat = torch.randn(B, N, 3, generator=g, dtype=torch.float64)
-    xin_e = x_hat.float()
-    noise = torch.randn(B, N, 3, generator=g)
-    D1 = (xin_e / (s1**2 + 1) + s1 / math.sqrt(s1**2 + 1) * Fref).double()
-    d_cur = (x_hat - D1) / t_hat
-    x_next = x_hat + (t_next - t_hat) * d_cur
-    xh, xn, dc = x_hat.to(cuda).clone(), torch.empty_like(x_hat, device=cuda), torch.empty_like(x_hat, device=cuda)
-    xin_next = torch.empty(B, N, 3, device=cuda)
-    ops.head(xd, w.to(cuda), b.to(cuda), mode=2, xin=xin_e.to(cuda), sigma=sig1, sigma_stride=0, x_hat=xh, x_next=xn,
-             d_cur=dc, xin_next=xin_next, t_hat=t_hat, t_next=t_next, **kw)
-    assert (xn.cpu() - x_next).abs().max().item() < 1e-3
-    assert (xin_next.cpu() - x_next.float()).abs().max().item() < 1e-3
-    # Heun: evaluate "at x_next" with the same features (only the arithmetic is under test)
-    s2 = 1.7
-    sig2 = torch.tensor([s2], device=cuda)
-    xin_h = xn.float()
-    D2 = (xin_h.cpu() / (s2**2 + 1) + s2 / math.sqrt(s2**2 + 1) * Fref).double()
-    d_prime = (xn.cpu() - D2) / t_next
-    x_new = x_hat + (t_next - t_hat) * (0.5 * dc.cpu() + 0.5 * d_prime) + churn * noise.double()
-    ops.head(xd, w.to(cuda), b.to(cuda), mode=3, xin=xin_h, sigma=sig2, sigma_stride=0, x_hat=xh, x_next=xn, d_cur=dc,
-             xin_next=xin_next, noise_next=noise.to(cuda), t_hat=t_hat, t_next=t_next, churn_next=churn, **kw)
-    assert (xh.cpu() - x_new).abs().max().item() < 1e-3
+    for sd in (1.0, 0.5):
+        c_skip = lambda s: sd**2 / (s**2 + sd**2)
+        c_out = lambda s: s * sd / (s**2 + sd**2) ** 0.5
+        s = sigma[:, None, None]
+        Dref = c_skip(s) * xin + c_out(s) * Fref
+        Dg = ops.head(xd, w.to(cuda), b.to(cuda), mode=1, xin=xin.to(cuda), sigma=sigma.to(cuda), sigma_data=sd, **kw)
+        assert (Dg.cpu() - Dref).abs().max().item() < 3e-4, sd
+        # Euler then Heun with a shared sigma (sampler use)
+        sig1 = torch.tensor([2.5], device=cuda)
+        s1 = 2.5
+        t_hat, t_next, churn = 2.5, 1.7, 0.3
+        x_hat = torch.randn(B, N, 3, generator=g, dtype=torch.float64)
+        xin_e = x_hat.float()
+        noise = torch.randn(B, N, 3, generator=g)
+        D1 = (c_skip(s1) * xin_e + c_out(s1) * Fref).double()
+        d_cur = (x_hat - D1) / t_hat
+        x_next = x_hat + (t_next - t_hat) * d_cur
+        xh, xn, dc = x_hat.to(cuda).clone(), torch.empty_like(x_hat, device=cuda), torch.empty_like(x_hat, device=cuda)
+        xin_next = torch.empty(B, N, 3, device=cuda)
+        ops.head(xd, w.to(cuda), b.to(cuda), mode=2, xin=xin_e.to(cuda), sigma=sig1, sigma_stride=0, sigma_data=sd, x_hat=xh,
+                 x_next=xn, d_cur=dc, xin_next=xin_next, t_hat=t_hat, t_next=t_next, **kw)
+        assert (xn.cpu() - x_next).abs().max().item() < 1e-3, sd
+        assert (xin_next.cpu() - x_next.float()).abs().max().item() < 1e-3, sd
+        # Heun: evaluate "at x_next" with the same features (only the arithmetic is under test)
+        s2 = 1.7
+        sig2 = torch.tensor([s2], device=cuda)
+        xin_h = xn.float()
+        D2 = (c_skip(s2) * xin_h.cpu() + c_out(s2) * Fref).double()
+        d_prime = (xn.cpu() - D2) / t_next
+        x_new = x_hat + (t_next - t_hat) * (0.5 * dc.cpu() + 0.5 * d_prime) + churn * noise.double()
+        ops.head(xd, w.to(cuda), b.to(cuda), mode=3, xin=xin_h, sigma=sig2, sigma_stride=0, sigma_data=sd, x_hat=xh, x_next=xn,
+                 d_cur=dc, xin_next=xin_next, noise_next=noise.to(cuda), t_hat=t_hat, t_next=t_next, churn_next=churn, **kw)
+        assert (xh.cpu() - x_new).abs().max().item() < 1e-3, sd
 
 
 def _proj(p, K):
@@ -269,17 +275,10 @@ def test_reparam_roundtrip(cuda, kind, dtype):
         assert (data.cpu() - (diff * torch.tensor(sig, dtype=dtype) + torch.tensor(mean, dtype=dtype))).abs().max() < 1e-6
 
 
-@pytest.mark.parametrize("tensor_cores,B,N,splits", [(False, 2, 2048, 1), (False, 2, 2048, 4), (False, 2, 300, 2),
-                                                     (True, 2, 2048, 1), (True, 2, 2048, 4), (True, 2, 300, 2),
-                                                     (True, 3, 1000, 3), (True, 80, 640, 1), (True, 1, 128, 1),
-                                                     (True, 2, 1024, -1), (False, 2, 1024, -1)])
-def test_pool_attention(cuda, monkeypatch, tensor_cores, B, N, splits):
-    """mma.sync kernel and tcgen05 / TMEM kernel (key splits + combine, ragged last tile, several items per warpgroup)
-    against torch SDPA.  Padding rows hold finite non-zero keys / values that must be masked out."""
+def _pool_case(cuda, B, N, splits, H, D, dtype=torch.float32):
     from gecco_b200 import ops
 
-    monkeypatch.setenv("GECCO_POOL_TC", "1" if tensor_cores else "0")
-    H, D, I = 8, 48, 64
+    I = 64
     C = H * D
     Np = (N + 127) // 128 * 128
     g = _gen(6)
@@ -296,23 +295,41 @@ def test_pool_attention(cuda, monkeypatch, tensor_cores, B, N, splits):
     out = ops.pool_attention(kvd, qs, clouds=B, rows_per_cloud=Np, valid_rows=N, heads=H, head_dim=D, k_off=0, v_off=C,
                              splits=splits)
     torch.cuda.synchronize()
-    kvr = kvd.float().cpu().view(B, Np, 3 * C)[:, :N]
+    kvr = kvd.to(dtype).cpu().view(B, Np, 3 * C)[:, :N]
     k = kvr[..., :C].reshape(B, N, H, D).transpose(1, 2)
     v = kvr[..., C:2 * C].reshape(B, N, H, D).transpose(1, 2)
     # queries as the kernel sees them (bf16-rounded after the scale fold): with logits in the hundreds the rounding of
     # the queries alone moves the softmax
-    qr = (qs.float().cpu() / (D**-0.5 * math.log2(math.e)))[None]
+    qr = (qs.to(dtype).cpu() / (D**-0.5 * math.log2(math.e)))[None]
     ref = F.scaled_dot_product_attention(qr.expand(B, -1, -1, -1), k, v).transpose(1, 2).reshape(B, I, C)
-    err = (out.float().cpu().view(B, I, C) - ref).abs().max().item()
+    return (out.to(dtype).cpu().view(B, I, C) - ref).abs().max().item()
+
+
+@pytest.mark.parametrize("tensor_cores,B,N,splits", [(False, 2, 2048, 1), (False, 2, 2048, 4), (False, 2, 300, 2),
+                                                     (True, 2, 2048, 1), (True, 2, 2048, 4), (True, 2, 300, 2),
+                                                     (True, 3, 1000, 3), (True, 80, 640, 1), (True, 1, 128, 1),
+                                                     (True, 2, 1024, -1), (False, 2, 1024, -1)])
+def test_pool_attention(cuda, monkeypatch, tensor_cores, B, N, splits):
+    """mma.sync kernel and tcgen05 / TMEM kernel (key splits + combine, ragged last tile, several items per warpgroup)
+    against torch SDPA.  Padding rows hold finite non-zero keys / values that must be masked out."""
+    monkeypatch.setenv("GECCO_POOL_TC", "1" if tensor_cores else "0")
+    err = _pool_case(cuda, B, N, splits, 8, 48)
     assert err < 2e-2, err
 
 
-@pytest.mark.parametrize("tensor_cores,B,Np", [(False, 2, 256), (True, 2, 256), (True, 5, 128), (True, 70, 384)])
-def test_unpool_attention(cuda, tensor_cores, B, Np):
-    """mma.sync kernel and tcgen05 / TMEM kernel (several tiles per CTA, CTAs spanning two clouds) against torch SDPA."""
+@pytest.mark.parametrize("B,N,splits", [(2, 2048, 1), (2, 2048, 4), (2, 300, 1), (2, 300, 4), (3, 1000, 3), (2, 1024, -1)])
+@pytest.mark.parametrize("H,D", [(12, 32), (6, 64)])
+def test_pool_attention_head_dims(cuda, B, N, splits, H, D):
+    """The mma.sync pool kernels of head dim 32 and 64 (num_heads 12 / 6 at feature_dim 384), which the tcgen05 kernel
+    refuses, against float64 SDPA on the same bf16 operands."""
+    err = _pool_case(cuda, B, N, splits, H, D, dtype=torch.float64)
+    assert err < 2e-2, err
+
+
+def _unpool_case(cuda, B, Np, H, D, tensor_cores, dtype=torch.float32):
     from gecco_b200 import ops
 
-    H, D, I = 8, 48, 64
+    I = 64
     C = H * D
     g = _gen(7)
     q = torch.randn(B * Np, C, generator=g)
@@ -321,12 +338,27 @@ def test_unpool_attention(cuda, tensor_cores, B, Np):
     kd = khv.to(cuda).bfloat16()
     out = ops.unpool_attention(qd, kd, clouds=B, rows_per_cloud=Np, heads=H, head_dim=D, v_off=C, tensor_cores=tensor_cores)
     torch.cuda.synchronize()
-    qr = (qd.float().cpu() / (D**-0.5 * math.log2(math.e)) ).view(B, Np, H, D).transpose(1, 2)
-    kr = kd.float().cpu().view(B, I, 2 * C)
+    qr = (qd.to(dtype).cpu() / (D**-0.5 * math.log2(math.e)) ).view(B, Np, H, D).transpose(1, 2)
+    kr = kd.to(dtype).cpu().view(B, I, 2 * C)
     k = kr[..., :C].reshape(B, I, H, D).transpose(1, 2)
     v = kr[..., C:].reshape(B, I, H, D).transpose(1, 2)
     ref = F.scaled_dot_product_attention(qr, k, v).transpose(1, 2).reshape(B * Np, C)
-    err = (out.float().cpu() - ref).abs().max().item()
+    return (out.to(dtype).cpu() - ref).abs().max().item()
+
+
+@pytest.mark.parametrize("tensor_cores,B,Np", [(False, 2, 256), (True, 2, 256), (True, 5, 128), (True, 70, 384)])
+def test_unpool_attention(cuda, tensor_cores, B, Np):
+    """mma.sync kernel and tcgen05 / TMEM kernel (several tiles per CTA, CTAs spanning two clouds) against torch SDPA."""
+    err = _unpool_case(cuda, B, Np, 8, 48, tensor_cores)
+    assert err < 3e-2, err
+
+
+@pytest.mark.parametrize("B,Np", [(2, 256), (5, 128), (3, 384)])
+@pytest.mark.parametrize("H,D", [(12, 32), (6, 64)])
+def test_unpool_attention_head_dims(cuda, B, Np, H, D):
+    """The mma.sync unpool kernels of head dim 32 and 64 (offered the tcgen05 scratch, which they must not take) against
+    float64 SDPA on the same bf16 operands."""
+    err = _unpool_case(cuda, B, Np, H, D, True, dtype=torch.float64)
     assert err < 3e-2, err
 
 
