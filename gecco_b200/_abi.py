@@ -42,6 +42,7 @@ class GemmArgs(C.Structure):
         ("sigma", C.c_void_p), ("sigma_stride", C.c_int32), ("sigma_data", C.c_float),
         ("wx", C.c_void_p),
         ("anorm", ANorm),
+        ("stat_gs", C.c_int32),
     ]
 
 
@@ -61,6 +62,7 @@ class MlpArgs(C.Structure):
         ("stats", C.c_void_p),
         ("anorm", ANorm),
         ("scratch", C.c_void_p),
+        ("stat_gs", C.c_int32),
     ]
 
 

@@ -201,8 +201,8 @@ Workspace carve(const gecco_engine* e, int clouds, int points, void* base) {
   w.h = c.take<float>((size_t)w.irows * C);
   w.h2 = c.take<float>((size_t)w.irows * C);
   w.partial = c.take<float>((size_t)clouds * d.num_heads * w.splits * I * (C / d.num_heads + 2));
-  // statistics at 12-channel (= C / adagn_groups) granularity: per layer {broadcast_norm, norm_1, norm_2, mlp_norm},
-  // plus the head norm, plus the image-feature GroupNorm
+  // statistics at the AdaGN group width (C / adagn_groups channels: one sum pair per group): per layer {broadcast_norm,
+  // norm_1, norm_2, mlp_norm}, plus the head norm, plus the image-feature GroupNorm
   const int sg = d.adagn_groups;
   w.n_stats = (long long)clouds * ((4LL * d.n_layers + 1) * sg * 2 + (d.kind == 1 ? d.img_groups * 2 : 0));
   w.stats = c.take<double>((size_t)w.n_stats);
@@ -375,7 +375,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     g.wx = e->net[GECCO_NW_EMBED_W];
     g.out_f32 = w.x; g.ldo32 = C;
     g.out_bf16 = xb_out; g.ldo16 = C;
-    g.stats = stat(0, 0);
+    g.stats = stat(0, 0); g.stat_gs = C / sg;
     TRYP(K_GEMM_IMG, 2 * Mv * Cd * ctot + 6 * Mv * Cd, Mv * (ctot * 2.0 + Cd * 6) + 2.0 * clouds * Cd * ctot, launch_gemm(g, s));
   }
 
@@ -448,7 +448,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       // AttentionPool (:47-65)
       TRYP(K_POOL_ATTN, 4 * Mv * I * Cd, Mv * Cd * 4 + Mi * Cd * 2, launch_pool_attention(pool, s));
       gecco_gemm_args g = gemm_base(w.pooled, C, L.pool_out_w, C, irows, C, C, I, I);
-      g.out_f32 = w.h; g.ldo32 = C; g.stats = stat(l, 1);
+      g.out_f32 = w.h; g.ldo32 = C; g.stats = stat(l, 1); g.stat_gs = C / sg;
       TRYP(K_INDUCER_CHAIN, 2 * Mi * Cd * Cd, Mi * Cd * 6 + 2 * Cd * Cd, launch_gemm(g, s));
       // h = norm_2(mlp(norm_1(h)))  (:108-110)
       gecco_adagn_args a = adagn_base(e, lw + GECCO_LW_N1, w.h, stat(l, 1), w.c_noise, clouds, I, I);
@@ -460,7 +460,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       TRYP(K_INDUCER_CHAIN, 2 * Mi * Cd * Hd, Mi * (Cd + Hd) * 2 + 2 * Cd * Hd, launch_gemm(g, s));
       g = gemm_base(w.hh, hid, L.bmlp_w2, hid, irows, C, hid, I, I);
       g.bias = lw[GECCO_LW_BMLP_B2];
-      g.out_f32 = w.h2; g.ldo32 = C; g.stats = stat(l, 2);
+      g.out_f32 = w.h2; g.ldo32 = C; g.stats = stat(l, 2); g.stat_gs = C / sg;
       TRYP(K_INDUCER_CHAIN, 2 * Mi * Cd * Hd, Mi * (Hd * 2 + Cd * 4) + 2 * Cd * Hd, launch_gemm(g, s));
       a = adagn_base(e, lw + GECCO_LW_N2, w.h2, stat(l, 2), w.c_noise, clouds, I, I);
       a.out_bf16 = w.h3; a.ldo16 = C;
@@ -500,7 +500,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       g.bias = lw[GECCO_LW_UNPOOL_OUT_B];
       g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
       g.out_bf16 = xb_out; g.ldo16 = C;
-      g.stats = stat(l, 3);
+      g.stats = stat(l, 3); g.stat_gs = C / sg;
       TRYP(K_GEMM_UNPOOL_OUT, 2 * Mv * Cd * Cd, Mv * Cd * 12 + 2 * Cd * Cd, launch_gemm(g, s));
     }
     // x = x + mlp(AdaGN_mlp(x, t))  (:165-166): mlp_norm folded into mlp.0; statistics for the next broadcast_norm /
@@ -514,7 +514,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       mp.w2 = L.mlp_w2; mp.ldw2 = hid; mp.b2 = lw[GECCO_LW_MLP_B2];
       mp.m = rows; mp.c = C; mp.hidden = hid; mp.rows_per_cloud = Np; mp.valid_rows = points;
       mp.res = w.x; mp.ldr = C; mp.out_f32 = w.x; mp.ldo32 = C; mp.out_bf16 = xb_out; mp.ldo16 = C;
-      mp.stats = next_stats;
+      mp.stats = next_stats; mp.stat_gs = C / sg;
       mp.anorm.stats = stat(l, 3); mp.anorm.stat_gs = C / sg; mp.anorm.groups = sg; mp.anorm.eps = 1e-5f;
       mp.anorm.t = w.c_noise; mp.anorm.t_stride = 1;
       mp.anorm.scale_w = lw[GECCO_LW_MN]; mp.anorm.scale_b = lw[GECCO_LW_MN + 1];
@@ -534,7 +534,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       g.bias = lw[GECCO_LW_MLP_B2];
       g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
       g.out_bf16 = xb_out; g.ldo16 = C;
-      g.stats = next_stats;
+      g.stats = next_stats; g.stat_gs = C / sg;
       TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * 10) + 2 * Cd * Hd, launch_gemm(g, s));
     } else {
       gecco_fold_adagn_args f = fold_base(e, lw + GECCO_LW_MN, stat(l, 3), w.c_noise, clouds, points);
@@ -551,7 +551,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       g.bias = lw[GECCO_LW_MLP_B2];
       g.res = w.x; g.ldr = C; g.out_f32 = w.x; g.ldo32 = C;
       g.out_bf16 = w.xb; g.ldo16 = C;
-      g.stats = next_stats;
+      g.stats = next_stats; g.stat_gs = C / sg;
       TRYP(K_GEMM_MLP2, 2 * Mv * Cd * Hd, Mv * (Hd * 2 + Cd * 10) + 2 * Cd * Hd, launch_gemm(g, s));
     }
   }
@@ -598,12 +598,15 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
   GECCO_REQUIRE(H > 0 && C % H == 0 && (C / H == 32 || C / H == 48 || C / H == 64),
                 "gecco_create: head dim must be 32, 48 or 64 (feature_dim %d, heads %d)", C, H);
   GECCO_REQUIRE(I == 64, "gecco_create: only 64 inducers are supported (got %d)", I);
-  GECCO_REQUIRE(d.adagn_groups > 0 && C % d.adagn_groups == 0 && C / d.adagn_groups == 12,
-                "gecco_create: AdaGN groups must be 12 channels wide (feature_dim %d, groups %d)", C, d.adagn_groups);
+  // The GEMM epilogues keep the AdaGN statistics per group of C / adagn_groups channels; they are instantiated for the
+  // widths that divide their 192-column panel.
+  GECCO_REQUIRE(d.adagn_groups > 0 && C % d.adagn_groups == 0 && epi_stat_width_supported(C / d.adagn_groups),
+                "gecco_create: feature_dim %d is not supported with %d AdaGN groups: the groups must be 4, 8, 12, 16, 24 or "
+                "32 channels wide (feature_dim 128, 256, 384, 512, 768 or 1024 with 32 groups)", C, d.adagn_groups);
   GECCO_REQUIRE(hid > 0 && hid % 8 == 0, "gecco_create: mlp_hidden must be a multiple of 8");
   GECCO_REQUIRE(d.head_norm >= 0 && d.head_norm <= 2, "gecco_create: bad head_norm");
-  GECCO_REQUIRE(d.head_norm != 2 || (d.head_groups > 0 && C % d.head_groups == 0 && (C / d.head_groups) % 12 == 0),
-                "gecco_create: head GroupNorm groups must be multiples of 12 channels");
+  GECCO_REQUIRE(d.head_norm != 2 || (d.head_groups > 0 && C % d.head_groups == 0 && (C / d.head_groups) % (C / d.adagn_groups) == 0),
+                "gecco_create: head GroupNorm groups must be multiples of the AdaGN group width (%d channels)", C / d.adagn_groups);
   int ctot = 0;
   if (d.kind == 1) {
     GECCO_REQUIRE(d.n_levels >= 1 && d.n_levels <= GECCO_MAX_LEVELS, "gecco_create: 1..%d pyramid levels", GECCO_MAX_LEVELS);

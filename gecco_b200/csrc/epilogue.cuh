@@ -1,6 +1,8 @@
 // Row-tile epilogue shared by the tcgen05 kernels: drains a 128-row x 192-column fp32 accumulator panel from
 // TMEM in 32-column chunks and applies, in this order,
 //   + bias[cloud][n]  + xyz embed  -> Gaussian activation -> + residual -> AdaGN statistics -> fp32 / bf16 stores.
+// The statistics are per (cloud, group of W consecutive columns), W a compile-time parameter that divides the panel
+// (EpiStats below).
 // The TMEM layout gives every thread one ROW of the tile; global memory wants whole row segments per request, so all
 // global traffic of the epilogue goes through TMA and swizzled shared memory.
 // Two epilogue groups of 128 threads (4 warps each, warp q <-> TMEM lanes 32q..) work on alternate chunks.  Each group
@@ -20,7 +22,7 @@ namespace gecco {
 constexpr int EPI_THREADS = 128;                      // per group
 constexpr int EPI_GROUPS = 2;
 constexpr int EPI_CHUNK = 32;                         // columns per chunk
-constexpr int EPI_PANEL = 192;                        // columns per panel (16 AdaGN groups of 12)
+constexpr int EPI_PANEL = 192;                        // columns per panel (16 AdaGN groups of 12 at C = 384)
 constexpr int EPI_RES_BYTES = 128 * EPI_CHUNK * 4;    // one fp32 chunk (TMA box {32, 128}, SWIZZLE_128B): an X buffer
 constexpr int EPI_O16_BYTES = 128 * EPI_CHUNK * 2;    // one bf16 chunk (TMA box {32, 128}, SWIZZLE_64B)
 constexpr int EPI_BIAS_BYTES = 8 * 384;                // per-warp bias staging (3 chunks x 32 floats)
@@ -36,7 +38,7 @@ struct EpiParams {
   int has_res;
   float* o32;           // fp32 output or nullptr (written through its tensor map)
   __nv_bfloat16* o16;   // bf16 output or nullptr
-  double* stats;  // [clouds][n_out / 12][2] or nullptr
+  double* stats;  // [clouds][n_out / W][2] or nullptr (W: the statistics width the kernel was instantiated for)
   const float* geom;  // [clouds, valid_rows, 3] or nullptr
   const float* sigma;
   int sigma_stride;
@@ -101,20 +103,49 @@ __device__ __forceinline__ void epi_load_residual_panel(const EpiParams& p, cons
   }
 }
 
-// Sum over the 32 lanes of v[i] lands in lane i (31 shuffles instead of 32 x 5).
-__device__ __forceinline__ float warp_reduce_scatter32(float (&v)[32], int lane) {
+// Sum over the 32 lanes of v[OFF + (lane % N)] lands in lane (N a power of two <= 32): log2(N) halving steps
+// (N - 1 shuffles; 31 instead of 32 x 5 at N = 32), then 5 - log2(N) butterfly steps over the lanes holding the same slot.
+template <int N, int OFF, int S>
+__device__ __forceinline__ float warp_reduce_scatter(float (&v)[S], int lane) {
+  static_assert(N >= 1 && N <= 32 && (N & (N - 1)) == 0 && OFF + N <= S, "reduce-scatter width");
 #pragma unroll
-  for (int off = 16; off >= 1; off >>= 1) {
+  for (int off = N / 2; off >= 1; off >>= 1) {
     const bool upper = (lane & off) != 0;
 #pragma unroll
     for (int i = 0; i < off; ++i) {
-      const float send = upper ? v[i] : v[i + off];
-      const float keep = upper ? v[i + off] : v[i];
-      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+      const float send = upper ? v[OFF + i] : v[OFF + i + off];
+      const float keep = upper ? v[OFF + i + off] : v[OFF + i];
+      v[OFF + i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
     }
   }
-  return v[0];
+  float r = v[OFF];
+#pragma unroll
+  for (int off = N; off < 32; off <<= 1) r += __shfl_xor_sync(0xffffffffu, r, off);
+  return r;
 }
+
+// Register layout of the AdaGN statistics a thread accumulates for its row over one panel, at a group width of W
+// columns (W = 0: no statistics).  Each thread sees three of the panel's six chunks (2 k + grp, k = 0..2).
+//  - W divides the chunk (4, 8, 16, 32): only the groups of those three chunks, slot 2 (k (32 / W) + j / W) + moment for
+//    column j of its k-th chunk;
+//  - W = 12, 24 (groups straddle chunks): every group of the panel, slot 2 g + moment (the other chunks' slots stay 0).
+// The warp reduce-scatters the slots in rounds of at most 32 (the last one padded to a power of two: kRegs registers)
+// and one lane per slot adds it into stats[cloud][n_out / W][{sum, sumsq}].
+constexpr int epi_pow2_ceil(int x) { return x <= 1 ? 1 : 2 * epi_pow2_ceil((x + 1) / 2); }
+template <int W>
+struct EpiStats {
+  static_assert(W == 0 || (W > 0 && EPI_PANEL % W == 0 && W % 4 == 0), "statistics width must divide the panel");
+  static constexpr bool kLocal = W > 0 && EPI_CHUNK % W == 0;
+  static constexpr int kSlots = W == 0 ? 0 : kLocal ? 3 * 2 * (EPI_CHUNK / W) : 2 * (EPI_PANEL / W);
+  static constexpr int kRounds = (kSlots + 31) / 32;
+  // lanes reduce-scatter round r spans (slots 32 r ...)
+  static constexpr __host__ __device__ int width(int r) { return kSlots - 32 * r >= 32 ? 32 : epi_pow2_ceil(kSlots - 32 * r); }
+  static constexpr int kRegs = W == 0 ? 1 : 32 * (kRounds - 1) + width(kRounds - 1);
+  // slot of column j of panel chunk c (c = 2 k + grp)
+  static constexpr __host__ __device__ int slot(int c, int j) {
+    return kLocal ? 2 * ((c >> 1) * (EPI_CHUNK / W) + j / W) : 2 * ((c * EPI_CHUNK + j) / W);
+  }
+};
 
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
   float4 v;
@@ -225,12 +256,12 @@ __device__ __forceinline__ void epi_prefetch(const EpiParams& p, const EpiThread
   } while (0)
 
 // One 32-column chunk after its accumulator values (+ bias) are in registers.  C: chunk index inside the panel
-// (compile-time, so the AdaGN group of every column is static).  `full`: tile completely inside the matrix.
-template <bool kStats, int C>
+// (compile-time, so the AdaGN group of every column is static).  W: statistics width (0: none).
+template <int W, int C>
 __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm, const EpiThread& t, float (&v)[EPI_CHUNK],
                                           int m0, int col0, bool rows_valid, bool row_valid, float g0, float g1, float g2,
                                           const CUtensorMap* tma_o32, const CUtensorMap* tma_o16,
-                                          float (&st)[kStats ? 32 : 1], uint32_t& cnt) {
+                                          float (&st)[EpiStats<W>::kRegs], uint32_t& cnt) {
   if (p.geom != nullptr) {
     const float4* wp = reinterpret_cast<const float4*>(p.wx + (long long)col0 * 3);
 #pragma unroll
@@ -273,13 +304,12 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm,
 #pragma unroll
     for (int j = 0; j < EPI_CHUNK; ++j) v[j] = 0.f;  // padding rows stay exactly zero
   }
-  if (kStats) {
+  if constexpr (W != 0) {
 #pragma unroll
     for (int j = 0; j < EPI_CHUNK; ++j) {
-      constexpr int kBase = C * EPI_CHUNK;
-      const int g = (kBase + j) / 12;  // static: n0 is a multiple of 192
-      st[2 * g] += v[j];
-      st[2 * g + 1] = fmaf(v[j], v[j], st[2 * g + 1]);
+      const int sl = EpiStats<W>::slot(C, j);  // static: n0 is a multiple of 192
+      st[sl] += v[j];
+      st[sl + 1] = fmaf(v[j], v[j], st[sl + 1]);
     }
   }
   // this thread's row goes back into the X buffer (over its own residual values), the warp's 32 x 32 block is then
@@ -321,7 +351,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm,
 // must have been staged by this thread (epi_bias_stage / epi_prefetch).  The group's three chunks (grp, grp + 2, grp + 4) are software
 // pipelined: the TMEM load of the next chunk is issued as soon as the current one has been consumed, because
 // tcgen05.ld latency is several hundred cycles while the tensor core is streaming accumulators through TMEM.
-template <bool kStats>
+template <int W>
 __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm, const EpiThread& t,
                                           const CUtensorMap* tma_o32, const CUtensorMap* tma_o16, uint32_t taddr, int m0,
                                           int n0, uint32_t& cnt) {
@@ -345,9 +375,10 @@ __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm,
     g1 = c_in * __ldg(gp + 1);
     g2 = c_in * __ldg(gp + 2);
   }
-  float st[kStats ? 32 : 1];  // [group 0..15][{sum, sumsq}] of this row over the panel
+  using Stats = EpiStats<W>;
+  float st[Stats::kRegs];  // {sum, sumsq} of this row per group (layout: EpiStats)
 #pragma unroll
-  for (int i = 0; i < (kStats ? 32 : 1); ++i) st[i] = 0.f;
+  for (int i = 0; i < Stats::kRegs; ++i) st[i] = 0.f;
   auto step = [&](auto kc) {
     constexpr int k = decltype(kc)::value;
     if (n0 + (2 * k + t.grp) * EPI_CHUNK < p.n_out) {  // uniform over the epilogue group
@@ -370,26 +401,37 @@ __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm,
       }
       if (k < 2 && n0 + (2 * k + 2 + t.grp) * EPI_CHUNK < p.n_out) tmem_ld32_issue(ta + (2 * k + 2) * EPI_CHUNK, rr[(k + 1) & 1]);
       const int col0 = n0 + (2 * k + t.grp) * EPI_CHUNK;
-      if constexpr (kStats) {  // the AdaGN group of every column must be static: one instantiation per chunk index
+      if constexpr (W != 0) {  // the AdaGN group of every column must be static: one instantiation per chunk index
         if (t.grp == 0)
-          epi_chunk<true, 2 * k>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+          epi_chunk<W, 2 * k>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
         else
-          epi_chunk<true, 2 * k + 1>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+          epi_chunk<W, 2 * k + 1>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
       } else {
-        epi_chunk<false, 0>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+        epi_chunk<0, 0>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
       }
     }
   };
   step(std::integral_constant<int, 0>{});
   step(std::integral_constant<int, 1>{});
   step(std::integral_constant<int, 2>{});
-  if constexpr (kStats) {
+  if constexpr (W != 0) {
     long long ts0__ = 0;
     if (GECCO_DBG_ON(p.dbg)) ts0__ = clock64();
-    const float mine = warp_reduce_scatter32(st, t.lane);
-    const int gidx = (n0 / 12) * 2 + t.lane;  // [group][{sum, sumsq}]
-    if (gidx < (p.n_out / 12) * 2 && m0 + t.q * 32 < p.M)
-      if (!(p.skip & 8)) atomicAdd(p.stats + (long long)cloud * (p.n_out / 12) * 2 + gidx, static_cast<double>(mine));
+    auto round = [&](auto kr) {
+      constexpr int r = decltype(kr)::value;
+      constexpr int N = Stats::width(r);
+      const float mine = warp_reduce_scatter<N, 32 * r>(st, t.lane);
+      const int s = 32 * r + (N == 32 ? t.lane : (t.lane & (N - 1)));  // this lane's slot
+      // [group][{sum, sumsq}] of the cloud
+      const int gidx = Stats::kLocal ? (n0 / W) * 2 + (2 * (s / (64 / W)) + t.grp) * (64 / W) + s % (64 / W)
+                                     : (n0 / W) * 2 + s;
+      const bool own = (N == 32 && 32 * r + 32 <= Stats::kSlots) || (t.lane < N && s < Stats::kSlots);
+      if (own && gidx < (p.n_out / W) * 2 && m0 + t.q * 32 < p.M)
+        if (!(p.skip & 8)) atomicAdd(p.stats + (long long)cloud * (p.n_out / W) * 2 + gidx, static_cast<double>(mine));
+    };
+    round(std::integral_constant<int, 0>{});
+    if constexpr (Stats::kRounds > 1) round(std::integral_constant<int, 1>{});
+    static_assert(Stats::kRounds <= 2, "at most two reduce-scatter rounds");
     if (GECCO_DBG_ON(p.dbg) && t.lane == 0 && t.q == 0 && t.grp == 0) p.dbg[(long long)blockIdx.x * 32 + 20] += clock64() - ts0__;
   }
 }

@@ -400,7 +400,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             if (et.lane == 0) mbar_arrive_leader(&acc_empty[slot]);  // one (remote) arrival per warp
           });
         } else {
-          epi_panel<kStats>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, nb * BN, cnt);
+          epi_panel<kStats ? 12 : 0>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, nb * BN, cnt);
           tc_fence_before_sync();
           __syncwarp();
           if (et.lane == 0) mbar_arrive_leader(&acc_empty[slot]);  // one (remote) arrival per warp
@@ -444,6 +444,7 @@ int launch_gemm_pair(const gecco_gemm_args& a, cudaStream_t stream, int* handled
   *handled = 0;
   const int sms = sm_count();
   if (!gemm_pair_shape_ok(a.m, a.rows_per_cloud, a.n_out, a.k)) return GECCO_OK;
+  if (a.stats != nullptr && epi_stat_width(a) != 12) return GECCO_OK;  // statistics epilogue built for 12-channel groups only
   const bool anorm = a.anorm.stats != nullptr;
   if (anorm) {
     GECCO_REQUIRE(a.k % BK == 0, "gemm: A-operand normalisation needs k %% 64 == 0 (got %d)", a.k);

@@ -7,6 +7,8 @@
 //   warps 4-11 : epilogue  (epilogue.cuh: tcgen05.ld -> bias / xyz-embed / activation / residual /
 //                           AdaGN statistics -> swizzled smem staging -> TMA bulk stores, fp32 and/or bf16;
 //                           two groups of 4 warps on alternate 32-column chunks)
+// One instantiation per AdaGN statistics width W (0: no statistics; 4, 8, 12, 16, 24, 32 channels: C / 32 for
+// C = 128 ... 1024).
 // The two TMEM slots let the epilogue of tile i overlap the main loop of tile i+1.
 #include "common.cuh"
 #include "epilogue.cuh"
@@ -41,7 +43,7 @@ struct KParams {
   int stages;
 };
 
-template <bool kStats>
+template <int W>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
                const __grid_constant__ CUtensorMap tma_res, const __grid_constant__ CUtensorMap tma_o32,
@@ -181,7 +183,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
       mbar_wait(&acc_full[slot], acc_phase);
       tc_fence_after_sync();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * ACC_COLS;
-      epi_panel<kStats>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, n0, cnt);
+      epi_panel<W>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, n0, cnt);
       tc_fence_before_sync();
       __syncwarp();
       if (et.lane == 0) mbar_arrive(&acc_empty[slot]);  // one arrival per warp
@@ -318,7 +320,11 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
                 a.rows_per_cloud);
   GECCO_REQUIRE(a.valid_rows > 0 && a.valid_rows <= a.rows_per_cloud, "gemm: valid_rows out of range");
   GECCO_REQUIRE(a.out_f32 || a.out_bf16, "gemm: no output buffer");
-  GECCO_REQUIRE(!a.stats || a.n_out % 12 == 0, "gemm: statistics epilogue needs n_out %% 12 == 0");
+  const int stat_w = epi_stat_width(a);
+  GECCO_REQUIRE(!a.stats || epi_stat_width_supported(stat_w),
+                "gemm: statistics width (stat_gs) must be 4, 8, 12, 16, 24 or 32 channels (got %d)", stat_w);
+  GECCO_REQUIRE(!a.stats || a.n_out % stat_w == 0, "gemm: statistics epilogue needs n_out (%d) %% stat_gs (%d) == 0", a.n_out,
+                stat_w);
   GECCO_REQUIRE(!a.geom || (a.sigma && a.wx), "gemm: xyz embed needs sigma and wx");
   GECCO_REQUIRE(!a.w_rows_per_cloud || a.rows_per_cloud % BM == 0,
                 "gemm: per-cloud weights need rows_per_cloud %% 128 == 0");
@@ -326,6 +332,8 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   GECCO_REQUIRE(a.anorm.stats == nullptr || gemm_anorm_supported(a.m, a.rows_per_cloud, a.n_out, a.k),
                 "gemm: A-operand normalisation is not available for this shape (m=%d rows_per_cloud=%d n_out=%d k=%d): see "
                 "gecco_gemm_anorm_supported", a.m, a.rows_per_cloud, a.n_out, a.k);
+  GECCO_REQUIRE(a.anorm.stats == nullptr || !a.stats || stat_w == 12,
+                "gemm: A-operand normalisation combined with statistics needs stat_gs == 12 (got %d)", stat_w);
   GECCO_REQUIRE(a.a != nullptr, "gemm: null operand");
   if (g_use_pairs) {
     int handled = 0;
@@ -361,13 +369,19 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
   const int smem_bytes = SMEM_FIXED + epi_bytes + p.stages * (A_STAGE_BYTES + B_STAGE_BYTES);
 
+  using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, KParams);
+  static const KernelFn kernels[7] = {gemm_tc_kernel<0>,  gemm_tc_kernel<4>,  gemm_tc_kernel<8>, gemm_tc_kernel<12>,
+                                      gemm_tc_kernel<16>, gemm_tc_kernel<24>, gemm_tc_kernel<32>};
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
-    if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(gemm_tc_kernel)");
+    for (KernelFn k : kernels) {
+      cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
+      if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(gemm_tc_kernel)");
+    }
     attr_set = true;
   }
+  const KernelFn kernel = !a.stats ? kernels[0] : stat_w == 4 ? kernels[1] : stat_w == 8 ? kernels[2] : stat_w == 12 ? kernels[3]
+                          : stat_w == 16 ? kernels[4] : stat_w == 24 ? kernels[5] : kernels[6];
   const int tiles = p.num_m_blocks * p.num_n_blocks;
   const int grid = tiles < sm_count() ? tiles : sm_count();
   cudaLaunchConfig_t cfg = {};
@@ -380,8 +394,7 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t le = a.stats ? cudaLaunchKernelEx(&cfg, gemm_tc_kernel<true>, ta, tw, tres, t32, t16, p)
-                           : cudaLaunchKernelEx(&cfg, gemm_tc_kernel<false>, ta, tw, tres, t32, t16, p);
+  cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, ta, tw, tres, t32, t16, p);
   if (le != cudaSuccess) return fail_cuda(le, "gemm_tc_kernel launch");
   GECCO_CHECK_LAUNCH("gemm_tc_kernel launch");
   return GECCO_OK;

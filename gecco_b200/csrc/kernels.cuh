@@ -23,6 +23,11 @@ bool g_use_pairs_ref();
 void set_fast_epilogue_option(int value);  // gemm_pair.cu: gecco_set_option("fast_epilogue", v)
 
 int launch_gemm(const gecco_gemm_args& a, cudaStream_t s);
+// AdaGN statistics widths the single-CTA GEMM epilogue is instantiated for (those dividing its 192-column panel: C / 32
+// for C = 128 ... 1024), and the width of a gecco_gemm / gecco_mlp call (stat_gs; 0 means 12).
+inline bool epi_stat_width_supported(int w) { return w == 4 || w == 8 || w == 12 || w == 16 || w == 24 || w == 32; }
+template <typename Args>
+inline int epi_stat_width(const Args& a) { return a.stat_gs != 0 ? a.stat_gs : 12; }
 void set_graphs_option(int value);  // engine.cu: gecco_set_option("graphs", v)
 void set_chain_option(int value);  // engine.cu: gecco_set_option("chain", v)
 void set_anorm_option(int value);  // engine.cu: gecco_set_option("anorm", v)

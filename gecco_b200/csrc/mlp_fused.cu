@@ -368,10 +368,10 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
       long long t_epi = 0;
       if (GECCO_DBG_ON(p.dbg)) t_epi = clock64();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-      epi_panel<kStats>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, 0, cnt);
+      epi_panel<kStats ? 12 : 0>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, 0, cnt);
       __syncwarp();
       epi_prefetch(p.e, et, m0, EPI_PANEL);
-      epi_panel<kStats>(p.e, es, et, &tma_o32, &tma_o16, taddr + EPI_PANEL, m0, EPI_PANEL, cnt);
+      epi_panel<kStats ? 12 : 0>(p.e, es, et, &tma_o32, &tma_o16, taddr + EPI_PANEL, m0, EPI_PANEL, cnt);
       tc_fence_before_sync();
       if (lane == 0) tma_store_wait_read<0>();  // the staging areas (= hidden chunk buffer, W2 ring) are free again
       __syncwarp();
@@ -401,15 +401,16 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 
 static bool mlp_fused_supported(const gecco_mlp_args& a) {
   return a.c == C && a.hidden >= HC && a.hidden % HC == 0 && a.m > 0 && a.m % (2 * BM) == 0 &&
-         a.rows_per_cloud % (2 * BM) == 0 && sm_count() >= 2;
+         a.rows_per_cloud % (2 * BM) == 0 && (a.stats == nullptr || epi_stat_width(a) == 12) && sm_count() >= 2;
 }
 
 static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
   GECCO_REQUIRE(a.a && a.w1 && a.w2 && a.b1 && a.b2, "mlp: null operand");
   GECCO_REQUIRE(a.res && a.out_f32, "mlp: the fp32 residual stream (res, out_f32) is required");
   GECCO_REQUIRE(mlp_fused_supported(a),
-                "mlp: fused kernel needs c == 384, hidden %% 128 == 0, m %% 256 == 0 and rows_per_cloud %% 256 == 0 "
-                "(c=%d hidden=%d m=%d rows_per_cloud=%d)", a.c, a.hidden, a.m, a.rows_per_cloud);
+                "mlp: fused kernel needs c == 384, hidden %% 128 == 0, m %% 256 == 0, rows_per_cloud %% 256 == 0 and "
+                "12-channel statistics (c=%d hidden=%d m=%d rows_per_cloud=%d stat_gs=%d)", a.c, a.hidden, a.m, a.rows_per_cloud,
+                a.stat_gs);
   GECCO_REQUIRE(a.valid_rows > 0 && a.valid_rows <= a.rows_per_cloud, "mlp: valid_rows out of range");
   GECCO_REQUIRE(a.act_alpha != 0.f, "mlp: act_alpha must be non-zero");
 

@@ -203,7 +203,7 @@ __device__ __forceinline__ void epi_panel_ldg(const MParams& p, const EpiThread&
   step(std::integral_constant<int, 1>{});
   step(std::integral_constant<int, 2>{});
   if constexpr (kStats) {
-    const float mine = warp_reduce_scatter32(st, t.lane);
+    const float mine = warp_reduce_scatter<32, 0>(st, t.lane);
     const int gidx = (n0 / 12) * 2 + t.lane;  // [group][{sum, sumsq}]
     atomicAdd(e.stats + (long long)cloud * (e.n_out / 12) * 2 + gidx, static_cast<double>(mine));
   }
@@ -553,7 +553,8 @@ bool mlp_pair_supported(const gecco_mlp_args& a) {
   return a.anorm.stats != nullptr && a.c == C && a.hidden == HID && a.m > 0 && a.m % (2 * BM) == 0 &&
          a.rows_per_cloud % (2 * BM) == 0 && a.w1_rows_per_cloud == 0 && a.scratch != nullptr && a.res != nullptr &&
          a.out_f32 != nullptr && a.out_bf16 != nullptr && a.anorm.groups > 0 && a.anorm.groups <= 128 && C % a.anorm.groups == 0 &&
-         a.anorm.stat_gs > 0 && (C / a.anorm.groups) % a.anorm.stat_gs == 0 && sm_count() >= 2 && g_use_pairs_ref();
+         a.anorm.stat_gs > 0 && (C / a.anorm.groups) % a.anorm.stat_gs == 0 && (a.stats == nullptr || epi_stat_width(a) == 12) &&
+         sm_count() >= 2 && g_use_pairs_ref();
 }
 
 int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {

@@ -42,6 +42,7 @@ def gemm(
     out_f32: Tensor | bool | None = None,
     out_bf16: Tensor | bool | None = None,
     stats: Tensor | None = None,
+    stat_gs: int = 12,
     rows_per_cloud: int | None = None,
     valid_rows: int | None = None,
     w_rows_per_cloud: int = 0,
@@ -54,6 +55,7 @@ def gemm(
     anorm: dict | None = None,
 ):
     """out = epilogue(a @ w.T) on the tcgen05 tensor cores; see gecco_gemm in include/gecco_b200.h.
+    stats (f64 [clouds, n_out / stat_gs, 2]) receives the AdaGN statistics per group of stat_gs channels (4, 8, 12, 16, 24 or 32).
     anorm = dict(stats f64 [clouds, K/stat_gs, 2], t fp32 [clouds], scale_w, scale_b, bias_w, bias_b, groups, stat_gs=12,
     eps=1e-5): `a` is the un-normalised bf16 tensor and AdaGN is applied to it inside the kernel."""
     assert a.dtype == torch.bfloat16
@@ -102,7 +104,7 @@ def gemm(
         args.out_bf16, args.ldo16 = out_bf16.data_ptr(), out_bf16.stride(0)
     if stats is not None:
         assert stats.dtype == torch.float64 and stats.is_contiguous()
-        args.stats = stats.data_ptr()
+        args.stats, args.stat_gs = stats.data_ptr(), stat_gs
     if geom is not None:
         assert geom.dtype == torch.float32 and geom.is_contiguous()
         assert sigma is not None and wx is not None and sigma.dtype == torch.float32 and wx.dtype == torch.float32
@@ -186,7 +188,7 @@ def gaussian_activation(x: Tensor, alpha: float, normalized: bool = True) -> Ten
     return out.to(x.dtype)
 
 
-STAT_GS = 12  # channel granularity of the AdaGN statistics kept by the GEMM epilogue (C / 32 for C = 384)
+STAT_GS = 12  # default channel granularity of the AdaGN statistics kept by the GEMM epilogue (C / 32 for C = 384)
 
 
 def group_stats(x: Tensor, rows_per_cloud: int, valid_rows: int, group_size: int, stats: Tensor | None = None) -> Tensor:

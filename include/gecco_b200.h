@@ -66,8 +66,8 @@ int gecco_set_option(const char* name, int value);
  *   + xyz embed: sum_j c_in(sigma)*geom[point,j]*wx[n,j]  (geom may be NULL; models/ray.py:99,113)
  *   Gaussian activation (exp(-z^2/(2 alpha^2)) - 0.7)/0.28 when act != 0 (models/activation.py:17-24)
  *   + res[m, n]                                       (res may be NULL; residual adds set_transformer.py:164,166)
- *   per (cloud, 12-channel group) sum / sum of squares of the result added into
- *   stats (double [clouds][n_out/12][2]) for the next AdaGN (models/normalization.py:36-44)
+ *   per (cloud, stat_gs-channel group) sum / sum of squares of the result added into
+ *   stats (double [clouds][n_out/stat_gs][2]) for the next AdaGN (models/normalization.py:36-44)
  * and written as fp32 (out_f32) and/or bf16 (out_bf16).
  * Rows are grouped in clouds of rows_per_cloud rows of which the first valid_rows
  * are real points (the rest is padding, excluded from stats).
@@ -103,6 +103,8 @@ typedef struct gecco_gemm_args {
   const float* sigma; int32_t sigma_stride; float sigma_data; /* sigma[cloud*sigma_stride] */
   const float* wx;          /* [n_out, 3] fp32 */
   gecco_anorm anorm;        /* anorm.stats == NULL: `a` is used as it is */
+  int32_t stat_gs;          /* channels per statistics group: 4, 8, 12, 16, 24 or 32 (0: 12); n_out % stat_gs == 0.
+                             * The CTA-pair kernel (and so anorm together with stats) takes 12 only. */
 } gecco_gemm_args;
 
 int gecco_gemm(const gecco_gemm_args* args, void* stream);
@@ -142,6 +144,7 @@ typedef struct gecco_mlp_args {
                        * w1_rows_per_cloud == 0); needs `scratch` */
   void* scratch;      /* anorm path: bf16 device scratch of min(m, 128 * #SMs) x hidden elements: the hidden activation of
                        * the row block a CTA is working on (rewritten every row block: L2-resident, never read after the call) */
+  int32_t stat_gs;    /* channels per statistics group: 0 or 12 (the only width these kernels are built for) */
 } gecco_mlp_args;
 
 int gecco_mlp(const gecco_mlp_args* args, void* stream);
@@ -354,7 +357,7 @@ int gecco_inducer_chain(const gecco_chain_args* args, void* stream);
 typedef struct gecco_model_desc {
   int32_t kind;          /* 0: LinearLift (models/linear_lift.py), 1: RayNetwork (models/ray.py) */
   int32_t n_layers, feature_dim, num_heads, num_inducers, mlp_hidden;
-  int32_t adagn_groups;  /* 32 (models/normalization.py:19) */
+  int32_t adagn_groups;  /* 32 (models/normalization.py:19); feature_dim / adagn_groups in {4, 8, 12, 16, 24, 32} */
   int32_t head_norm;     /* 0 none, 1 LayerNorm (linear_lift.py:26-29), 2 GroupNorm over points (ray.py:56-59) */
   int32_t head_groups;   /* 16 */
   int32_t img_groups;    /* 16 (ray.py:53) */
@@ -393,7 +396,11 @@ enum gecco_layer_weight {      /* `layers.{l}.` + ...  (models/set_transformer.p
 
 typedef struct gecco_engine gecco_engine;
 
-/* Packs the fp32 weights into the kernel layouts (bf16 operands, folded softmax scale).  The fp32 arrays
+/* Accepted models: feature_dim C a multiple of 128 up to 1024 whose AdaGN groups (C / adagn_groups channels) are 4, 8,
+ * 12, 16, 24 or 32 channels wide -- with the reference's 32 groups, C = 128, 256, 384, 512, 768 or 1024; head dim
+ * C / num_heads of 32, 48 or 64; 64 inducers; mlp_hidden a multiple of 8; a head GroupNorm whose groups are multiples of
+ * the AdaGN group width.  Anything else returns GECCO_ERR_INVALID with a message naming the parameter.
+ * Packs the fp32 weights into the kernel layouts (bf16 operands, folded softmax scale).  The fp32 arrays
  * that are used in place (biases, AdaGN linears, embed / head weights) must stay alive and unchanged
  * until gecco_destroy; re-create the handle after a weight update.  Synchronises `stream` once. */
 int gecco_create(const gecco_model_desc* desc, const float* const* net_weights /* [GECCO_NW_COUNT] */,
