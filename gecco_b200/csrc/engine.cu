@@ -182,7 +182,8 @@ Workspace carve(const gecco_engine* e, int clouds, int points, void* base) {
   w.Np = ceil_div(points, 128) * 128;
   w.rows = clouds * w.Np;
   w.irows = clouds * I;
-  w.splits = pool_splits(clouds, d.num_heads, ceil_div(points, 64));
+  // the mma.sync pool core runs one CTA per 64 inducers of each split
+  w.splits = pool_splits(clouds, d.num_heads * (I / 64), ceil_div(points, 64));
   int wide = 3 * C;
   if (hid > wide) wide = hid;
   if (ctx > wide) wide = ctx;
@@ -597,7 +598,8 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
   GECCO_REQUIRE(C > 0 && C % 128 == 0 && C <= 1024, "gecco_create: feature_dim must be a multiple of 128 (<= 1024), got %d", C);
   GECCO_REQUIRE(H > 0 && C % H == 0 && (C / H == 32 || C / H == 48 || C / H == 64),
                 "gecco_create: head dim must be 32, 48 or 64 (feature_dim %d, heads %d)", C, H);
-  GECCO_REQUIRE(I == 64, "gecco_create: only 64 inducers are supported (got %d)", I);
+  // whole blocks of 64 inducers (the query rows of one pool CTA, the key chunk of the unpool core), up to 256
+  GECCO_REQUIRE(I >= 64 && I <= 256 && I % 64 == 0, "gecco_create: num_inducers must be 64, 128, 192 or 256 (got %d inducers)", I);
   // The GEMM epilogues keep the AdaGN statistics per group of C / adagn_groups channels; they are instantiated for the
   // widths that divide their 192-column panel.
   GECCO_REQUIRE(d.adagn_groups > 0 && C % d.adagn_groups == 0 && epi_stat_width_supported(C / d.adagn_groups),

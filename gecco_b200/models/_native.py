@@ -15,6 +15,7 @@ from torch import Tensor
 from .. import ops
 
 ROW_TILE = 128  # rows per cloud are padded to the row tile of the tcgen05 kernels
+SUPPORTED_INDUCERS = (64, 128, 192, 256)  # whole 64-row blocks of the attention cores
 _LOG2E = 1.4426950408889634
 
 
@@ -98,8 +99,8 @@ def unpool_forward(mha, x: Tensor, h: Tensor, residual: Tensor | None = None) ->
     H = mha.num_heads
     d = C // H
     I = h.shape[1]
-    if I != 64:
-        raise ValueError(f"gecco_b200: the unpool attention kernels support 64 inducers, got {I}")
+    if I not in SUPPORTED_INDUCERS:
+        raise ValueError(f"gecco_b200: the unpool attention kernels support 64, 128, 192 or 256 inducers, got {I}")
     a, N, Np = pad_rows(x)
     w, b = mha.in_proj_weight, mha.in_proj_bias
     qs = _LOG2E / math.sqrt(d)

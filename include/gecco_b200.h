@@ -285,9 +285,9 @@ int gecco_pack_features(const float* nchw, void* nhwc_bf16, int32_t images, int3
  * AttentionPool's scaled_dot_product_attention with the learned inducer queries
  * (models/set_transformer.py:57-63).  kv holds the bf16 kv_proj output, K of head h at
  * columns k_off + h*head_dim, V at v_off + h*head_dim ("b n (t h d)" layout, :50-55).
- * q_inducers: bf16 [heads][64][head_dim] = inducers * (head_dim^-0.5 * log2 e).
+ * inducers I: 64, 128, 192 or 256.  q_inducers: bf16 [heads][I][head_dim] = inducers * (head_dim^-0.5 * log2 e).
  * The keys are processed in `splits` ranges; partial is scratch of
- * clouds*heads*splits*64*(head_dim+2) floats.  out: bf16 [clouds*64, heads*head_dim]
+ * clouds*heads*splits*I*(head_dim+2) floats.  out: bf16 [clouds*I, heads*head_dim]
  * ("b h i d -> b i (h d)", :63), the operand of out_proj.
  * ------------------------------------------------------------------------ */
 typedef struct gecco_pool_args {
@@ -305,9 +305,9 @@ int gecco_pool_attention_partial(const gecco_pool_args* args, int32_t* splits_us
 
 /* Attention core of Broadcast.unpool = nn.MultiheadAttention(query=points, key=value=inducers)
  * (models/set_transformer.py:90,112) between the in- and out-projections: per head
- * softmax(q k^T) v over the 64 inducers.  q: bf16 rows [clouds*rows_per_cloud] with head h at
+ * softmax(q k^T) v over the I inducers (64, 128, 192 or 256).  q: bf16 rows [clouds*rows_per_cloud] with head h at
  * columns h*head_dim, already multiplied by head_dim^-0.5 * log2 e (folded into the q
- * projection); kv: bf16 [clouds*64, *] with k at column h*head_dim and v at v_off + h*head_dim. */
+ * projection); kv: bf16 [clouds*I, *] with k at column h*head_dim and v at v_off + h*head_dim. */
 typedef struct gecco_unpool_args {
   const void* q; int64_t ldq;
   const void* kv; int64_t ldkv; int32_t v_off;
@@ -315,8 +315,8 @@ typedef struct gecco_unpool_args {
   int32_t heads, head_dim, inducers;
   void* out_bf16; int64_t ldo;
   void* vt_scratch;   /* optional bf16 [clouds * heads * head_dim * inducers] device scratch (v transposed per cloud): when given
-                       * and heads == 8, head_dim == 48, rows_per_cloud % 128 == 0 the tcgen05 / TMEM kernel runs, otherwise
-                       * (NULL or other shapes) the mma.sync kernel */
+                       * and heads == 8, head_dim == 48, inducers == 64, rows_per_cloud % 128 == 0 the tcgen05 / TMEM kernel
+                       * runs, otherwise (NULL or other shapes) the mma.sync kernel */
   int32_t vt_ready;   /* nonzero: vt_scratch already holds V transposed (written by gecco_inducer_chain) */
 } gecco_unpool_args;
 int gecco_unpool_attention(const gecco_unpool_args* args, void* stream);
@@ -398,8 +398,9 @@ typedef struct gecco_engine gecco_engine;
 
 /* Accepted models: feature_dim C a multiple of 128 up to 1024 whose AdaGN groups (C / adagn_groups channels) are 4, 8,
  * 12, 16, 24 or 32 channels wide -- with the reference's 32 groups, C = 128, 256, 384, 512, 768 or 1024; head dim
- * C / num_heads of 32, 48 or 64; 64 inducers; mlp_hidden a multiple of 8; a head GroupNorm whose groups are multiples of
- * the AdaGN group width.  Anything else returns GECCO_ERR_INVALID with a message naming the parameter.
+ * C / num_heads of 32, 48 or 64; num_inducers 64, 128, 192 or 256; mlp_hidden a multiple of 8; a head GroupNorm whose
+ * groups are multiples of the AdaGN group width.  Anything else returns GECCO_ERR_INVALID with a message naming the
+ * parameter.
  * Packs the fp32 weights into the kernel layouts (bf16 operands, folded softmax scale).  The fp32 arrays
  * that are used in place (biases, AdaGN linears, embed / head weights) must stay alive and unchanged
  * until gecco_destroy; re-create the handle after a weight update.  Synchronises `stream` once. */
