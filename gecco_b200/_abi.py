@@ -18,6 +18,10 @@ class GeccoError(RuntimeError):
     pass
 
 
+# activation codes (GECCO_ACT_*)
+ACT_NONE, ACT_GAUSSIAN, ACT_GAUSSIAN_RAW, ACT_RELU = 0, 1, 2, 3
+
+
 class ANorm(C.Structure):
     _fields_ = [
         ("stats", C.c_void_p), ("stat_gs", C.c_int32), ("groups", C.c_int32), ("eps", C.c_float),
@@ -63,6 +67,7 @@ class MlpArgs(C.Structure):
         ("anorm", ANorm),
         ("scratch", C.c_void_p),
         ("stat_gs", C.c_int32),
+        ("act", C.c_int32),
     ]
 
 
@@ -184,6 +189,7 @@ class ChainArgs(C.Structure):
         ("t", C.c_void_p), ("t_stride", C.c_int32), ("eps", C.c_float),
         ("hn", C.c_void_p), ("hh", C.c_void_p), ("h3", C.c_void_p), ("khv", C.c_void_p), ("vt", C.c_void_p),
         ("cache_out", C.c_void_p),
+        ("act", C.c_int32),
     ]
 
 
@@ -200,6 +206,7 @@ class ModelDesc(C.Structure):
         ("reparam", C.c_int32),
         ("mean", C.c_float * 3), ("sigma", C.c_float * 3), ("logit_scale", C.c_float),
         ("sigma_data", C.c_float),
+        ("mlp_act", C.c_int32),
     ]
 
 

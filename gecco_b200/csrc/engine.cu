@@ -304,6 +304,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
   const gecco_model_desc& d = e->d;
   const int C = d.feature_dim, I = d.num_inducers, H = d.num_heads, hid = d.mlp_hidden, hd = C / H;
   const int sg = d.adagn_groups, Np = w.Np, rows = w.rows, irows = w.irows;
+  const int act = mlp_act_of(d.mlp_act);  // every MLP's hidden activation, in the epilogue of its first projection
   const long long per_norm = (long long)clouds * sg * 2;
   const float sigma_data = t_embed ? 1.f : d.sigma_data;
   // algorithmic work per launch (profiling only)
@@ -420,7 +421,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     ch.pooled = w.pooled;
     ch.w_pool_out = L.pool_out_w; ch.w_mlp0 = L.bmlp_w0; ch.w_mlp2 = L.bmlp_w2; ch.w_kv = L.kv_w;
     ch.b_mlp0 = lw[GECCO_LW_BMLP_B0]; ch.b_mlp2 = lw[GECCO_LW_BMLP_B2]; ch.b_kv = lw[GECCO_LW_UNPOOL_IN_B] + C;
-    ch.act_alpha = L.bmlp_alpha;
+    ch.act_alpha = L.bmlp_alpha; ch.act = act;
     for (int i = 0; i < 4; ++i) { ch.norm[0][i] = lw[GECCO_LW_N1 + i]; ch.norm[1][i] = lw[GECCO_LW_N2 + i]; }
     ch.t = w.c_noise; ch.t_stride = 1; ch.eps = 1e-5f;
     // key / value projections of this layer's inducer states: the workspace buffers, or the per-layer slots of the
@@ -456,7 +457,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       a.out_bf16 = w.hn; a.ldo16 = C;
       TRYP(K_INDUCER_CHAIN, 2 * Mi * Cd, Mi * Cd * 6, launch_adagn(a, s));
       g = gemm_base(w.hn, C, L.bmlp_w0, C, irows, hid, C, I, I);
-      g.bias = lw[GECCO_LW_BMLP_B0]; g.act = 1; g.act_alpha = L.bmlp_alpha;
+      g.bias = lw[GECCO_LW_BMLP_B0]; g.act = act; g.act_alpha = L.bmlp_alpha;
       g.out_bf16 = w.hh; g.ldo16 = hid;
       TRYP(K_INDUCER_CHAIN, 2 * Mi * Cd * Hd, Mi * (Cd + Hd) * 2 + 2 * Cd * Hd, launch_gemm(g, s));
       g = gemm_base(w.hh, hid, L.bmlp_w2, hid, irows, C, hid, I, I);
@@ -511,7 +512,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     if (an) {
       mp.a = w.xb; mp.lda = C;
       mp.w1 = L.mlp_w0; mp.ldw1 = C; mp.b1 = lw[GECCO_LW_MLP_B0];
-      mp.act_alpha = L.mlp_alpha;
+      mp.act_alpha = L.mlp_alpha; mp.act = act;
       mp.w2 = L.mlp_w2; mp.ldw2 = hid; mp.b2 = lw[GECCO_LW_MLP_B2];
       mp.m = rows; mp.c = C; mp.hidden = hid; mp.rows_per_cloud = Np; mp.valid_rows = points;
       mp.res = w.x; mp.ldr = C; mp.out_f32 = w.x; mp.ldo32 = C; mp.out_bf16 = xb_out; mp.ldo16 = C;
@@ -528,7 +529,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
     } else if (an) {
       gecco_gemm_args g = gemm_base(w.xb, C, L.mlp_w0, C, rows, hid, C, Np, points);
       set_anorm(g, lw + GECCO_LW_MN, stat(l, 3));
-      g.bias = lw[GECCO_LW_MLP_B0]; g.bias_stride = 0; g.act = 1; g.act_alpha = L.mlp_alpha;
+      g.bias = lw[GECCO_LW_MLP_B0]; g.bias_stride = 0; g.act = act; g.act_alpha = L.mlp_alpha;
       g.out_bf16 = w.big; g.ldo16 = hid;
       TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd * 2 + Hd * 2) + 2.0 * Cd * Hd, launch_gemm(g, s));
       g = gemm_base(w.big, hid, L.mlp_w2, hid, rows, C, hid, Np, points);
@@ -545,7 +546,7 @@ int run_eval(gecco_engine* e, const Workspace& w, const float* xin, const float*
       TRYP(K_FOLD_ADAGN, 2.0 * clouds * Hd * Cd, Hd * Cd * (4.0 + 2.0 * clouds), launch_fold_adagn(f, s));
       gecco_gemm_args g = gemm_base(w.xb, C, w.wfold, C, rows, hid, C, Np, points);
       g.w_rows_per_cloud = hid;
-      g.bias = w.bfold; g.bias_stride = hid; g.act = 1; g.act_alpha = L.mlp_alpha;
+      g.bias = w.bfold; g.bias_stride = hid; g.act = act; g.act_alpha = L.mlp_alpha;
       g.out_bf16 = w.big; g.ldo16 = hid;
       TRYP(K_GEMM_MLP0, 2 * Mv * Cd * Hd, Mv * (Cd + Hd) * 2 + 2.0 * clouds * Cd * Hd, launch_gemm(g, s));
       g = gemm_base(w.big, hid, L.mlp_w2, hid, rows, C, hid, Np, points);
@@ -606,6 +607,9 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
                 "gecco_create: feature_dim %d is not supported with %d AdaGN groups: the groups must be 4, 8, 12, 16, 24 or "
                 "32 channels wide (feature_dim 128, 256, 384, 512, 768 or 1024 with 32 groups)", C, d.adagn_groups);
   GECCO_REQUIRE(hid > 0 && hid % 8 == 0, "gecco_create: mlp_hidden must be a multiple of 8");
+  const int act = mlp_act_of(d.mlp_act);
+  GECCO_REQUIRE(act == GECCO_ACT_GAUSSIAN || act == GECCO_ACT_GAUSSIAN_RAW || act == GECCO_ACT_RELU,
+                "gecco_create: unknown MLP activation %d (supported: 1 normalised Gaussian, 2 raw Gaussian, 3 ReLU)", d.mlp_act);
   GECCO_REQUIRE(d.head_norm >= 0 && d.head_norm <= 2, "gecco_create: bad head_norm");
   GECCO_REQUIRE(d.head_norm != 2 || (d.head_groups > 0 && C % d.head_groups == 0 && (C / d.head_groups) % (C / d.adagn_groups) == 0),
                 "gecco_create: head GroupNorm groups must be multiples of the AdaGN group width (%d channels)", C / d.adagn_groups);
@@ -622,7 +626,8 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
   for (int i : {GECCO_NW_EMBED_W, GECCO_NW_EMBED_B, GECCO_NW_OUT_W, GECCO_NW_OUT_B})
     GECCO_REQUIRE(net_weights[i] != nullptr, "gecco_create: network weight %d missing", i);
   for (int i = 0; i < d.n_layers * GECCO_LW_COUNT; ++i)
-    GECCO_REQUIRE(layer_weights[i] != nullptr, "gecco_create: layer weight %d (layer %d, slot %d) missing", i,
+    GECCO_REQUIRE(layer_weights[i] != nullptr ||
+                      (!act_is_gaussian(act) && (i % GECCO_LW_COUNT == GECCO_LW_BMLP_ALPHA || i % GECCO_LW_COUNT == GECCO_LW_MLP_ALPHA)), "gecco_create: layer weight %d (layer %d, slot %d) missing", i,
                   i / GECCO_LW_COUNT, i % GECCO_LW_COUNT);
 
   int dev = 0;
@@ -661,7 +666,7 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
   };
   // softmax scale and the exp -> exp2 change of base folded into the query side of both attentions
   const float qscale = (float)(1.4426950408889634 / sqrt((double)(C / H)));
-  std::vector<float> alphas(2 * d.n_layers);
+  std::vector<float> alphas(2 * d.n_layers, 0.f);  // ReLU reads no alpha
   for (int l = 0; l < d.n_layers; ++l) {
     const float* const* lw = layer_weights + (size_t)l * GECCO_LW_COUNT;
     gecco_engine::Layer& L = e->layers[l];
@@ -681,8 +686,10 @@ extern "C" int gecco_create(const gecco_model_desc* desc, const float* const* ne
     scale_add_f32_kernel<<<ceil_div(C, 256), 256, 0, s>>>(lw[GECCO_LW_UNPOOL_IN_B], nullptr, L.bcat + 2 * C, C, qscale);
     L.wcat16 = pack(L.wcat, (size_t)3 * C * C, 1.f);  // stream-ordered after the two kernels that fill wcat
     L.mlp_w0 = pack(lw[GECCO_LW_MLP_W0], (size_t)hid * C, 1.f);
-    cudaMemcpyAsync(&alphas[2 * l], lw[GECCO_LW_BMLP_ALPHA], sizeof(float), cudaMemcpyDeviceToHost, s);
-    cudaMemcpyAsync(&alphas[2 * l + 1], lw[GECCO_LW_MLP_ALPHA], sizeof(float), cudaMemcpyDeviceToHost, s);
+    if (act_is_gaussian(act)) {
+      cudaMemcpyAsync(&alphas[2 * l], lw[GECCO_LW_BMLP_ALPHA], sizeof(float), cudaMemcpyDeviceToHost, s);
+      cudaMemcpyAsync(&alphas[2 * l + 1], lw[GECCO_LW_MLP_ALPHA], sizeof(float), cudaMemcpyDeviceToHost, s);
+    }
   }
   e->img_bias = nullptr;
   if (d.kind == 1) {

@@ -1,6 +1,6 @@
 // Row-tile epilogue shared by the tcgen05 kernels: drains a 128-row x 192-column fp32 accumulator panel from
 // TMEM in 32-column chunks and applies, in this order,
-//   + bias[cloud][n]  + xyz embed  -> Gaussian activation -> + residual -> AdaGN statistics -> fp32 / bf16 stores.
+//   + bias[cloud][n]  + xyz embed  -> activation -> + residual -> AdaGN statistics -> fp32 / bf16 stores.
 // The statistics are per (cloud, group of W consecutive columns), W a compile-time parameter that divides the panel
 // (EpiStats below).
 // The TMEM layout gives every thread one ROW of the tile; global memory wants whole row segments per request, so all
@@ -33,8 +33,8 @@ struct EpiParams {
   int rows_per_cloud, valid_rows;
   const float* bias;  // [clouds][bias_stride] or nullptr
   int bias_stride;
-  int act;
-  float act_k;  // -log2(e) / (2 alpha^2)
+  int act;      // GECCO_ACT_*: the kernel's ACT template parameter applies it; at ACT == GECCO_ACT_GAUSSIAN, 0 means none
+  float act_k;  // -log2(e) / (2 alpha^2) (the Gaussians)
   int has_res;
   float* o32;           // fp32 output or nullptr (written through its tensor map)
   __nv_bfloat16* o16;   // bf16 output or nullptr
@@ -163,6 +163,16 @@ __device__ __forceinline__ float ex2_approx(float x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
+// The hidden projection's activation (include/gecco_b200.h GECCO_ACT_*) on accumulator + bias v, a compile-time choice of
+// each kernel instantiation; k = -log2(e) / (2 alpha^2).
+template <int ACT>
+__device__ __forceinline__ float epi_act(float v, float k) {
+  static_assert(ACT == GECCO_ACT_GAUSSIAN || ACT == GECCO_ACT_GAUSSIAN_RAW || ACT == GECCO_ACT_RELU, "activation code");
+  if constexpr (ACT == GECCO_ACT_GAUSSIAN) return fmaf(ex2_approx(v * v * k), 1.0f / 0.28f, -0.7f / 0.28f);
+  else if constexpr (ACT == GECCO_ACT_GAUSSIAN_RAW) return ex2_approx(v * v * k);
+  else return fmaxf(v, 0.f);
+}
+
 // 32 lanes x 32 consecutive 32-bit columns -> 32 registers per thread.
 __device__ __forceinline__ void tmem_ld32_issue(uint32_t addr, uint32_t (&r)[32]) {
   asm volatile(
@@ -256,8 +266,9 @@ __device__ __forceinline__ void epi_prefetch(const EpiParams& p, const EpiThread
   } while (0)
 
 // One 32-column chunk after its accumulator values (+ bias) are in registers.  C: chunk index inside the panel
-// (compile-time, so the AdaGN group of every column is static).  W: statistics width (0: none).
-template <int W, int C>
+// (compile-time, so the AdaGN group of every column is static).  W: statistics width (0: none).  ACT: the activation;
+// the Gaussian instantiation applies it when p.act != 0, the others always.
+template <int W, int C, int ACT = GECCO_ACT_GAUSSIAN>
 __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm, const EpiThread& t, float (&v)[EPI_CHUNK],
                                           int m0, int col0, bool rows_valid, bool row_valid, float g0, float g1, float g2,
                                           const CUtensorMap* tma_o32, const CUtensorMap* tma_o16,
@@ -275,9 +286,9 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm,
       }
     }
   }
-  if (p.act) {
+  if (ACT != GECCO_ACT_GAUSSIAN || p.act) {
 #pragma unroll
-    for (int j = 0; j < EPI_CHUNK; ++j) v[j] = fmaf(ex2_approx(v[j] * v[j] * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
+    for (int j = 0; j < EPI_CHUNK; ++j) v[j] = epi_act<ACT>(v[j], p.act_k);
   }
   // The previous chunk's bulk stores have finished reading their staging (its X buffer and the bf16 area): with a
   // residual that X buffer goes back to the loader, which refills it while this chunk is processed.
@@ -351,7 +362,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& p, const EpiSmem& sm,
 // must have been staged by this thread (epi_bias_stage / epi_prefetch).  The group's three chunks (grp, grp + 2, grp + 4) are software
 // pipelined: the TMEM load of the next chunk is issued as soon as the current one has been consumed, because
 // tcgen05.ld latency is several hundred cycles while the tensor core is streaming accumulators through TMEM.
-template <int W>
+template <int W, int ACT = GECCO_ACT_GAUSSIAN>
 __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm, const EpiThread& t,
                                           const CUtensorMap* tma_o32, const CUtensorMap* tma_o16, uint32_t taddr, int m0,
                                           int n0, uint32_t& cnt) {
@@ -403,11 +414,11 @@ __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm,
       const int col0 = n0 + (2 * k + t.grp) * EPI_CHUNK;
       if constexpr (W != 0) {  // the AdaGN group of every column must be static: one instantiation per chunk index
         if (t.grp == 0)
-          epi_chunk<W, 2 * k>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+          epi_chunk<W, 2 * k, ACT>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
         else
-          epi_chunk<W, 2 * k + 1>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+          epi_chunk<W, 2 * k + 1, ACT>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
       } else {
-        epi_chunk<0, 0>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
+        epi_chunk<0, 0, ACT>(p, sm, t, v, m0, col0, rows_valid, row_valid, g0, g1, g2, tma_o32, tma_o16, st, cnt);
       }
     }
   };
@@ -437,7 +448,7 @@ __device__ __forceinline__ void epi_panel(const EpiParams& p, const EpiSmem& sm,
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Fast path for the bf16-only projections (k|v|q, MLP up): bias (+ Gaussian activation) -> bf16, whole tiles only (all
+// Fast path for the bf16-only projections (k|v|q, MLP up): bias (+ activation ACT, GECCO_ACT_NONE: none) -> bf16, whole tiles only (all
 // 128 rows valid, n_out a multiple of the panel), no residual / statistics / fp32 copy / xyz embed.  Everything is
 // compile-time, the three chunks of a warp are drained from TMEM back to back (three tcgen05.ld in flight) and the
 // accumulator slot is handed back to the MMA issuer BEFORE the conversion and the stores; the three 32 x 32 bf16 blocks
@@ -454,7 +465,7 @@ constexpr int EPI_FAST_O16_BYTES = EPI_FAST_BUFS * EPI_O16_BYTES;  // per group:
 
 __host__ __device__ inline int epi_fast_smem_bytes() { return EPI_GROUPS * EPI_FAST_O16_BYTES + EPI_BIAS_BYTES; }
 
-template <bool kAct, typename ReleaseFn>
+template <int ACT, typename ReleaseFn>
 __device__ __forceinline__ void epi_tile_fast(const EpiParams& p, const EpiThread& t, const CUtensorMap* tma_o16, uint32_t taddr,
                                               int m0, int n0, uint32_t stage_base, bool row_valid, ReleaseFn release) {
   uint32_t rr[3][EPI_CHUNK];
@@ -477,11 +488,11 @@ __device__ __forceinline__ void epi_tile_fast(const EpiParams& p, const EpiThrea
     for (int j = 0; j < EPI_CHUNK / 4; ++j) {
       float v0 = __uint_as_float(rr[k][4 * j + 0]) + b[j].x, v1 = __uint_as_float(rr[k][4 * j + 1]) + b[j].y;
       float v2 = __uint_as_float(rr[k][4 * j + 2]) + b[j].z, v3 = __uint_as_float(rr[k][4 * j + 3]) + b[j].w;
-      if (kAct) {
-        v0 = fmaf(ex2_approx(v0 * v0 * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
-        v1 = fmaf(ex2_approx(v1 * v1 * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
-        v2 = fmaf(ex2_approx(v2 * v2 * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
-        v3 = fmaf(ex2_approx(v3 * v3 * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
+      if constexpr (ACT != GECCO_ACT_NONE) {
+        v0 = epi_act<ACT>(v0, p.act_k);
+        v1 = epi_act<ACT>(v1, p.act_k);
+        v2 = epi_act<ACT>(v2, p.act_k);
+        v3 = epi_act<ACT>(v3, p.act_k);
       }
       pw[2 * j] = zero_row ? 0u : pack_bf16x2(v0, v1);
       pw[2 * j + 1] = zero_row ? 0u : pack_bf16x2(v2, v3);

@@ -80,7 +80,9 @@ __device__ __forceinline__ int num_kb_of(const PParams& p) { return p.num_kb; }
     }                                       \
   } while (0)
 
-// kEpi: 0 generic epilogue, 1 generic + AdaGN statistics, 2 fast bf16-only epilogue (epi_tile_fast), 3 fast + Gaussian activation
+// kEpi: 0 generic epilogue (Gaussian activation when p.e.act != 0), 1 generic + AdaGN statistics, 2 fast bf16-only epilogue
+// (epi_tile_fast), 3 fast + Gaussian activation, 4 fast + raw Gaussian, 5 fast + ReLU, 6 generic + raw Gaussian,
+// 7 generic + ReLU
 template <int kEpi, bool kANorm>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
@@ -97,7 +99,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   uint8_t* sB = smem + MAX_KB * A_KB_BYTES + (kANorm ? ANORM_SMEM : 0);  // [BSTAGES] weight half-tiles, kbps k-blocks each
   uint8_t* sEpi = sB + BSTAGES * stage_bytes;
   constexpr bool kStats = kEpi == 1;
-  constexpr bool kFast = kEpi >= 2;
+  constexpr bool kFast = kEpi >= 2 && kEpi <= 5;
+  constexpr int kAct = kEpi == 2 ? GECCO_ACT_NONE : (kEpi == 4 || kEpi == 6) ? GECCO_ACT_GAUSSIAN_RAW
+                       : (kEpi == 5 || kEpi == 7) ? GECCO_ACT_RELU : GECCO_ACT_GAUSSIAN;
   EpiSmem es;
   uint64_t* bars;
   if constexpr (kFast) {
@@ -394,13 +398,13 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         if constexpr (kFast) {
           // a 128-row tile lies inside one cloud (rows_per_cloud % 256 == 0)
           const bool row_valid = (m0 % p.e.rows_per_cloud) + q * 32 + (int)et.lane < p.e.valid_rows;
-          epi_tile_fast<kEpi == 3>(p.e, et, &tma_o16, taddr, m0, nb * BN, smem_u32(es.o16), row_valid, [&] {
+          epi_tile_fast<kAct>(p.e, et, &tma_o16, taddr, m0, nb * BN, smem_u32(es.o16), row_valid, [&] {
             tc_fence_before_sync();
             __syncwarp();
             if (et.lane == 0) mbar_arrive_leader(&acc_empty[slot]);  // one (remote) arrival per warp
           });
         } else {
-          epi_panel<kStats ? 12 : 0>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, nb * BN, cnt);
+          epi_panel<kStats ? 12 : 0, kAct>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, nb * BN, cnt);
           tc_fence_before_sync();
           __syncwarp();
           if (et.lane == 0) mbar_arrive_leader(&acc_empty[slot]);  // one (remote) arrival per warp
@@ -471,7 +475,7 @@ int launch_gemm_pair(const gecco_gemm_args& a, cudaStream_t stream, int* handled
   p.e.rows_per_cloud = a.rows_per_cloud; p.e.valid_rows = a.valid_rows;
   p.e.bias = a.bias; p.e.bias_stride = a.bias_stride;
   p.e.act = a.act;
-  p.e.act_k = a.act ? static_cast<float>(-1.4426950408889634 / (2.0 * (double)a.act_alpha * (double)a.act_alpha)) : 0.f;
+  p.e.act_k = act_k_of(a.act, a.act_alpha);
   p.e.has_res = a.res != nullptr;
   p.e.o32 = a.out_f32;
   p.e.o16 = static_cast<__nv_bfloat16*>(a.out_bf16);
@@ -506,20 +510,25 @@ int launch_gemm_pair(const gecco_gemm_args& a, cudaStream_t stream, int* handled
   const int smem_bytes = SMEM_FIXED + epi_bytes + p.bstages * p.kbps * B_STAGE_BYTES;
 
   using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, PParams);
-  static const KernelFn kernels[4][2] = {{gemm_pair_kernel<0, false>, gemm_pair_kernel<0, true>},
+  static const KernelFn kernels[8][2] = {{gemm_pair_kernel<0, false>, gemm_pair_kernel<0, true>},
                                          {gemm_pair_kernel<1, false>, gemm_pair_kernel<1, true>},
                                          {gemm_pair_kernel<2, false>, gemm_pair_kernel<2, true>},
-                                         {gemm_pair_kernel<3, false>, gemm_pair_kernel<3, true>}};
+                                         {gemm_pair_kernel<3, false>, gemm_pair_kernel<3, true>},
+                                         {gemm_pair_kernel<4, false>, gemm_pair_kernel<4, true>},
+                                         {gemm_pair_kernel<5, false>, gemm_pair_kernel<5, true>},
+                                         {gemm_pair_kernel<6, false>, gemm_pair_kernel<6, true>},
+                                         {gemm_pair_kernel<7, false>, gemm_pair_kernel<7, true>}};
   static bool attr_set = false;
   if (!attr_set) {
-    for (int i = 0; i < 4; ++i)
+    for (int i = 0; i < 8; ++i)
       for (int j = 0; j < 2; ++j) {
         cudaError_t e = cudaFuncSetAttribute(kernels[i][j], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
         if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(gemm_pair_kernel)");
       }
     attr_set = true;
   }
-  const int epi_kind = fast ? (a.act ? 3 : 2) : (a.stats ? 1 : 0);
+  const int epi_kind = fast ? 2 + a.act                                           // 2 + GECCO_ACT_*
+                       : a.act == GECCO_ACT_GAUSSIAN_RAW ? 6 : a.act == GECCO_ACT_RELU ? 7 : (a.stats ? 1 : 0);
   int pairs = sms / 2;
   if (pairs > p.num_pair_blocks) pairs = p.num_pair_blocks;
   cudaLaunchConfig_t cfg = {};

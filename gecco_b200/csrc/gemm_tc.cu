@@ -43,7 +43,8 @@ struct KParams {
   int stages;
 };
 
-template <int W>
+// W: statistics width (0: none); ACT: activation (GECCO_ACT_GAUSSIAN: the Gaussian when p.e.act != 0, or none)
+template <int W, int ACT = GECCO_ACT_GAUSSIAN>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
                const __grid_constant__ CUtensorMap tma_res, const __grid_constant__ CUtensorMap tma_o32,
@@ -183,7 +184,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
       mbar_wait(&acc_full[slot], acc_phase);
       tc_fence_after_sync();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * ACC_COLS;
-      epi_panel<W>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, n0, cnt);
+      epi_panel<W, ACT>(p.e, es, et, &tma_o32, &tma_o16, taddr, m0, n0, cnt);
       tc_fence_before_sync();
       __syncwarp();
       if (et.lane == 0) mbar_arrive(&acc_empty[slot]);  // one arrival per warp
@@ -326,6 +327,11 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   GECCO_REQUIRE(!a.stats || a.n_out % stat_w == 0, "gemm: statistics epilogue needs n_out (%d) %% stat_gs (%d) == 0", a.n_out,
                 stat_w);
   GECCO_REQUIRE(!a.geom || (a.sigma && a.wx), "gemm: xyz embed needs sigma and wx");
+  GECCO_REQUIRE(a.act >= GECCO_ACT_NONE && a.act <= GECCO_ACT_RELU, "gemm: unknown activation code %d", a.act);
+  GECCO_REQUIRE(a.act <= GECCO_ACT_GAUSSIAN || !a.stats,
+                "gemm: the raw Gaussian / ReLU activations are not combined with statistics");
+  GECCO_REQUIRE(a.act == GECCO_ACT_NONE || a.act == GECCO_ACT_RELU || a.act_alpha != 0.f,
+                "gemm: act_alpha must be non-zero for the Gaussian activations");
   GECCO_REQUIRE(!a.w_rows_per_cloud || a.rows_per_cloud % BM == 0,
                 "gemm: per-cloud weights need rows_per_cloud %% 128 == 0");
 
@@ -353,7 +359,7 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   p.e.rows_per_cloud = a.rows_per_cloud; p.e.valid_rows = a.valid_rows; p.w_rows_per_cloud = a.w_rows_per_cloud;
   p.e.bias = a.bias; p.e.bias_stride = a.bias_stride;
   p.e.act = a.act;
-  p.e.act_k = a.act ? static_cast<float>(-1.4426950408889634 / (2.0 * (double)a.act_alpha * (double)a.act_alpha)) : 0.f;
+  p.e.act_k = act_k_of(a.act, a.act_alpha);
   p.e.has_res = a.res != nullptr;
   p.e.o32 = a.out_f32;
   p.e.o16 = static_cast<__nv_bfloat16*>(a.out_bf16);
@@ -370,8 +376,9 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
   const int smem_bytes = SMEM_FIXED + epi_bytes + p.stages * (A_STAGE_BYTES + B_STAGE_BYTES);
 
   using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, KParams);
-  static const KernelFn kernels[7] = {gemm_tc_kernel<0>,  gemm_tc_kernel<4>,  gemm_tc_kernel<8>, gemm_tc_kernel<12>,
-                                      gemm_tc_kernel<16>, gemm_tc_kernel<24>, gemm_tc_kernel<32>};
+  static const KernelFn kernels[9] = {gemm_tc_kernel<0>,  gemm_tc_kernel<4>,  gemm_tc_kernel<8>, gemm_tc_kernel<12>,
+                                      gemm_tc_kernel<16>, gemm_tc_kernel<24>, gemm_tc_kernel<32>,
+                                      gemm_tc_kernel<0, GECCO_ACT_GAUSSIAN_RAW>, gemm_tc_kernel<0, GECCO_ACT_RELU>};
   static bool attr_set = false;
   if (!attr_set) {
     for (KernelFn k : kernels) {
@@ -380,7 +387,8 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t stream) {
     }
     attr_set = true;
   }
-  const KernelFn kernel = !a.stats ? kernels[0] : stat_w == 4 ? kernels[1] : stat_w == 8 ? kernels[2] : stat_w == 12 ? kernels[3]
+  const KernelFn kernel = a.act == GECCO_ACT_GAUSSIAN_RAW ? kernels[7] : a.act == GECCO_ACT_RELU ? kernels[8]
+                          : !a.stats ? kernels[0] : stat_w == 4 ? kernels[1] : stat_w == 8 ? kernels[2] : stat_w == 12 ? kernels[3]
                           : stat_w == 16 ? kernels[4] : stat_w == 24 ? kernels[5] : kernels[6];
   const int tiles = p.num_m_blocks * p.num_n_blocks;
   const int grid = tiles < sm_count() ? tiles : sm_count();

@@ -151,6 +151,8 @@ __device__ __forceinline__ void store_bf16(__nv_bfloat16* dst, const float (&v)[
   }
 }
 
+// kAct: the MLP's hidden activation (GECCO_ACT_GAUSSIAN, GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU)
+template <int kAct>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(THREADS, 1)
 inducer_chain_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ CUtensorMap ta1,
                      const __grid_constant__ CUtensorMap ta2, const __grid_constant__ CUtensorMap ta3,
@@ -430,7 +432,7 @@ inducer_chain_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_const
         }
         named_bar_sync(3, EPI_THREADS_ALL);  // s_red may be rewritten by the next AdaGN stage
       } else {
-        // ---------------- 192 columns per CTA, 48 per thread: + bias (-> Gaussian activation) -> bf16
+        // ---------------- 192 columns per CTA, 48 per thread: + bias (-> activation) -> bf16
         __nv_bfloat16* out = s == 1 ? p.hh : p.khv;
         float v[48];
         tmem_load<48>(tlane + g * 48, v);
@@ -447,7 +449,11 @@ inducer_chain_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_const
         }
         if (s == 1) {
 #pragma unroll
-          for (int i = 0; i < 48; ++i) v[i] = fmaf(ex2f(v[i] * v[i] * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
+          for (int i = 0; i < 48; ++i) {
+            if constexpr (kAct == GECCO_ACT_GAUSSIAN) v[i] = fmaf(ex2f(v[i] * v[i] * p.act_k), 1.0f / 0.28f, -0.7f / 0.28f);
+            else if constexpr (kAct == GECCO_ACT_GAUSSIAN_RAW) v[i] = ex2f(v[i] * v[i] * p.act_k);
+            else v[i] = fmaxf(v[i], 0.f);
+          }
         }
         stage_bf16<48>(stg + lane * 96, v);
         warp_tile_to_global<96>(stg, reinterpret_cast<uint8_t*>(out + grow0 * HID + col0), HID * 2, rows_valid, lane);
@@ -503,6 +509,9 @@ int launch_inducer_chain(const gecco_chain_args& a, cudaStream_t stream) {
   }
   const int m = a.clouds * NI;
   CUtensorMap ta[4], tw[4];
+  const int act = mlp_act_of(a.act);
+  GECCO_REQUIRE(act == GECCO_ACT_GAUSSIAN || act == GECCO_ACT_GAUSSIAN_RAW || act == GECCO_ACT_RELU,
+                "inducer chain: unknown activation code %d", a.act);
   const void* as[4] = {a.pooled, a.hn, a.hh, a.h3};
   const void* ws[4] = {a.w_pool_out ? a.w_pool_out : a.w_kv, a.w_mlp0 ? a.w_mlp0 : a.w_kv, a.w_mlp2 ? a.w_mlp2 : a.w_kv, a.w_kv};
   const int ks[4] = {C, C, HID, C};
@@ -523,17 +532,23 @@ int launch_inducer_chain(const gecco_chain_args& a, cudaStream_t stream) {
     for (int i = 0; i < 4; ++i) p.n_w[n][i] = a.norm[n][i];
   p.t = a.t; p.t_stride = a.t_stride; p.eps = a.eps;
   p.b_mlp0 = a.b_mlp0; p.b_mlp2 = a.b_mlp2; p.b_kv = a.b_kv;
-  p.act_k = a.first_stage == 0 ? static_cast<float>(-1.4426950408889634 / (2.0 * (double)a.act_alpha * (double)a.act_alpha)) : 0.f;
+  p.act_k = a.first_stage == 0 ? act_k_of(act, a.act_alpha) : 0.f;
   p.hn = static_cast<__nv_bfloat16*>(a.hn); p.hh = static_cast<__nv_bfloat16*>(a.hh);
   p.h3 = static_cast<__nv_bfloat16*>(a.h3); p.khv = static_cast<__nv_bfloat16*>(a.khv);
   p.vt = static_cast<__nv_bfloat16*>(a.vt);
   p.cache_out = a.cache_out;
   p.dbg = g_gemm_debug;
 
+  using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap,
+                            CUtensorMap, CParams);
+  static const KernelFn kernels[3] = {inducer_chain_kernel<GECCO_ACT_GAUSSIAN>, inducer_chain_kernel<GECCO_ACT_GAUSSIAN_RAW>,
+                                      inducer_chain_kernel<GECCO_ACT_RELU>};  // [act - GECCO_ACT_GAUSSIAN]
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(inducer_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(inducer_chain_kernel)");
+    for (KernelFn k : kernels) {
+      cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+      if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(inducer_chain_kernel)");
+    }
     attr_set = true;
   }
   cudaLaunchConfig_t cfg = {};
@@ -546,7 +561,7 @@ int launch_inducer_chain(const gecco_chain_args& a, cudaStream_t stream) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, inducer_chain_kernel, ta[0], ta[1], ta[2], ta[3], tw[0], tw[1], tw[2], tw[3], p);
+  cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[act - GECCO_ACT_GAUSSIAN], ta[0], ta[1], ta[2], ta[3], tw[0], tw[1], tw[2], tw[3], p);
   if (le != cudaSuccess) return fail_cuda(le, "inducer_chain_kernel launch");
   GECCO_CHECK_LAUNCH("inducer_chain_kernel launch");
   return GECCO_OK;

@@ -28,6 +28,13 @@ int launch_gemm(const gecco_gemm_args& a, cudaStream_t s);
 inline bool epi_stat_width_supported(int w) { return w == 4 || w == 8 || w == 12 || w == 16 || w == 24 || w == 32; }
 template <typename Args>
 inline int epi_stat_width(const Args& a) { return a.stat_gs != 0 ? a.stat_gs : 12; }
+// Activation of a gecco_mlp / gecco_inducer_chain call or an engine model (0 there means the normalised Gaussian), and the
+// exponent scale -log2(e) / (2 alpha^2) an epilogue takes for the Gaussians (0 for none / ReLU, which do not read alpha).
+inline int mlp_act_of(int act) { return act == GECCO_ACT_NONE ? GECCO_ACT_GAUSSIAN : act; }
+inline bool act_is_gaussian(int act) { return act == GECCO_ACT_GAUSSIAN || act == GECCO_ACT_GAUSSIAN_RAW; }
+inline float act_k_of(int act, float alpha) {
+  return act_is_gaussian(act) ? static_cast<float>(-1.4426950408889634 / (2.0 * (double)alpha * (double)alpha)) : 0.f;
+}
 void set_graphs_option(int value);  // engine.cu: gecco_set_option("graphs", v)
 void set_chain_option(int value);  // engine.cu: gecco_set_option("chain", v)
 void set_anorm_option(int value);  // engine.cu: gecco_set_option("anorm", v)

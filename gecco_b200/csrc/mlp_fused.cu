@@ -3,7 +3,7 @@
 //     x <- x + W2 . g(W1_b . xb + b1_b) + b2          (W1_b, b1_b: mlp.0 with AdaGN_mlp folded in per cloud)
 // as ONE tcgen05 kernel.  The 768-wide hidden activation never leaves the SM: it is produced in 128-column chunks in
 // TMEM, pulled into registers by the epilogue warps (which frees the TMEM buffer for the next chunk at once), passed
-// through the Gaussian activation, written as bf16 into shared memory in the UMMA K-major 128B-swizzled layout and
+// through the activation, written as bf16 into shared memory in the UMMA K-major 128B-swizzled layout and
 // consumed as the A operand of the second GEMM, whose 128 x 384 fp32 accumulator stays in TMEM for the whole row
 // block.  Compared with the two-GEMM path this removes one write and one read of the [rows, 768] bf16 hidden tensor
 // per layer (402 MB at 64 clouds x 2048 points).
@@ -80,11 +80,8 @@ struct MParams {
   long long* dbg;              // development aid, nullptr in production
 };
 
-__device__ __forceinline__ float gauss_act(float v, float k) {
-  return fmaf(ex2_approx(v * v * k), 1.0f / 0.28f, -0.7f / 0.28f);
-}
-
-template <bool kStats>
+// kAct: the hidden activation (GECCO_ACT_GAUSSIAN, GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU)
+template <bool kStats, int kAct>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 mlp_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w1,
                  const __grid_constant__ CUtensorMap tma_w2, const __grid_constant__ CUtensorMap tma_res,
@@ -338,18 +335,18 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const float4 bi = __ldg(bp + i);
-          pk[2 * i] = pack_bf16x2(gauss_act(__uint_as_float(r0[4 * i + 0]) + bi.x, p.act_k),
-                                  gauss_act(__uint_as_float(r0[4 * i + 1]) + bi.y, p.act_k));
-          pk[2 * i + 1] = pack_bf16x2(gauss_act(__uint_as_float(r0[4 * i + 2]) + bi.z, p.act_k),
-                                      gauss_act(__uint_as_float(r0[4 * i + 3]) + bi.w, p.act_k));
+          pk[2 * i] = pack_bf16x2(epi_act<kAct>(__uint_as_float(r0[4 * i + 0]) + bi.x, p.act_k),
+                                  epi_act<kAct>(__uint_as_float(r0[4 * i + 1]) + bi.y, p.act_k));
+          pk[2 * i + 1] = pack_bf16x2(epi_act<kAct>(__uint_as_float(r0[4 * i + 2]) + bi.z, p.act_k),
+                                      epi_act<kAct>(__uint_as_float(r0[4 * i + 3]) + bi.w, p.act_k));
         }
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const float4 bi = __ldg(bp + 8 + i);
-          pk[16 + 2 * i] = pack_bf16x2(gauss_act(__uint_as_float(r1[4 * i + 0]) + bi.x, p.act_k),
-                                       gauss_act(__uint_as_float(r1[4 * i + 1]) + bi.y, p.act_k));
-          pk[16 + 2 * i + 1] = pack_bf16x2(gauss_act(__uint_as_float(r1[4 * i + 2]) + bi.z, p.act_k),
-                                           gauss_act(__uint_as_float(r1[4 * i + 3]) + bi.w, p.act_k));
+          pk[16 + 2 * i] = pack_bf16x2(epi_act<kAct>(__uint_as_float(r1[4 * i + 0]) + bi.x, p.act_k),
+                                       epi_act<kAct>(__uint_as_float(r1[4 * i + 1]) + bi.y, p.act_k));
+          pk[16 + 2 * i + 1] = pack_bf16x2(epi_act<kAct>(__uint_as_float(r1[4 * i + 2]) + bi.z, p.act_k),
+                                           epi_act<kAct>(__uint_as_float(r1[4 * i + 3]) + bi.w, p.act_k));
         }
         if (GECCO_DBG_ON(p.dbg)) c_act += clock64() - tl0;
         // the second GEMM of the previous chunk has finished reading the shared-memory chunk
@@ -412,7 +409,10 @@ static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
                 "12-channel statistics (c=%d hidden=%d m=%d rows_per_cloud=%d stat_gs=%d)", a.c, a.hidden, a.m, a.rows_per_cloud,
                 a.stat_gs);
   GECCO_REQUIRE(a.valid_rows > 0 && a.valid_rows <= a.rows_per_cloud, "mlp: valid_rows out of range");
-  GECCO_REQUIRE(a.act_alpha != 0.f, "mlp: act_alpha must be non-zero");
+  const int act = mlp_act_of(a.act);
+  GECCO_REQUIRE(act == GECCO_ACT_GAUSSIAN || act == GECCO_ACT_GAUSSIAN_RAW || act == GECCO_ACT_RELU,
+                "mlp: unknown activation code %d", a.act);
+  GECCO_REQUIRE(!act_is_gaussian(act) || a.act_alpha != 0.f, "mlp: act_alpha must be non-zero");
 
   const int clouds = ceil_div(a.m, a.rows_per_cloud);
   const uint64_t w1_rows = a.w1_rows_per_cloud ? (uint64_t)a.w1_rows_per_cloud * (clouds - 1) + a.hidden : (uint64_t)a.hidden;
@@ -434,7 +434,7 @@ static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
   p.e.stats = a.stats;
   p.e.geom = nullptr; p.e.sigma = nullptr; p.e.sigma_stride = 0; p.e.sigma_data = 1.f; p.e.wx = nullptr;
   p.b1 = a.b1; p.b1_stride = a.b1_stride;
-  p.act_k = static_cast<float>(-1.4426950408889634 / (2.0 * (double)a.act_alpha * (double)a.act_alpha));
+  p.act_k = act_k_of(act, a.act_alpha);
   p.w1_rows_per_cloud = a.w1_rows_per_cloud;
   p.num_chunks = a.hidden / HC;
   p.num_pair_blocks = a.m / (2 * BM);
@@ -443,11 +443,18 @@ static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
   p.e.skip = epi_skip_option();
   p.e.hints = 0;
 
+  using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, MParams);
+  static const KernelFn kernels[3][2] = {  // [act - GECCO_ACT_GAUSSIAN][stats]
+      {mlp_fused_kernel<false, GECCO_ACT_GAUSSIAN>, mlp_fused_kernel<true, GECCO_ACT_GAUSSIAN>},
+      {mlp_fused_kernel<false, GECCO_ACT_GAUSSIAN_RAW>, mlp_fused_kernel<true, GECCO_ACT_GAUSSIAN_RAW>},
+      {mlp_fused_kernel<false, GECCO_ACT_RELU>, mlp_fused_kernel<true, GECCO_ACT_RELU>}};
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(mlp_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(mlp_fused_kernel)");
+    for (int i = 0; i < 3; ++i)
+      for (int j = 0; j < 2; ++j) {
+        cudaError_t e = cudaFuncSetAttribute(kernels[i][j], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(mlp_fused_kernel)");
+      }
     attr_set = true;
   }
   int pairs = sm_count() / 2;
@@ -462,8 +469,7 @@ static int launch_mlp_fused(const gecco_mlp_args& a, cudaStream_t stream) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t le = a.stats ? cudaLaunchKernelEx(&cfg, mlp_fused_kernel<true>, ta, tw1, tw2, tres, t32, t16, p)
-                           : cudaLaunchKernelEx(&cfg, mlp_fused_kernel<false>, ta, tw1, tw2, tres, t32, t16, p);
+  cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[act - GECCO_ACT_GAUSSIAN][a.stats ? 1 : 0], ta, tw1, tw2, tres, t32, t16, p);
   if (le != cudaSuccess) return fail_cuda(le, "mlp_fused_kernel launch");
   GECCO_CHECK_LAUNCH("mlp_fused_kernel launch");
   return GECCO_OK;

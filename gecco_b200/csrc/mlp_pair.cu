@@ -209,7 +209,8 @@ __device__ __forceinline__ void epi_panel_ldg(const MParams& p, const EpiThread&
   }
 }
 
-template <bool kStats>
+// kAct: the hidden activation (GECCO_ACT_GAUSSIAN, GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU)
+template <bool kStats, int kAct>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 mlp_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w1,
                 const __grid_constant__ CUtensorMap tma_w2, const __grid_constant__ CUtensorMap tma_hs,
@@ -499,7 +500,7 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * ACC_COLS;
         long long tf0 = 0, tf1 = 0;
         if (p.dbg != nullptr) tf0 = clock64();
-        epi_tile_fast<true>(p.u, et, &tma_hs, taddr, srow, nb * BN, smem_u32(es.o16), row_valid, [&] {
+        epi_tile_fast<kAct>(p.u, et, &tma_hs, taddr, srow, nb * BN, smem_u32(es.o16), row_valid, [&] {
           tc_fence_before_sync();
           __syncwarp();
           if (et.lane == 0) mbar_arrive_leader(&acc_empty[slot]);
@@ -561,7 +562,10 @@ int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {
   GECCO_REQUIRE(mlp_pair_supported(a), "mlp (pair kernel): unsupported shape or missing A-operand normalisation / scratch");
   GECCO_REQUIRE(a.a && a.w1 && a.w2 && a.b1 && a.b2, "mlp: null operand");
   GECCO_REQUIRE(a.valid_rows > 0 && a.valid_rows <= a.rows_per_cloud, "mlp: valid_rows out of range");
-  GECCO_REQUIRE(a.act_alpha != 0.f, "mlp: act_alpha must be non-zero");
+  const int act = mlp_act_of(a.act);
+  GECCO_REQUIRE(act == GECCO_ACT_GAUSSIAN || act == GECCO_ACT_GAUSSIAN_RAW || act == GECCO_ACT_RELU,
+                "mlp: unknown activation code %d", a.act);
+  GECCO_REQUIRE(!act_is_gaussian(act) || a.act_alpha != 0.f, "mlp: act_alpha must be non-zero");
   GECCO_REQUIRE(a.anorm.t && a.anorm.scale_w && a.anorm.scale_b && a.anorm.bias_w && a.anorm.bias_b, "mlp: incomplete AdaGN");
 
   const int num_pair_blocks = a.m / (2 * BM);
@@ -588,8 +592,8 @@ int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {
     e.skip = 0; e.dbg = nullptr;
   };
   base(p.u, HID);
-  p.u.bias = a.b1; p.u.act = 1;
-  p.u.act_k = static_cast<float>(-1.4426950408889634 / (2.0 * (double)a.act_alpha * (double)a.act_alpha));
+  p.u.bias = a.b1; p.u.act = act;
+  p.u.act_k = act_k_of(act, a.act_alpha);
   p.u.o16 = static_cast<__nv_bfloat16*>(a.scratch);
   base(p.d, C);
   p.d.bias = a.b2; p.d.has_res = 1; p.d.o32 = a.out_f32; p.d.o16 = static_cast<__nv_bfloat16*>(a.out_bf16);
@@ -603,11 +607,19 @@ int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {
   p.u.hints = POL_HIDDEN << 6;  // bf16 stores of the first product's epilogue: the hidden tiles going to the scratch
   p.d.hints = 0;
 
+  using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap,
+                            CUtensorMap, MParams);
+  static const KernelFn kernels[3][2] = {  // [act - GECCO_ACT_GAUSSIAN][stats]
+      {mlp_pair_kernel<false, GECCO_ACT_GAUSSIAN>, mlp_pair_kernel<true, GECCO_ACT_GAUSSIAN>},
+      {mlp_pair_kernel<false, GECCO_ACT_GAUSSIAN_RAW>, mlp_pair_kernel<true, GECCO_ACT_GAUSSIAN_RAW>},
+      {mlp_pair_kernel<false, GECCO_ACT_RELU>, mlp_pair_kernel<true, GECCO_ACT_RELU>}};
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(mlp_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(mlp_pair_kernel)");
+    for (int i = 0; i < 3; ++i)
+      for (int j = 0; j < 2; ++j) {
+        cudaError_t e = cudaFuncSetAttribute(kernels[i][j], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        if (e != cudaSuccess) return fail_cuda(e, "cudaFuncSetAttribute(mlp_pair_kernel)");
+      }
     attr_set = true;
   }
   cudaLaunchConfig_t cfg = {};
@@ -620,8 +632,8 @@ int launch_mlp_pair(const gecco_mlp_args& a, cudaStream_t stream) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t le = a.stats ? cudaLaunchKernelEx(&cfg, mlp_pair_kernel<true>, ta, tw1, tw2, ths, thl, tres, t32, t16, p)
-                           : cudaLaunchKernelEx(&cfg, mlp_pair_kernel<false>, ta, tw1, tw2, ths, thl, tres, t32, t16, p);
+  cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[act - GECCO_ACT_GAUSSIAN][a.stats ? 1 : 0], ta, tw1, tw2, ths, thl, tres,
+                                      t32, t16, p);
   if (le != cudaSuccess) return fail_cuda(le, "mlp_pair_kernel launch");
   GECCO_CHECK_LAUNCH("mlp_pair_kernel launch");
   return GECCO_OK;

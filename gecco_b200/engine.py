@@ -26,20 +26,41 @@ def _get(mod, path: str):
     return mod
 
 
+_SUPPORTED_ACTIVATIONS = "GaussianActivation(normalized=True), GaussianActivation(normalized=False) or nn.ReLU"
+
+
+def _activation_code(act) -> int:
+    """GECCO_ACT_* of an MLP's activation module; anything else is refused."""
+    from .models.activation import GaussianActivation
+
+    if isinstance(act, GaussianActivation):
+        return _abi.ACT_GAUSSIAN if act.normalized else _abi.ACT_GAUSSIAN_RAW
+    if isinstance(act, torch.nn.ReLU):
+        return _abi.ACT_RELU
+    raise ValueError(f"gecco_b200: the CUDA path does not support the MLP activation {type(act).__name__}; "
+                     f"supported: {_SUPPORTED_ACTIVATIONS}")
+
+
+def _alpha(act):
+    """The Gaussian's alpha parameter; ReLU has none (the library does not read the slot)."""
+    return getattr(act, "alpha", None)
+
+
 def _layer_tensors(layer) -> list:
-    """fp32 tensors of one BroadcastingLayer in gecco_layer_weight order (include/gecco_b200.h)."""
+    """fp32 tensors of one BroadcastingLayer in gecco_layer_weight order (include/gecco_b200.h); None for the alphas of
+    a ReLU model."""
     t = []
     t += [_get(layer, "broadcast_norm." + n) for n in _NORM_LEAVES]
     t += [layer.broadcast.pool.inducers, layer.broadcast.pool.kv_proj.weight, layer.broadcast.pool.out_proj.weight]
     t += [_get(layer, "broadcast.norm_1." + n) for n in _NORM_LEAVES]
     m = layer.broadcast.mlp
-    t += [m[0].weight, m[0].bias, m[1].alpha, m[2].weight, m[2].bias]
+    t += [m[0].weight, m[0].bias, _alpha(m[1]), m[2].weight, m[2].bias]
     t += [_get(layer, "broadcast.norm_2." + n) for n in _NORM_LEAVES]
     u = layer.broadcast.unpool
     t += [u.in_proj_weight, u.in_proj_bias, u.out_proj.weight, u.out_proj.bias]
     t += [_get(layer, "mlp_norm." + n) for n in _NORM_LEAVES]
     m = layer.mlp
-    t += [m[0].weight, m[0].bias, m[1].alpha, m[2].weight, m[2].bias]
+    t += [m[0].weight, m[0].bias, _alpha(m[1]), m[2].weight, m[2].bias]
     assert len(t) == _abi.LW_COUNT
     return t
 
@@ -66,7 +87,6 @@ class Engine:
 
     # ------------------------------------------------------------------ handle management
     def _describe(self):
-        from .models.activation import GaussianActivation
         from .models.linear_lift import LinearLift
         from .models.ray import RayNetwork
 
@@ -113,12 +133,19 @@ class Engine:
         d.mlp_hidden = l0.mlp[0].out_features
         d.adagn_groups = l0.broadcast_norm.gn.num_groups
         d.sigma_data = self.sigma_data
+        acts = set()
         for layer in layers:
             for m in (layer.mlp, layer.broadcast.mlp):
-                if len(m) != 3 or not isinstance(m[1], GaussianActivation) or not m[1].normalized:
-                    raise ValueError("gecco_b200: the CUDA path supports depth-1 MLPs with the normalised GaussianActivation only")
+                if len(m) != 3:
+                    raise ValueError("gecco_b200: the CUDA path supports depth-1 MLPs only")
+                acts.add((_activation_code(m[1]), type(m[1]).__name__, getattr(m[1], "normalized", None)))
             if layer.broadcast_norm.scale.weight.shape[1] != 1:
                 raise ValueError("gecco_b200: t_embed_dim must be 1")
+        if len({a[0] for a in acts}) != 1:
+            names = ", ".join(sorted(n if z is None else f"{n}(normalized={z})" for _, n, z in acts))
+            raise ValueError(f"gecco_b200: every MLP of the model must use the same activation (found {names}); "
+                             f"supported: {_SUPPORTED_ACTIVATIONS}")
+        d.mlp_act = next(iter(acts))[0]
         net_t = [embed.weight, embed.bias, None if img is None else img.weight, None if img is None else img.bias,
                  out.weight, out.bias]
         layer_t = [t for layer in layers for t in _layer_tensors(layer)]
@@ -152,7 +179,7 @@ class Engine:
 
     def _ensure(self, device: torch.device):
         desc, net_t, layer_t = self._describe_cached()
-        tensors = [t for t in net_t if t is not None] + layer_t
+        tensors = [t for t in net_t + layer_t if t is not None]
         for t in tensors:
             if not t.is_cuda or t.dtype != torch.float32:
                 raise _abi.GeccoError("gecco_b200: model parameters must be float32 CUDA tensors (there is no CPU path); "
@@ -170,7 +197,7 @@ class Engine:
         keep = [t.detach().clone().contiguous() for t in tensors]
         it = iter(keep)
         net_ptrs = (C.c_void_p * _abi.NW_COUNT)(*[None if t is None else next(it).data_ptr() for t in net_t])
-        layer_ptrs = (C.c_void_p * len(layer_t))(*[next(it).data_ptr() for _ in layer_t])
+        layer_ptrs = (C.c_void_p * len(layer_t))(*[None if t is None else next(it).data_ptr() for t in layer_t])
         handle = C.c_void_p()
         with torch.cuda.device(device):
             stream = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)

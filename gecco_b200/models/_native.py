@@ -12,7 +12,7 @@ import math
 import torch
 from torch import Tensor
 
-from .. import ops
+from .. import _abi, ops
 
 ROW_TILE = 128  # rows per cloud are padded to the row tile of the tcgen05 kernels
 SUPPORTED_INDUCERS = (64, 128, 192, 256)  # whole 64-row blocks of the attention cores
@@ -49,16 +49,27 @@ def f32(b: Tensor | None, scale: float = 1.0) -> Tensor | None:
 
 
 def linear(a: Tensor, weight: Tensor, bias: Tensor | None, *, rows_per_cloud: int, valid_rows: int, act_alpha: float | None = None,
-           res: Tensor | None = None, want_f32: bool = False, want_bf16: bool = False, w_scale: float = 1.0):
+           act: int | None = None, res: Tensor | None = None, want_f32: bool = False, want_bf16: bool = False,
+           w_scale: float = 1.0):
     """a: bf16 [M, K]; returns (fp32 | None, bf16 | None) of epilogue(a @ weight.T + bias) (gecco_gemm)."""
-    return ops.gemm(a, bf16(weight, w_scale), bias=f32(bias, w_scale), act_alpha=act_alpha, res=res, out_f32=want_f32 or None,
-                    out_bf16=want_bf16 or None, rows_per_cloud=rows_per_cloud, valid_rows=valid_rows)
+    return ops.gemm(a, bf16(weight, w_scale), bias=f32(bias, w_scale), act_alpha=act_alpha, act=act, res=res,
+                    out_f32=want_f32 or None, out_bf16=want_bf16 or None, rows_per_cloud=rows_per_cloud, valid_rows=valid_rows)
+
+
+def epilogue_activation(act) -> tuple[int, float | None] | None:
+    """(GECCO_ACT_* code, alpha) of an activation module the GEMM epilogue applies (the two GaussianActivation forms and
+    nn.ReLU), else None."""
+    from .activation import GaussianActivation
+
+    if isinstance(act, GaussianActivation):
+        return (_abi.ACT_GAUSSIAN if act.normalized else _abi.ACT_GAUSSIAN_RAW), float(act.alpha)
+    if isinstance(act, torch.nn.ReLU):
+        return _abi.ACT_RELU, None
+    return None
 
 
 def mlp_forward(mlp, x: Tensor, residual: Tensor | None = None) -> Tensor:
     """MLP.forward (mlp.py:5-39) on [B, N, C_in]; `residual` ([B, N, C_out]) is added in the last epilogue."""
-    from .activation import GaussianActivation
-
     B, N, _ = x.shape
     a, N, Np = pad_rows(x)
     mods = list(mlp)
@@ -66,10 +77,11 @@ def mlp_forward(mlp, x: Tensor, residual: Tensor | None = None) -> Tensor:
     h16 = None
     while rest:
         act, nxt, rest = rest[0], rest[1], rest[2:]
-        if isinstance(act, GaussianActivation) and act.normalized:
+        fused = epilogue_activation(act)
+        if fused is not None:
             # activation fused into the epilogue of the projection that feeds it
             _, h16 = linear(a if h16 is None else h16, lin.weight, lin.bias, rows_per_cloud=Np, valid_rows=N,
-                            act_alpha=float(act.alpha), want_bf16=True)
+                            act=fused[0], act_alpha=fused[1], want_bf16=True)
         else:
             z, _ = linear(a if h16 is None else h16, lin.weight, lin.bias, rows_per_cloud=Np, valid_rows=N, want_f32=True)
             h16 = act(z).to(torch.bfloat16)  # any other activation module runs on the fp32 projection output

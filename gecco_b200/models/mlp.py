@@ -2,9 +2,9 @@
 
 Linear -> activation -> [Linear -> activation] x (depth-1) -> Linear as an nn.Sequential, so the state_dict keys
 are `0.weight, 0.bias, 1.alpha, 2.weight, 2.bias` for depth 1.  Inside the denoiser engine the point-side MLP runs as
-tcgen05 GEMMs with the activation, bias and residual in their epilogues (depth 1 with GaussianActivation, the only
-configuration the reference uses, set_transformer.py:80-83,148-150); the stand-alone `forward` below runs the same
-GEMM kernel per Linear for any depth.
+tcgen05 GEMMs with the activation, bias and residual in their epilogues (depth 1, with GaussianActivation in either
+form or nn.ReLU, the reference's default; every MLP of a model uses the same one); the stand-alone `forward` below runs
+the same GEMM kernel per Linear for any depth.  Other activation modules are refused by the engine.
 """
 from typing import Callable
 
@@ -24,8 +24,9 @@ class MLP(nn.Sequential):
 
     @torch.no_grad()
     def forward(self, x):
-        """[..., in_features] -> [..., out_features]; every Linear is one `gecco_gemm` launch, a normalised
-        GaussianActivation is fused into the epilogue of the projection in front of it."""
+        """[..., in_features] -> [..., out_features]; every Linear is one `gecco_gemm` launch.  GaussianActivation (either
+        form) and nn.ReLU are fused into the epilogue of the projection in front of them; any other activation module
+        runs as its own torch forward on the fp32 projection output."""
         from . import _native
 
         lead = x.shape[:-1]

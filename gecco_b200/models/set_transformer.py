@@ -6,6 +6,9 @@ module: `gecco_b200.engine.Engine` walks this tree once, packs the weights and r
 engine (csrc/engine.cu).  Every module here ALSO has the reference's stand-alone `forward` (same arguments and return
 conventions), executed with the same C-ABI kernels through `models/_native.py`: tcgen05 GEMMs with fused bias /
 activation / residual epilogues, the two attention cores and the AdaGN kernels.  No torch math, no CPU path.
+`activation` (every MLP of the model): nn.ReLU (the reference's default), GaussianActivation (normalised, the reference
+configurations' choice) or GaussianActivation(normalized=False), e.g. `functools.partial(GaussianActivation,
+normalized=False)`; the engine refuses any other module.
 """
 from __future__ import annotations
 

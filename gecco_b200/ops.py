@@ -38,6 +38,7 @@ def gemm(
     bias: Tensor | None = None,
     bias_stride: int = 0,
     act_alpha: float | None = None,
+    act: int | None = None,
     res: Tensor | None = None,
     out_f32: Tensor | bool | None = None,
     out_bf16: Tensor | bool | None = None,
@@ -57,7 +58,9 @@ def gemm(
     """out = epilogue(a @ w.T) on the tcgen05 tensor cores; see gecco_gemm in include/gecco_b200.h.
     stats (f64 [clouds, n_out / stat_gs, 2]) receives the AdaGN statistics per group of stat_gs channels (4, 8, 12, 16, 24 or 32).
     anorm = dict(stats f64 [clouds, K/stat_gs, 2], t fp32 [clouds], scale_w, scale_b, bias_w, bias_b, groups, stat_gs=12,
-    eps=1e-5): `a` is the un-normalised bf16 tensor and AdaGN is applied to it inside the kernel."""
+    eps=1e-5): `a` is the un-normalised bf16 tensor and AdaGN is applied to it inside the kernel.
+    act: the epilogue activation (_abi.ACT_*); without it, act_alpha alone selects the normalised Gaussian.  act_alpha is
+    read for the two Gaussians only."""
     assert a.dtype == torch.bfloat16
     lib = _lib_for(a)
     assert w.dtype == torch.bfloat16
@@ -91,7 +94,9 @@ def gemm(
     args.rows_per_cloud, args.valid_rows, args.w_rows_per_cloud = rows_per_cloud, valid_rows, w_rows_per_cloud
     args.bias = 0 if bias is None else bias.data_ptr()
     args.bias_stride = bias_stride
-    args.act = 0 if act_alpha is None else 1
+    if act is None:
+        act = _abi.ACT_NONE if act_alpha is None else _abi.ACT_GAUSSIAN
+    args.act = act
     args.act_alpha = 1.0 if act_alpha is None else float(act_alpha)
     if res is not None:
         assert res.dtype == torch.float32 and res.stride(1) == 1
@@ -124,12 +129,13 @@ def set_option(name: str, value: int) -> None:
     _abi.check(_abi.load().gecco_set_option(name.encode(), C.c_int(int(value))))
 
 
-def mlp(a: Tensor, w1: Tensor, b1: Tensor, act_alpha: float, w2: Tensor, b2: Tensor, res: Tensor, *,
+def mlp(a: Tensor, w1: Tensor, b1: Tensor, act_alpha: float | None, w2: Tensor, b2: Tensor, res: Tensor, *,
         out_f32: Tensor | None = None, out_bf16: Tensor | bool | None = None, stats: Tensor | None = None,
         rows_per_cloud: int | None = None, valid_rows: int | None = None, w1_rows_per_cloud: int = 0,
-        b1_stride: int = 0, anorm: dict | None = None):
+        b1_stride: int = 0, anorm: dict | None = None, act: int = _abi.ACT_GAUSSIAN):
     """out = res + w2 @ g(w1_cloud @ a + b1_cloud) + b2 with the hidden activation kept on chip; see gecco_mlp in
-    include/gecco_b200.h (models/set_transformer.py:165-166)."""
+    include/gecco_b200.h (models/set_transformer.py:165-166).  g: `act` (_abi.ACT_GAUSSIAN, ACT_GAUSSIAN_RAW or
+    ACT_RELU); act_alpha is read for the Gaussians."""
     lib = _lib_for(a)
     assert a.dtype == torch.bfloat16 and w1.dtype == torch.bfloat16 and w2.dtype == torch.bfloat16
     assert a.dim() == 2 and a.stride(1) == 1 and w1.stride(1) == 1 and w2.stride(1) == 1
@@ -150,7 +156,8 @@ def mlp(a: Tensor, w1: Tensor, b1: Tensor, act_alpha: float, w2: Tensor, b2: Ten
     args.a, args.lda = a.data_ptr(), a.stride(0)
     args.w1, args.ldw1, args.w1_rows_per_cloud = w1.data_ptr(), w1.stride(0), w1_rows_per_cloud
     args.b1, args.b1_stride = b1.data_ptr(), b1_stride
-    args.act_alpha = float(act_alpha)
+    args.act_alpha = 0.0 if act_alpha is None else float(act_alpha)
+    args.act = act
     args.w2, args.ldw2 = w2.data_ptr(), w2.stride(0)
     args.b2 = b2.data_ptr()
     args.m, args.c, args.hidden = m, c, hidden
@@ -442,13 +449,15 @@ def pool_attention_partial(kv: Tensor, q_inducers: Tensor, *, clouds: int, rows_
     return (partial, used.value) if used.value > 1 else (out, 1)
 
 
-def inducer_chain(pooled: Tensor, w_pool_out: Tensor, norm1: list[Tensor], w_mlp0: Tensor, b_mlp0: Tensor, act_alpha: float,
-                  w_mlp2: Tensor, b_mlp2: Tensor, norm2: list[Tensor], w_kv: Tensor, b_kv: Tensor, t: Tensor, *,
-                  partial: Tensor | None = None, splits: int = 1, eps: float = 1e-5, want_cache: bool = True, first_stage: int = 0):
+def inducer_chain(pooled: Tensor, w_pool_out: Tensor, norm1: list[Tensor], w_mlp0: Tensor, b_mlp0: Tensor,
+                  act_alpha: float | None, w_mlp2: Tensor, b_mlp2: Tensor, norm2: list[Tensor], w_kv: Tensor, b_kv: Tensor,
+                  t: Tensor, *, partial: Tensor | None = None, splits: int = 1, eps: float = 1e-5, want_cache: bool = True,
+                  first_stage: int = 0, act: int = _abi.ACT_GAUSSIAN):
     """Inducer side of one Broadcast layer in one launch (gecco_inducer_chain).  pooled: bf16 [clouds*64, C] (input when
     splits <= 1, scratch otherwise); weights bf16 [n_out, k]; norm1 / norm2: [scale.weight, scale.bias, bias.weight,
     bias.bias] fp32 [C]; t: fp32 [clouds].  Returns (h3 bf16 [clouds*64, C], khv bf16 [clouds*64, 2C], vt bf16 [clouds, C, 64],
-    cache fp32 [clouds*64, C] or None).  first_stage = 3: `pooled` is taken as h3 (bf16 cached inducer states)."""
+    cache fp32 [clouds*64, C] or None).  first_stage = 3: `pooled` is taken as h3 (bf16 cached inducer states).
+    act: the MLP's activation (_abi.ACT_GAUSSIAN, ACT_GAUSSIAN_RAW or ACT_RELU); act_alpha is read for the Gaussians."""
     lib = _lib_for(pooled)
     m, c = pooled.shape
     clouds = m // 64
@@ -470,7 +479,8 @@ def inducer_chain(pooled: Tensor, w_pool_out: Tensor, norm1: list[Tensor], w_mlp
     a.pooled = pooled.data_ptr()
     a.w_pool_out, a.w_mlp0, a.w_mlp2, a.w_kv = w_pool_out.data_ptr(), w_mlp0.data_ptr(), w_mlp2.data_ptr(), w_kv.data_ptr()
     a.b_mlp0, a.b_mlp2, a.b_kv = b_mlp0.data_ptr(), b_mlp2.data_ptr(), b_kv.data_ptr()
-    a.act_alpha = act_alpha
+    a.act_alpha = 0.0 if act_alpha is None else act_alpha
+    a.act = act
     for n, ws in enumerate((norm1, norm2)):
         for i in range(4):
             assert ws[i].dtype == torch.float32 and ws[i].is_contiguous()

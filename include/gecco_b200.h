@@ -64,7 +64,7 @@ int gecco_set_option(const char* name, int value);
  * Epilogue, applied in this order on the fp32 accumulator:
  *   + bias[cloud*bias_stride + n]                     (bias may be NULL)
  *   + xyz embed: sum_j c_in(sigma)*geom[point,j]*wx[n,j]  (geom may be NULL; models/ray.py:99,113)
- *   Gaussian activation (exp(-z^2/(2 alpha^2)) - 0.7)/0.28 when act != 0 (models/activation.py:17-24)
+ *   activation `act` (GECCO_ACT_*, below; act_alpha is read for the two Gaussians only)
  *   + res[m, n]                                       (res may be NULL; residual adds set_transformer.py:164,166)
  *   per (cloud, stat_gs-channel group) sum / sum of squares of the result added into
  *   stats (double [clouds][n_out/stat_gs][2]) for the next AdaGN (models/normalization.py:36-44)
@@ -80,6 +80,19 @@ int gecco_set_option(const char* name, int value);
  * mean / rstd come from stats (double [clouds][K/stat_gs][2] sums over the valid rows, as written by a producing
  * epilogue), groups = number of normalisation groups, t[cloud*t_stride] the noise embedding, scale/bias the two
  * nn.Linear(1, K) of AdaGN.  Supported where gecco_gemm_anorm_supported() says so (CTA-pair kernel shapes). */
+/* Activation codes of the hidden projection's epilogue (models/activation.py:17-24, nn.ReLU), applied to the fp32
+ * accumulator + bias z:
+ *   GECCO_ACT_NONE 0          z
+ *   GECCO_ACT_GAUSSIAN 1      (exp(-z^2 / (2 alpha^2)) - 0.7) / 0.28   GaussianActivation(normalized=True)
+ *   GECCO_ACT_GAUSSIAN_RAW 2  exp(-z^2 / (2 alpha^2))                 GaussianActivation(normalized=False)
+ *   GECCO_ACT_RELU 3          max(z, 0)                               nn.ReLU
+ * In gecco_mlp_args.act, gecco_chain_args.act and gecco_model_desc.mlp_act there is always an activation: 0 (the
+ * zero-initialised value) means GECCO_ACT_GAUSSIAN there. */
+#define GECCO_ACT_NONE 0
+#define GECCO_ACT_GAUSSIAN 1
+#define GECCO_ACT_GAUSSIAN_RAW 2
+#define GECCO_ACT_RELU 3
+
 typedef struct gecco_anorm {
   const double* stats; int32_t stat_gs; int32_t groups; float eps;
   const float* t; int32_t t_stride;
@@ -94,7 +107,7 @@ typedef struct gecco_gemm_args {
   int32_t valid_rows;       /* <= rows_per_cloud */
   int32_t w_rows_per_cloud; /* 0: one weight for all clouds; else row offset between per-cloud weights */
   const float* bias; int32_t bias_stride;
-  int32_t act; float act_alpha;
+  int32_t act; float act_alpha;  /* GECCO_ACT_*; the ReLU / raw Gaussian activations do not combine with stats */
   const float* res; int64_t ldr;
   float* out_f32;  int64_t ldo32;
   void* out_bf16;  int64_t ldo16;
@@ -116,7 +129,7 @@ int gecco_gemm_anorm_supported(int32_t m, int32_t rows_per_cloud, int32_t n_out,
 /* ------------------------------------------------------------------------
  * Fused point-side MLP with residual (BroadcastingLayer.forward, models/set_transformer.py:165-166;
  * MLP, models/mlp.py:5-39; GaussianActivation, models/activation.py:17-24):
- *   out = res + W2 . g(W1_b . a + b1_b) + b2,   g(z) = (exp(-z^2 / (2 alpha^2)) - 0.7) / 0.28
+ *   out = res + W2 . g(W1_b . a + b1_b) + b2,   g = the activation `act` (GECCO_ACT_*, 0: GECCO_ACT_GAUSSIAN)
  * a:  bf16 [m, c] (the bf16 copy of the residual stream), W1_b: bf16 [hidden, c] per cloud
  * (w1_rows_per_cloud = row offset between clouds, 0 = shared), b1_b fp32 [clouds][b1_stride];
  * W2: bf16 [c, hidden], b2 fp32 [c].  The hidden activation stays on chip (TMEM -> shared memory).
@@ -145,6 +158,7 @@ typedef struct gecco_mlp_args {
   void* scratch;      /* anorm path: bf16 device scratch of min(m, 128 * #SMs) x hidden elements: the hidden activation of
                        * the row block a CTA is working on (rewritten every row block: L2-resident, never read after the call) */
   int32_t stat_gs;    /* channels per statistics group: 0 or 12 (the only width these kernels are built for) */
+  int32_t act;        /* GECCO_ACT_GAUSSIAN (or 0), GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU; act_alpha is read for the Gaussians */
 } gecco_mlp_args;
 
 int gecco_mlp(const gecco_mlp_args* args, void* stream);
@@ -323,7 +337,7 @@ int gecco_unpool_attention(const gecco_unpool_args* args, void* stream);
 
 /* The inducer side of Broadcast.forward (models/set_transformer.py:106-112) in one launch:
  *   pooled (or the key-split partials of gecco_pool_attention) -> pool.out_proj -> norm_1 (AdaGN) -> mlp
- *   (Linear, Gaussian activation, Linear) -> norm_2 (AdaGN) -> unpool key | value in-projection (+ V transposed per cloud).
+ *   (Linear, activation `act`, Linear) -> norm_2 (AdaGN) -> unpool key | value in-projection (+ V transposed per cloud).
  * A cluster of four CTAs owns two clouds; the AdaGN statistics over (64 inducers, 12 channels) are computed inside the
  * producing accumulator tile.  Shapes: 64 inducers, C = 384, hidden = 768, 8 heads, 32 groups (gecco-torch's only
  * configuration); gecco_inducer_chain returns GECCO_ERR_INVALID for anything else (the engine then runs the stages as
@@ -344,6 +358,7 @@ typedef struct gecco_chain_args {
   const float* t; int32_t t_stride; float eps;
   void *hn, *hh, *h3, *khv, *vt;
   float* cache_out;
+  int32_t act;                            /* GECCO_ACT_GAUSSIAN (or 0), GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU */
 } gecco_chain_args;
 int gecco_inducer_chain(const gecco_chain_args* args, void* stream);
 
@@ -365,6 +380,8 @@ typedef struct gecco_model_desc {
   int32_t reparam;       /* reparam of the lookup: 0 none, 1 gaussian, 2 uvl (ray.py:71) */
   float mean[3], sigma[3], logit_scale;
   float sigma_data;      /* EDMPrecond.sigma_data (diffusion.py:31) */
+  int32_t mlp_act;       /* activation of every MLP: GECCO_ACT_GAUSSIAN (or 0), GECCO_ACT_GAUSSIAN_RAW or GECCO_ACT_RELU; with
+                          * ReLU the GECCO_LW_*_ALPHA weights may be NULL and are not read */
 } gecco_model_desc;
 
 /* fp32 device pointers in the reference state_dict schema (SURVEY.md §8b). */
